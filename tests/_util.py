@@ -10,6 +10,13 @@ def load_golden(name):
     return torch.load(os.path.join(GOLDEN, name), map_location="cpu", weights_only=False)
 
 
+def load_wsrglow_golden():
+    """wsrglow_tiny.pt with the gradients of its flows, which are stored in a file of their own to keep each under 1 MB."""
+    fx = load_golden("wsrglow_tiny.pt")
+    fx["grads"].update(load_golden("wsrglow_tiny_wn_grads.pt"))
+    return fx
+
+
 def rel_l2(a, b):
     a = a.detach().double().cpu()
     b = b.detach().double().cpu()

@@ -1,9 +1,10 @@
 """Model-level parity the reference's own tests lack: WaveGlow against the golden fixture of the unmodified reference and
-against the CPU oracle, per precision mode.  The block-level properties (input storage freed and restored, exact
-invertibility, naive vs constant-memory gradients) are checked by the reference's OWN tests/test_fwd_bwd.py, run unmodified
-against these modules by tests/test_reference_suite.py -- no transcription of it lives here."""
+against the CPU oracle, per precision mode.  Block level: chains of 1x1 convs and affine couplings with the constant-memory
+backward against the same chains storing their activations (input storage freed and restored, gradients, invertibility),
+the properties the reference's own tests/test_fwd_bwd.py checks."""
 import pytest
 import torch
+from torch import nn
 
 import constant_memory_waveglow_b200 as cm
 from constant_memory_waveglow_b200 import precision
@@ -85,3 +86,56 @@ def test_waveglow_128ch_against_oracle(prec):
     with torch.no_grad():
         xr, _ = m.reverse(z.detach().clone(), h.cuda())
     assert rel_l2(xr, x) < max(tol["roundtrip"], 2e-5), rel_l2(xr, x)
+
+
+# ------------------------------------------------------------------------------------------------
+# block level
+# ------------------------------------------------------------------------------------------------
+def _chain(efficient, reverse_mode, cin, aux, ch, depth):
+    torch.manual_seed(0)
+    return nn.ModuleList([m for _ in range(2) for m in (
+        cm.InvertibleConv1x1(2 * cin, efficient, reverse_mode),
+        cm.AffineCouplingBlock(cm.WN, efficient, reverse_mode, in_channels=cin, aux_channels=aux, zero_init=False,
+                               dilation_channels=ch, residual_channels=ch, skip_channels=ch, depth=depth))]).cuda()
+
+
+def _run(blocks, x, y, inverse=False):
+    h, logdet = x, 0
+    for b in (reversed(blocks) if inverse else blocks):
+        args = (h, y) if isinstance(b, cm.AffineCouplingBlock) else (h,)
+        h, ld = b.reverse(*args) if inverse else b(*args)
+        logdet = logdet + ld.sum()
+    return h, logdet
+
+
+@pytest.mark.parametrize("reverse_mode", [False, True])
+@pytest.mark.parametrize("cin,aux,ch,depth,B,T", [(4, 12, 32, 2, 2, 300), (8, 40, 128, 4, 2, 1000)])
+def test_constant_memory_chain_matches_stored_activations(cin, aux, ch, depth, B, T, reverse_mode):
+    """Two flows (1x1 conv -> affine coupling), so every block's freed input is the previous block's output: the
+    constant-memory chain frees its input, restores it in the backward and gives the outputs and gradients of the chain
+    that stores its activations; the inverse chain returns the input."""
+    precision.set_precision("fp32")
+    g = torch.Generator().manual_seed(1)
+    x = (torch.rand(B, 2 * cin, T, generator=g) * 2 - 1).cuda()
+    y = torch.randn(B, aux, T, generator=g).cuda()
+    dz = torch.randn(B, 2 * cin, T, generator=g).cuda()
+    stored = _chain(False, reverse_mode, cin, aux, ch, depth)
+    res = {}
+    for efficient in (False, True):
+        blocks = stored if not efficient else _chain(True, reverse_mode, cin, aux, ch, depth)
+        blocks.load_state_dict(stored.state_dict())
+        xg, yg = x.clone().requires_grad_(True), y.clone().requires_grad_(True)
+        xin = xg.clone()
+        z, logdet = _run(blocks, xin, yg)
+        assert (xin.untyped_storage().size() == 0) == efficient          # only the constant-memory chain frees it
+        ((z * dz).sum() + logdet).backward()
+        assert xin.untyped_storage().size() > 0 and rel_l2(xin, x) < 1e-5  # restored in place by the backward
+        with torch.no_grad():
+            xr, ldr = _run(blocks, z.detach().clone(), y, inverse=True)
+        assert rel_l2(xr, x) < 1e-5 and abs(ldr.item() + logdet.item()) < 1e-4 * max(abs(logdet.item()), 1.0)
+        res[efficient] = dict(z=z.detach(), logdet=logdet.detach(), dx=xg.grad, dy=yg.grad,
+                              **{n: p.grad for n, p in blocks.named_parameters()})
+    for k, want in res[False].items():
+        got = res[True][k]
+        assert got is not None and want is not None, k
+        assert rel_l2(got, want) < 2e-5, (k, rel_l2(got, want))

@@ -1,12 +1,12 @@
 """WSRGlow (config 5 of BASELINE.json; reference model/wsrglow.py) through the CUDA path against the CPU oracle
-and the fixture the unmodified reference produced (tests/golden/wsrglow_tiny.pt)."""
+and the fixture the unmodified reference produced (tests/golden/wsrglow_tiny*.pt)."""
 import pytest
 import torch
 
 import constant_memory_waveglow_b200 as cm
 from constant_memory_waveglow_b200 import precision
 from oracle import flow_oracle as O
-from tests._util import load_golden, rel_l2
+from tests._util import load_wsrglow_golden, rel_l2
 
 pytestmark = pytest.mark.gpu
 
@@ -46,7 +46,7 @@ def test_conditioning_kernel_matches_op_by_op_form():
 
 
 def test_conditioning_front_end_matches_reference():
-    fx = load_golden("wsrglow_tiny.pt")
+    fx = load_wsrglow_golden()
     m, sd = build(fx)
     cond = m._get_cond(fx["c"].clone().cuda()).cpu()
     ref = O.wsrglow_cond(sd, fx["c"])
@@ -63,7 +63,7 @@ def test_wsrglow_train_step_against_reference_fixture(prec, tz, tg):
     # tz for fp16 is 2e-3, not 1e-3: the fixture's log-det values (1.8, 7.8) are nearly cancelling sums of 8192 log_s terms
     # of a 64-channel toy model, so their RELATIVE error overstates the per-element error (z itself is within 3e-4); the
     # full-size configurations are held to 1e-3 in tests/test_gpu_lj_parity.py
-    fx = load_golden("wsrglow_tiny.pt")
+    fx = load_wsrglow_golden()
     precision.set_precision(prec)
     m, sd = build(fx)
     x, c = fx["x"].cuda(), fx["c"].cuda()

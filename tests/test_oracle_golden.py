@@ -6,6 +6,7 @@ import pytest
 import torch
 
 from oracle import flow_oracle as O
+from tests._util import load_wsrglow_golden
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -114,7 +115,7 @@ def test_random_state_has_reference_keys():
 def test_wsrglow_tiny_against_reference():
     """WSRGlow 2x (model/wsrglow.py): conditioning front end + flow, outputs and gradients from the
     unmodified reference; weights are regenerated from the seed the fixture records."""
-    fx = load("wsrglow_tiny.pt")
+    fx = load_wsrglow_golden()
     ga = fx["gen_args"]
     sd = O.wsrglow_random_state(**ga)
     assert list(sd.keys()) == fx["state_keys"] or set(sd.keys()) == set(fx["state_keys"])

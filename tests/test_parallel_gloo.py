@@ -158,7 +158,9 @@ def _trainer_worker(rank, world, port, root, out):
             dist.destroy_process_group()
 
 
-def test_trainer_two_ranks_gloo(tmp_path):
+def test_trainer_two_ranks_gloo(tmp_path, monkeypatch):
+    # the ranks are CPU processes on any machine: with a GPU visible Trainer.fit would give each rank a device of its own
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
     world = 2
     port = _free_port()
     mgr = mp.Manager()
