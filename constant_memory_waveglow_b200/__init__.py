@@ -4,7 +4,7 @@ Host side: PyTorch modules / autograd Functions with the reference's names and s
 Device side: hand-written CUDA (tcgen05 / TMEM / TMA GEMM engine + fp32 CUDA-core engine +
 HBM-bound flow primitives) behind the C ABI of include/cmwg_b200.h, loaded with ctypes.
 """
-from .base import FlowBase, Reversible
+from .base import FlowBase, Reversible, pad_batch
 from .efficient_modules import (AffineCouplingBlock, AffineCouplingFunc, Conv1x1Func, InvAffineCouplingFunc,
                                 InvConv1x1Func, InvertibleConv1x1)
 from .loss import WaveGlowLoss
@@ -19,4 +19,4 @@ from .melglow import MelGlow, WN_LVC
 __all__ = ["FlowBase", "Reversible", "AffineCouplingBlock", "InvertibleConv1x1", "AffineCouplingFunc",
            "InvAffineCouplingFunc", "Conv1x1Func", "InvConv1x1Func", "WaveGlowLoss", "WN", "NonCausalLayer",
            "WaveGlow", "WSRGlow", "MRWaveGlow", "MelGlow", "WN_LVC", "WaveFlow", "WN2D", "NonCausalLayer2D", "fused_gate", "add_weight_norms", "remove_weight_norms", "get_instance", "set_precision",
-           "get_precision", "invalidate_packs"]
+           "get_precision", "invalidate_packs", "pad_batch"]

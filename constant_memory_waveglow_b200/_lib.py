@@ -65,6 +65,7 @@ SIGNATURES = {
     "cmwg_conv1x1_backward_workspace": (_SZ, [_I, _I, _I]),
     "cmwg_conv1x1_backward": (_I, [_VP, _VP, _I, _VP, _LL, _VP, _LL, _VP, _I, _I, _I, _VP, _LL, _VP, _LL, _VP, _VP, _VP]),
     "cmwg_coupling_apply": (_I, [_VP, _LL, _VP, _VP, _LL, _VP, _I, _I, _I, _I, _VP]),
+    "cmwg_coupling_apply_varlen": (_I, [_VP, _LL, _VP, _VP, _LL, _VP, _I, _I, _I, _VP, _I, _VP]),
     "cmwg_coupling_bwd": (_I, [_VP, _LL, _VP, _VP, _LL, _VP, _LL, _VP, _VP, _VP, _I, _I, _I, _I, _VP]),
     "cmwg_wn_tc_supported": (_I, [C.POINTER(WnConfig)]),
     "cmwg_wn_aux_padded": (_I, [C.POINTER(WnConfig)]),
@@ -75,6 +76,9 @@ SIGNATURES = {
     "cmwg_wn_workspace_bytes": (_SZ, [C.POINTER(WnConfig), _I, _I]),
     "cmwg_wn_saved_bytes": (_SZ, [C.POINTER(WnConfig), _I, _I]),
     "cmwg_wn_forward": (_I, [C.POINTER(WnConfig), _VP, _VP, _LL, _VP, _I, _I, _VP, _VP, _VP, _VP]),
+    "cmwg_wn_varlen_workspace_bytes": (_SZ, [C.POINTER(WnConfig), _I, _I]),
+    "cmwg_wn_forward_varlen": (_I, [C.POINTER(WnConfig), _VP, _VP, _LL, _VP, _I, _I, C.POINTER(C.c_int), _VP, _VP, _VP,
+                                    _VP]),
     "cmwg_wn_line_state_bytes": (_SZ, [C.POINTER(WnConfig), _I, _I]),
     "cmwg_wn_forward_lines": (_I, [C.POINTER(WnConfig), _VP, _VP, _LL, _VP, _I, _I, _I, _I, _VP, _VP, _VP, _VP]),
     "cmwg_waveflow_affine": (_I, [_VP, _I, _VP, _VP, _I, _I, _I, _I, _I, _I, _I, _VP]),
@@ -99,12 +103,15 @@ SIGNATURES = {
     "cmwg_nll_loss": (_I, [_VP, _VP, _I, _I, C.c_float, _I, _VP, _VP, _VP, _VP]),
     "cmwg_sum_per_batch": (_I, [_VP, _LL, _I, _I, _VP, _I, C.c_float, _VP]),
     "cmwg_logdet_accumulate": (_I, [_VP, _LL, _I, _I, _VP, _VP, _VP, _VP]),
+    "cmwg_logdet_accumulate_varlen": (_I, [_VP, _LL, _I, _I, _I, _VP, _VP, _VP, _VP, _VP]),
     "cmwg_profile_enable": (_I, [_I]),
     "cmwg_profile_collect": (_I, [C.POINTER(C.c_double), C.POINTER(C.c_longlong)]),
     "cmwg_mega_clk_read": (_I, [C.POINTER(C.c_longlong), _I]),
     "cmwg_debug_counter": (C.c_ulonglong, [_I]),
     "cmwg_wgrad_plan_splits": (_I, [_I, _I, _I, _I]),
     "cmwg_mega_task_list": (_I, [_I, _I, _I, _I, C.POINTER(C.c_int), _I, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "cmwg_mega_task_list_varlen": (_I, [_I, _I, _I, C.POINTER(C.c_int), C.POINTER(C.c_int), _I, C.POINTER(C.c_int),
+                                        C.POINTER(C.c_int), C.POINTER(C.c_int), _I, C.POINTER(C.c_int)]),
     "cmwg_selftest_tc_gemm": (_I, [_VP, _VP, _VP, _I, _I, _I, _I, _I, _VP]),
 }
 

@@ -1,15 +1,17 @@
-"""Command line of the harness: ``python -m constant_memory_waveglow_b200.cli {train,synth} ...``.
+"""Command line of the harness: ``python -m constant_memory_waveglow_b200.cli {train,synth,synth-batch} ...``.
 
 The reference's own ``train.py`` runs unchanged on the ``pytorch_lightning`` / ``model`` / ``datasets`` shims at the
 repository root; its ``inference.py`` cannot in this image (``torchaudio.load`` / ``save`` need the absent TorchCodec),
 so the two entry points exist here with the reference's flags (``train.py:81-93``, ``inference.py:62-70``) on top of the
-RIFF reader/writer of ``datasets.py``.  Multi-GPU: launch ``train`` under ``torchrun --nproc-per-node N``.
+RIFF reader/writer of ``datasets.py``.  Multi-GPU: launch ``train`` under ``torchrun --nproc-per-node N``.  ``synth-batch``
+re-synthesises many files, batching utterances of different lengths into one call each (``WaveGlow.infer(lengths=...)``).
 """
 from __future__ import annotations
 
 import argparse
 import json
 import math
+import os
 import sys
 
 import torch
@@ -97,11 +99,71 @@ def synth(argv) -> None:
     wav_write(args.outfile, x.reshape(1, -1), sr)
 
 
+def _load_for_synthesis(ckpt: str):
+    lit = TR.LightModel.load_from_checkpoint(ckpt, map_location="cpu")
+    model, conditioner = lit.model, lit.conditioner
+    model.apply(remove_weight_norms)
+    dev = torch.device("cuda")
+    return model.to(dev).eval(), conditioner.to(dev), dev
+
+
+def item_noise(seed: int, index: int, n: int, sigma: float) -> torch.Tensor:
+    """The noise of file `index` (command-line order) of a synth-batch run: N(0, sigma^2), n samples, from a CPU generator
+    seeded by (seed, index) alone -- a rerun reproduces every file whatever the batching."""
+    g = torch.Generator().manual_seed(int(seed) * 1_000_003 + int(index))
+    return torch.randn(n, generator=g) * sigma
+
+
+def synth_batch(argv) -> None:
+    p = argparse.ArgumentParser(prog="cli synth-batch",
+                                description="analysis + synthesis of many files, batched by length (one output per input)")
+    p.add_argument("ckpt", type=str)
+    p.add_argument("outdir", type=str)
+    p.add_argument("infiles", type=str, nargs="+")
+    p.add_argument("-s", "--sigma", type=float, default=0.6)
+    p.add_argument("--max-batch", type=int, default=16, help="utterances per synthesis call")
+    p.add_argument("--seed", type=int, default=0, help="noise seed; file i draws from a generator seeded by (seed, i)")
+    args = p.parse_args(argv)
+    if args.max_batch < 1:
+        p.error("--max-batch must be >= 1")
+    stems = [os.path.splitext(os.path.basename(f))[0] for f in args.infiles]
+    if len(set(stems)) != len(stems):
+        p.error("input files must have distinct names: outputs are written as OUTDIR/<name>.wav")
+    model, conditioner, dev = _load_for_synthesis(args.ckpt)
+    from .base import pad_batch
+    from .datasets import wav_info
+    os.makedirs(args.outdir, exist_ok=True)
+    hop = model._hop_length
+    conds, rates = [], []
+    with torch.no_grad():
+        for f in args.infiles:
+            rates.append(wav_info(f).sample_rate)
+            conds.append(conditioner(wav_read(f).mean(0, keepdim=True).to(dev))[0])
+        order = sorted(range(len(conds)), key=lambda i: conds[i].shape[-1])
+        total, cost = 0, 0.0
+        for s0 in range(0, len(order), args.max_batch):
+            idx = order[s0:s0 + args.max_batch]
+            h, frames = pad_batch([conds[i] for i in idx])
+            z = torch.zeros((len(idx), h.shape[-1] * hop))
+            for j, i in enumerate(idx):
+                z[j, :frames[j] * hop] = item_noise(args.seed, i, frames[j] * hop, args.sigma)
+            z = z.to(dev)
+            x, dt = _timed(lambda: model.infer(h, args.sigma, z=z, lengths=frames))
+            cost += dt
+            for j, i in enumerate(idx):
+                n = frames[j] * hop
+                total += n
+                wav_write(os.path.join(args.outdir, stems[i] + ".wav"), x[j, :n].reshape(1, -1).cpu(), rates[i])
+    print("{} files, {} samples, synthesis {:.4f} s, {:.4f} kHz".format(len(conds), total, cost, total / max(cost, 1e-9) / 1e3))
+
+
 def main(argv=None) -> None:
     argv = list(sys.argv[1:] if argv is None else argv)
-    if not argv or argv[0] not in ("train", "synth"):
-        raise SystemExit("usage: python -m constant_memory_waveglow_b200.cli {train,synth} [flags]  (-h after the verb)")
-    (train if argv[0] == "train" else synth)(argv[1:])
+    verbs = {"train": train, "synth": synth, "synth-batch": synth_batch}
+    if not argv or argv[0] not in verbs:
+        raise SystemExit("usage: python -m constant_memory_waveglow_b200.cli {train,synth,synth-batch} [flags]  "
+                         "(-h after the verb)")
+    verbs[argv[0]](argv[1:])
 
 
 if __name__ == "__main__":

@@ -42,6 +42,7 @@ struct GemmDesc {
   int bn;         // N tile (tc engine)
   int is_fp16;
   int tag;        // CMWG_KCLASS_* for the profiler
+  const int* row_len;  // nullptr, or per-item lengths (1-D WN): the epilogue writes 0 at rows t >= row_len[b] (tc engine)
 };
 
 struct FfGemmParams {

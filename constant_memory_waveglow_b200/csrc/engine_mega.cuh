@@ -100,7 +100,31 @@ struct alignas(64) MegaParams {
   const float* w_end;           // [MEGA_END_MAXC][Cs] fp32, rows >= cout zero
   int cout;
   int store_skip;               // also keep the fp32 cumulative skip slab (training: the `end` weight gradient reads it)
+  // Per-item lengths (cmwg_wn_forward_varlen).  rt_tab == nullptr: every item has tiles_per_batch row tiles and row tile rt is
+  // (rt / tiles_per_batch, rt % tiles_per_batch).  Otherwise rt_tab[rt] = (item, tile within the item, tiles of the item): the
+  // list holds only the tiles that contain valid rows.  row_len != nullptr: the residual epilogues write 0 at rows
+  // t >= row_len[item], so every layer input is zero past the item's end, as the TMA zero fill leaves it for a call of that length.
+  const int4* rt_tab;
+  const int* row_len;
 };
+
+struct MegaTile {
+  int b, tb, ntb;   // batch item, row tile within it, row tiles of the item
+};
+__host__ __device__ __forceinline__ MegaTile mega_tile(const int4* tab, int tiles_per_batch, int rt) {
+  MegaTile m;
+  if (tab != nullptr) {
+    const int4 e = tab[rt];
+    m.b = e.x; m.tb = e.y; m.ntb = e.z;
+  } else {
+    m.b = rt / tiles_per_batch; m.tb = rt - m.b * tiles_per_batch; m.ntb = tiles_per_batch;
+  }
+  return m;
+}
+// row `trow` of item b lies past the item's end: its residual output is 0 (a select: the accumulator there may be anything)
+__device__ __forceinline__ bool mega_dead_row(const int* row_len, int b, int trow) {
+  return row_len != nullptr && trow >= __ldg(row_len + b);
+}
 
 __device__ __forceinline__ uint32_t ld_acquire_u32(const uint32_t* p) {
   uint32_t v;
@@ -213,7 +237,8 @@ __device__ __forceinline__ void mega_epilogue_task(const Epi& epi, uint32_t tmem
                                                    uint32_t tmem_empty_remote, int q, int cg, int lane, uint32_t wbuf,
                                                    uint64_t* ibar, uint32_t& it, const CUtensorMap* om0,
                                                    const CUtensorMap* om1, const CUtensorMap* om2, const CUtensorMap* im0,
-                                                   const CUtensorMap* im1, int b, int r0, int cbase, MegaSig sig, MegaSig* prev, int dbg, uint32_t* tt) {
+                                                   const CUtensorMap* im1, int b, int r0, int cbase, MegaSig sig, MegaSig* prev, int dbg, uint32_t* tt,
+                                                   bool dead = false) {
   constexpr int NCH = GW / 128;                      // 32-column chunks per warp
   constexpr int OUTW = Epi::kOutF32 ? 16 : 8;
   constexpr int OCH = Epi::kOutF32 ? TC_CHUNK32_BYTES : TC_CHUNK16_BYTES;
@@ -281,6 +306,12 @@ __device__ __forceinline__ void mega_epilogue_task(const Epi& epi, uint32_t tmem
         } else {
           epi.compute(c0 + 16 * h, v, o);
         }
+      }
+      if (dead) {   // this lane's row is past its item's end (per-item lengths)
+#pragma unroll
+        for (int i = 0; i < Epi::kOut; ++i)
+#pragma unroll
+          for (int j = 0; j < OUTW; ++j) o[i][j] = 0u;
       }
 #pragma unroll
       for (int i = 0; i < NST; ++i) {
@@ -404,7 +435,8 @@ __device__ __forceinline__ void mega_inplace_direct(const Epi& epi, uint32_t tad
 // warp's two staging buffers (one mbarrier phase); each chunk is updated in place and stored.
 __device__ __forceinline__ void mega_res1_task(const AddTcEpi& epi, uint32_t tmem_tile, uint64_t* tmem_full, uint32_t full_phase,
                                                uint32_t tmem_empty_remote, int q, int cg, int lane, uint32_t wbuf, uint64_t* ibar,
-                                               uint32_t& it, const CUtensorMap* om, int b, int r0, MegaSig sig, uint32_t* tt) {
+                                               uint32_t& it, const CUtensorMap* om, int b, int r0, MegaSig sig, uint32_t* tt,
+                                               bool dead = false) {
   const uint32_t taddr = tmem_tile + ((uint32_t)(q * 32) << 16) + cg * (MEGA_BN / 4);
   const uint32_t c_a = (uint32_t)clock();
   mbar_wait(tmem_full, full_phase);
@@ -432,6 +464,10 @@ __device__ __forceinline__ void mega_res1_task(const AddTcEpi& epi, uint32_t tme
 #pragma unroll
       for (int j = 0; j < 8; ++j) inh[0][j] = in[8 * h + j];
       epi.compute(c0 + 16 * h, v, inh, o);
+      if (dead) {
+#pragma unroll
+        for (int j = 0; j < 8; ++j) o[0][j] = 0u;
+      }
       stage_store16h(buf, lane, h, o[0]);
     }
     fence_proxy_async();
@@ -544,7 +580,8 @@ constexpr size_t mega_smem_bytes() {
   return (size_t)mega_stages<SAVE>() * MEGA_STAGE_BYTES + TC_EPI_WARPS * mega_warp_bytes<SAVE>() + TC_BAR_BYTES + 1024;
 }
 
-template <bool SAVE>
+// VARLEN: per-item lengths (rt_tab / row_len set); a separate instance, so the dense kernel carries none of it
+template <bool SAVE, bool VARLEN = false>
 __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __grid_constant__ MegaParams p) {
   extern __shared__ uint8_t smem_raw[];
   constexpr int STAGES = mega_stages<SAVE>();
@@ -594,7 +631,8 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
       for (int task = pair; task < p.total_tasks; task += npairs) {
         const MegaTask t = mega_decode(p, task);
         if (t.type == MEGA_NONE) continue;
-        const int b = t.rt / p.tiles_per_batch, tb = t.rt - b * p.tiles_per_batch;
+        const MegaTile mt = mega_tile(VARLEN ? p.rt_tab : nullptr, p.tiles_per_batch, t.rt);
+        const int b = mt.b, tb = mt.tb;
         const int t0 = tb * (2 * TC_BM) + rank * TC_BM;
         const int nrow = rank * (MEGA_BN / 2);
         const long long cf = clock64();
@@ -603,7 +641,7 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
         } else if (t.type == MEGA_G) {
           if (t.layer > 0 && !(p.dbg & 1)) {
             const uint32_t* f1 = mega_rflag(p, t.layer - 1, t.rt);
-            mega_wait_flags3(tb > 0 ? f1 - 1 : f1, f1, tb + 1 < p.tiles_per_batch ? f1 + 1 : f1, rtarget, !(p.dbg & 32));
+            mega_wait_flags3(tb > 0 ? f1 - 1 : f1, f1, tb + 1 < mt.ntb ? f1 + 1 : f1, rtarget, !(p.dbg & 32));
             if (!(p.dbg & 16)) fence_proxy_async_all();
           }
         } else {
@@ -648,9 +686,9 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
         if (t.type == MEGA_NONE) continue;
         if (t.type == MEGA_G) {
           if (t.layer > 0) {
-            const int tb = t.rt % p.tiles_per_batch;
+            const MegaTile mt = mega_tile(VARLEN ? p.rt_tab : nullptr, p.tiles_per_batch, t.rt);
             const uint32_t* f1 = mega_rflag(p, t.layer - 1, t.rt);
-            mega_wait_flags3(tb > 0 ? f1 - 1 : f1, f1, tb + 1 < p.tiles_per_batch ? f1 + 1 : f1, rtarget);
+            mega_wait_flags3(mt.tb > 0 ? f1 - 1 : f1, f1, mt.tb + 1 < mt.ntb ? f1 + 1 : f1, rtarget);
           }
         } else {
           mega_wait_flag(mega_gflag(p, t.type == MEGA_R ? t.layer : p.depth - 1, t.rt), gtarget);
@@ -758,8 +796,10 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
     for (int task = pair; task < p.total_tasks; task += npairs) {
       const MegaTask t = mega_decode(p, task);
       if (t.type == MEGA_NONE) continue;
-      const int b = t.rt / p.tiles_per_batch, tb = t.rt - b * p.tiles_per_batch;
+      const MegaTile mt = mega_tile(VARLEN ? p.rt_tab : nullptr, p.tiles_per_batch, t.rt);
+      const int b = mt.b, tb = mt.tb;
       const int r0 = tb * (2 * TC_BM) + rank * TC_BM + q * 32;
+      const bool dead = VARLEN && mega_dead_row(p.row_len, b, r0 + lane);
       const uint32_t tile = tmem_base + acc * MEGA_BN;
       const uint32_t te = tmem_empty_addr + 8 * acc;
       const uint32_t dcnt = smem_u32(done_cnt + (seq & 3));
@@ -803,7 +843,7 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
         // h_1 = W_res g_0 + W_start x_a, all of it from the tensor core: nothing to load, one 16-bit stream to store
         mega_epilogue_task<RoundTcEpi, MEGA_BN>(round_epi, tile, &s.tmem_full[acc], acc_phase, te, q, cg, lane, wbuf, ibar, it,
                                                 &p.hi_c16[1], nullptr, nullptr, nullptr, nullptr, b, r0, 0,
-                                                MegaSig{mega_rflag(p, 0, t.rt), dcnt}, prev, p.dbg, tt + 4);
+                                                MegaSig{mega_rflag(p, 0, t.rt), dcnt}, prev, p.dbg, tt + 4, dead);
       } else if (t.type == MEGA_R && !p.res_lo) {
         if (lane == 0) {  // the warp's whole share of the layer input (two chunks), ahead of the accumulator
           mega_wait_flag(mega_gflag(p, t.layer, t.rt), gtarget);  // implies R(layer-1, rt) is complete
@@ -815,7 +855,7 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
         }
         __syncwarp();
         mega_res1_task(add_epi, tile, &s.tmem_full[acc], acc_phase, te, q, cg, lane, wbuf, ibar, it, &p.hi_c16[t.layer + 1], b, r0,
-                       MegaSig{mega_rflag(p, t.layer, t.rt), dcnt}, tt + 4);
+                       MegaSig{mega_rflag(p, t.layer, t.rt), dcnt}, tt + 4, dead);
       } else if (t.type == MEGA_R) {
         if (lane == 0) {  // chunk 0 of the layer input's (hi, lo) pair, ahead of the accumulator
           if (!(p.dbg & 1)) mega_wait_flag(mega_gflag(p, t.layer, t.rt), gtarget);  // implies R(layer-1, rt) is complete
@@ -829,7 +869,7 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
         mega_epilogue_task<SplitTcEpi<true>, MEGA_BN>(split_epi, tile, &s.tmem_full[acc], acc_phase, te, q, cg, lane, ubuf, ibar,
                                                       it, &p.hi_c16[t.layer + 1], &p.lo_c16[t.layer + 1], nullptr,
                                                       &p.hi_c16[t.layer], &p.lo_c16[t.layer], b, r0, 0,
-                                                      MegaSig{mega_rflag(p, t.layer, t.rt), dcnt}, prev, p.dbg, tt + 4);
+                                                      MegaSig{mega_rflag(p, t.layer, t.rt), dcnt}, prev, p.dbg, tt + 4, dead);
       } else if (p.lst != nullptr) {
         if (p.lagged) {   // staging is about to be used as plain memory: no store may still be reading it
           if (lane == 0) bulk_wait_read<0>();

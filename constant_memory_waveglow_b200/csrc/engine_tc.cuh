@@ -73,6 +73,7 @@ struct alignas(64) TcGemmParams {
   int h0, nh;                   // line window [h0, h0 + nh) of every batch item (nh = H: all lines)
   uint32_t idesc;
   uint32_t desc_lbo, desc_sbo;  // >>4 encoded; overridable by the self test
+  const int* row_len;           // GemmDesc::row_len
 };
 
 struct alignas(64) TcWgradParams {
@@ -588,6 +589,12 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_gemm_kernel(const __grid_con
               epi.compute(c0 + 16 * h, v, o);
             }
           }
+          if (p.row_len != nullptr && r0 + lane >= __ldg(p.row_len + b)) {   // past the item's end: select 0
+#pragma unroll
+            for (int i = 0; i < Epi::kOut; ++i)
+#pragma unroll
+              for (int j = 0; j < OUTW; ++j) o[i][j] = 0u;
+          }
 #pragma unroll
           for (int i = 0; i < Epi::kOut; ++i) {
             if constexpr (Epi::kOutF32) stage_store32h(obuf + i * ET::kOutChunk, lane, h, o[i]);
@@ -828,6 +835,8 @@ int tc_gemm_launch_bn(const GemmDesc& d, const TcIo& io, const Epi& epi, cudaStr
   p.idesc = make_idesc(d.is_fp16, 2 * TC_BM, BN, 0, 0);
   p.desc_lbo = lbo_override >= 0 ? (uint32_t)lbo_override : 1u;
   p.desc_sbo = sbo_override >= 0 ? (uint32_t)sbo_override : (1024u >> 4);
+  CMWG_REQUIRE(d.row_len == nullptr || H == 1, "tc_gemm: per-item lengths need the 1-D layout");
+  p.row_len = d.row_len;
   if (p.total_tiles == 0) return CMWG_OK;
   auto kern = tc_gemm_kernel<BN, Epi>;
   constexpr size_t smem = tc_smem_bytes<BN, Epi>();

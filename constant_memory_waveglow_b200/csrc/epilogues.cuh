@@ -141,6 +141,8 @@ struct ResSkipEpi {
   float* skip;           // [rows][Cs] fp32 cumulative skip
   const float* bias;     // nullptr or [nb]
   int Cr, Cs, cr_eff, first_layer, f16;
+  const int* row_len;    // nullptr, or per-item lengths: the residual output is 0 at rows t >= row_len[b] (row = b * T + t)
+  int T;
   template <int NC>
   __device__ __forceinline__ void load(long long row, int col0, float (&aux)[NC]) const {
     if (col0 < cr_eff) {
@@ -163,6 +165,13 @@ struct ResSkipEpi {
 #pragma unroll
     for (int j = 0; j < NC; ++j) w[j] = v[j] + aux[j] + (bias ? bias[col0 + j] : 0.f);
     if (col0 < cr_eff) {
+      if (row_len != nullptr) {
+        const long long b = row / T;
+        if (row - b * T >= __ldg(row_len + b)) {
+#pragma unroll
+          for (int j = 0; j < NC; ++j) w[j] = 0.f;
+        }
+      }
       long long o = row * Cr + col0;
       if (res_dst32) store_f32<NC>(res_dst32 + o, w);
       if (res_dst_op) store_ops<OpT, NC>(res_dst_op + o, w, f16);

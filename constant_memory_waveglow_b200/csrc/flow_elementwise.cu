@@ -465,7 +465,9 @@ __global__ void __launch_bounds__(256) coupling_apply_kernel(const float* __rest
                                                              const float* __restrict__ lst,
                                                              float* __restrict__ z, long long z_bs,
                                                              float* __restrict__ neg_ls, int cin, int T,
-                                                             int inverse, long long total) {
+                                                             int inverse, long long total,
+                                                             const int* __restrict__ len = nullptr) {
+  // len != nullptr: columns t >= len[b] of z and neg_ls are written as 0 (a select: the flow state there may be non-finite)
   // idx enumerates (b, j, t/VEC)
   int nv = T / VEC;
   for (long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x; idx < total;
@@ -495,6 +497,12 @@ __global__ void __launch_bounds__(256) coupling_apply_kernel(const float* __rest
       float e = expf(l[v]);
       o[v] = inverse ? (bb[v] - s[v]) / e : fmaf(bb[v], e, s[v]);
       nl[v] = -l[v];
+    }
+    if (len != nullptr) {
+      const int lb = __ldg(len + b);
+#pragma unroll
+      for (int v = 0; v < VEC; ++v)
+        if (t + v >= lb) a[v] = o[v] = nl[v] = 0.f;
     }
     if (VEC == 4) {
       *reinterpret_cast<float4*>(za) = make_float4(a[0], a[1 % VEC], a[2 % VEC], a[3 % VEC]);
@@ -626,6 +634,29 @@ __global__ void __launch_bounds__(1024) logdet_accumulate_kernel(const float* __
   for (; i < N; i += 1024) s0 += p[i];
   const float s = block_sum_1024((s0 + s1) + (s2 + s3), red);
   if (threadIdx.x == 0) out[b] = ((prev ? prev[b] : 0.f) + (ldw ? *ldw : 0.f)) + s;
+}
+
+// per-item lengths: out[b] = prev[b] + *ldw * len[b] + sum over channels c < C and columns t < len[b] of a[b, c, t].
+// The valid (C, n) block is walked as the contiguous C * n tensor logdet_accumulate_kernel sums for the item alone, in the same
+// order, and ldw * n is the `logdet * T` of that call: the result is bit-identical to it.
+__global__ void __launch_bounds__(1024) logdet_accumulate_varlen_kernel(const float* __restrict__ a, long long a_bs, int C,
+                                                                        int T, const int* __restrict__ len,
+                                                                        const float* __restrict__ prev,
+                                                                        const float* __restrict__ ldw, float* __restrict__ out) {
+  __shared__ float red[32];
+  const int b = blockIdx.x;
+  const int n = min(max(len[b], 0), T);
+  const int N = C * n;
+  const float* p = a + b * a_bs;
+  auto at = [&](int i) { const int c = i / n; return p[(long long)c * T + (i - c * n)]; };
+  float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
+  int i = threadIdx.x;
+  for (; i + 3 * 1024 < N; i += 4 * 1024) {
+    s0 += at(i); s1 += at(i + 1024); s2 += at(i + 2048); s3 += at(i + 3072);
+  }
+  for (; i < N; i += 1024) s0 += at(i);
+  const float s = block_sum_1024((s0 + s1) + (s2 + s3), red);
+  if (threadIdx.x == 0) out[b] = ((prev ? prev[b] : 0.f) + (ldw ? *ldw * (float)n : 0.f)) + s;
 }
 
 __global__ void __launch_bounds__(1024) nll_rows_kernel(const float* __restrict__ z, int T, float* __restrict__ rows) {
@@ -841,6 +872,29 @@ int cmwg_coupling_apply(const float* x, long long x_bstride, const float* lst, f
   return CMWG_OK;
 }
 
+int cmwg_coupling_apply_varlen(const float* x, long long x_bstride, const float* lst, float* z, long long z_bstride,
+                               float* neg_log_s, int B, int cin, int T, const int* lengths_dev, int inverse, void* stream) {
+  CMWG_REQUIRE(lengths_dev, "cmwg_coupling_apply_varlen: null lengths");
+  if (B == 0 || T == 0 || cin == 0) return CMWG_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  bool vec = (T % 4 == 0) && (x_bstride % 4 == 0) && (z_bstride % 4 == 0) && (((uintptr_t)x & 15) == 0) &&
+             (((uintptr_t)z & 15) == 0) && (((uintptr_t)lst & 15) == 0) && (((uintptr_t)neg_log_s & 15) == 0);
+  if (vec) {
+    long long total = (long long)B * cin * (T / 4);
+    int blocks = (int)std::min<long long>(ceil_div_ll(total, 256), (long long)num_sms() * 8);
+    coupling_apply_kernel<4><<<blocks, 256, 0, st>>>(x, x_bstride, lst, z, z_bstride, neg_log_s, cin, T, inverse, total,
+                                                     lengths_dev);
+  } else {
+    long long total = (long long)B * cin * T;
+    int blocks = (int)std::min<long long>(ceil_div_ll(total, 256), (long long)num_sms() * 8);
+    coupling_apply_kernel<1><<<blocks, 256, 0, st>>>(x, x_bstride, lst, z, z_bstride, neg_log_s, cin, T, inverse, total,
+                                                     lengths_dev);
+  }
+  CMWG_COUNT_LAUNCH();
+  CMWG_LAUNCH_CHECK();
+  return CMWG_OK;
+}
+
 int cmwg_coupling_bwd(const float* out, long long out_bstride, const float* lst, const float* dout,
                       long long dout_bstride, const float* dls, long long dls_bstride, float* restored, float* dlst,
                       float* din, int B, int cin, int T, int inverse, void* stream) {
@@ -880,6 +934,16 @@ int cmwg_logdet_accumulate(const float* a, long long a_bstride, int B, int N, co
   CMWG_REQUIRE(a && out, "cmwg_logdet_accumulate: null argument");
   if (B == 0) return CMWG_OK;
   logdet_accumulate_kernel<<<B, 1024, 0, (cudaStream_t)stream>>>(a, a_bstride, N, prev, log_det_w, out);
+  CMWG_COUNT_LAUNCH();
+  CMWG_LAUNCH_CHECK();
+  return CMWG_OK;
+}
+
+int cmwg_logdet_accumulate_varlen(const float* a, long long a_bstride, int B, int C, int T, const int* lengths_dev,
+                                  const float* prev, const float* log_det_w, float* out, void* stream) {
+  CMWG_REQUIRE(a && out && lengths_dev, "cmwg_logdet_accumulate_varlen: null argument");
+  if (B == 0) return CMWG_OK;
+  logdet_accumulate_varlen_kernel<<<B, 1024, 0, (cudaStream_t)stream>>>(a, a_bstride, C, T, lengths_dev, prev, log_det_w, out);
   CMWG_COUNT_LAUNCH();
   CMWG_LAUNCH_CHECK();
   return CMWG_OK;

@@ -577,10 +577,10 @@ static __global__ void __launch_bounds__(256) foldend_dw_kernel(const FoldEndDwP
 }
 
 // taps of x_a into the padding columns of the conditioning slab: ycl[row][aux + tap * cin + c] = x[b][c][t + (tap - centre)]
-// (zero outside [0, T): the dilated conv's 'same' padding of h_0 = W_start x_a, which has no bias here)
+// (zero outside [0, T), or [0, row_len[b]): the dilated conv's 'same' padding of h_0 = W_start x_a, which has no bias here)
 static __global__ void __launch_bounds__(256) cond_aug_kernel(const float* __restrict__ x, long long x_bs, int cin, int R,
                                                               int B, int T, uint16_t* __restrict__ ycl, int aux, int auxp,
-                                                              int is_fp16) {
+                                                              int is_fp16, const int* __restrict__ row_len) {
   pdl_trigger();
   pdl_wait();
   const long long rows = (long long)B * T;
@@ -591,7 +591,8 @@ static __global__ void __launch_bounds__(256) cond_aug_kernel(const float* __res
     const int j = (int)(idx / rows), tap = j / cin, c = j % cin;
     const int b = (int)(row / T), t = (int)(row - (long long)b * T);
     const int ts = t + tap - ct;
-    const float v = (ts >= 0 && ts < T) ? x[b * x_bs + (long long)c * T + ts] : 0.f;
+    const int tv = row_len ? row_len[b] : T;   // per-item lengths: x_a is zero from the item's end on, as past T
+    const float v = (ts >= 0 && ts < tv) ? x[b * x_bs + (long long)c * T + ts] : 0.f;
     ycl[row * auxp + aux + j] = f32_to_op16(v, is_fp16);
   }
 }
@@ -710,8 +711,10 @@ static __global__ void __launch_bounds__(256) smallk_to_slab_kernel(const float*
                                                                     int T, int blocks_per_batch, int t_off,
                                                                     int t_end, float* __restrict__ o32,
                                                                     OpT* __restrict__ ohi, OpT* __restrict__ olo,
-                                                                    int is_fp16, const float* __restrict__ gscale) {
-  // rows [t_off, t_end) of every batch item are computed; T stays the row count of one item (strides)
+                                                                    int is_fp16, const float* __restrict__ gscale,
+                                                                    const int* __restrict__ row_len) {
+  // rows [t_off, t_end) of every batch item are computed; T stays the row count of one item (strides).  row_len != nullptr:
+  // rows t >= row_len[b] are written as 0 (bias included), so the slab is zero past the item's end
   extern __shared__ float sm[];
   pdl_trigger();
   pdl_wait();
@@ -720,6 +723,7 @@ static __global__ void __launch_bounds__(256) smallk_to_slab_kernel(const float*
   float* wsm = sm + K * SMALLK_ROWS;   // [K][C]  (k-major: 4 consecutive outputs are one float4)
   const int b = blockIdx.x / blocks_per_batch;
   const int t0 = t_off + (blockIdx.x % blocks_per_batch) * SMALLK_ROWS;
+  const int t_live = row_len ? row_len[b] : t_end;
   for (int idx = threadIdx.x; idx < K * SMALLK_ROWS; idx += 256) {
     int i = idx / SMALLK_ROWS, r = idx % SMALLK_ROWS;
     int t = t0 + r;
@@ -761,6 +765,10 @@ static __global__ void __launch_bounds__(256) smallk_to_slab_kernel(const float*
               for (int j = 0; j < 8; ++j) acc[j] = fmaf(wr[i][j], xv, acc[j]);
             }
           }
+          if (t >= t_live) {
+#pragma unroll
+            for (int j = 0; j < 8; ++j) acc[j] = 0.f;
+          }
           const long long off = ((long long)b * T + t) * C + o;
           uint32_t h[4], l[4];
 #pragma unroll
@@ -791,6 +799,10 @@ static __global__ void __launch_bounds__(256) smallk_to_slab_kernel(const float*
           acc[4] = fmaf(w1.x, xv, acc[4]); acc[5] = fmaf(w1.y, xv, acc[5]);
           acc[6] = fmaf(w1.z, xv, acc[6]); acc[7] = fmaf(w1.w, xv, acc[7]);
         }
+        if (t >= t_live) {
+#pragma unroll
+          for (int j = 0; j < 8; ++j) acc[j] = 0.f;
+        }
         const long long off = ((long long)b * T + t) * C + o;
         uint32_t h[4], l[4];
 #pragma unroll
@@ -819,6 +831,7 @@ static __global__ void __launch_bounds__(256) smallk_to_slab_kernel(const float*
       acc[0] = fmaf(w.x, xv, acc[0]); acc[1] = fmaf(w.y, xv, acc[1]);
       acc[2] = fmaf(w.z, xv, acc[2]); acc[3] = fmaf(w.w, xv, acc[3]);
     }
+    if (t >= t_live) acc[0] = acc[1] = acc[2] = acc[3] = 0.f;
     const long long off = ((long long)b * T + t) * C + o;
     if (o32) *reinterpret_cast<float4*>(o32 + off) = make_float4(acc[0], acc[1], acc[2], acc[3]);
     if constexpr (sizeof(OpT) == 4) {
@@ -842,7 +855,7 @@ static __global__ void __launch_bounds__(256) smallk_to_slab_kernel(const float*
 template <typename OpT>
 static int smallk_to_slab(const float* in, long long in_bs, const float* W, int so, int si, const float* bias, int K,
                           int C, int B, int T, float* o32, OpT* ohi, OpT* olo, int is_fp16, cudaStream_t st,
-                          int t_off = 0, int t_n = -1, const float* gscale = nullptr) {
+                          int t_off = 0, int t_n = -1, const float* gscale = nullptr, const int* row_len = nullptr) {
   if (t_n < 0) t_n = T - t_off;
   const int bpb = ceil_div(t_n, SMALLK_ROWS);
   if (B * bpb == 0) return CMWG_OK;
@@ -850,7 +863,7 @@ static int smallk_to_slab(const float* in, long long in_bs, const float* W, int 
   if (smem > 48 * 1024)
     CMWG_CHECK_CUDA(cudaFuncSetAttribute(smallk_to_slab_kernel<OpT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   CMWG_CHECK_CUDA(launch_pdl(smallk_to_slab_kernel<OpT>, dim3(B * bpb), dim3(256), smem, st, in, in_bs, W, so, si, bias, K,
-                             C, T, bpb, t_off, t_off + t_n, o32, ohi, olo, is_fp16, gscale));
+                             C, T, bpb, t_off, t_off + t_n, o32, ohi, olo, is_fp16, gscale, row_len));
   CMWG_COUNT_LAUNCH();
   CMWG_LAUNCH_CHECK();
   return CMWG_OK;

@@ -176,6 +176,29 @@ static inline size_t line_state_slab_bytes(const WnDims& d, int B, int T) {
   return align_up((size_t)B * d.H * T * d.Cr * d.opsize, 1024);
 }
 
+// Per-item lengths of a padded batch (cmwg_wn_forward_varlen): item b has valid rows [0, len[b]).  `host` plans the task
+// kernel's list (only row tiles that hold valid rows); `dev` (the same values, on the device) drives the masks that keep every
+// layer input zero from row len[b] on -- what the TMA zero fill gives a call of length len[b].
+struct VarLen {
+  const int* host = nullptr;
+  const int* dev = nullptr;
+  bool on() const { return dev != nullptr; }
+};
+
+// row-tile table of the task kernel for per-item lengths (MegaParams::rt_tab), in the workspace behind the layouts
+static inline size_t varlen_tab_offset(const WnDims& d, int B, int T) {
+  FwdLayout FL;
+  make_fwd_layout(d, B, T, &FL);
+  BwdLayout BL;
+  make_bwd_layout(d, B, T, &BL);
+  return align_up(FL.ws_total > BL.total ? FL.ws_total : BL.total, 1024);
+}
+static inline int varlen_row_tiles(const int* len, int B) {
+  int rt = 0;
+  for (int b = 0; b < B; ++b) rt += ceil_div(len[b], 2 * TC_BM);
+  return rt;
+}
+
 
 // ------------------------------------------------------------------------------------------------
 // single-kernel forward (engine_mega.cuh): every gate / residual / skip GEMM tile of the WN as one task list
@@ -260,9 +283,9 @@ static inline bool mega_shapes_ok(const WnDims& d, int B, int T) {
          B >= 1 && T >= 1;
 }
 
-template <bool SAVE>
+template <bool SAVE, bool VARLEN = false>
 static int mega_launch(const MegaParams& p, cudaStream_t st) {
-  auto kern = wn_fwd_mega_kernel<SAVE>;
+  auto kern = wn_fwd_mega_kernel<SAVE, VARLEN>;
   constexpr size_t smem = mega_smem_bytes<SAVE>();
   static_assert(smem <= TC_SMEM_LIMIT, "shared memory budget exceeded");
   static bool attr_set = false;
@@ -284,9 +307,39 @@ static inline bool mega_end_fused(const WnDims& d) {  // CMWG_MEGA_END=0: separa
   return !(e && e[0] == '0') && 2 * d.cin <= MEGA_END_MAXC && !d.bias && d.Cs == MEGA_BN;
 }
 
+// tab[rt] = (item, tile within the item, tiles of the item) for the RT row tiles of per-item lengths len (clamped to [1, T]:
+// a device copy that disagrees with the planning copy must not index outside the slabs)
+static __global__ void varlen_tiles_kernel(const int* __restrict__ len, int B, int T, int RT, int4* __restrict__ tab) {
+  const int rt = blockIdx.x * blockDim.x + threadIdx.x;
+  if (rt >= RT) return;
+  int start = 0;
+  for (int b = 0; b < B; ++b) {
+    const int n = (min(max(len[b], 1), T) + 2 * TC_BM - 1) / (2 * TC_BM);
+    if (rt < start + n || b == B - 1) {
+      const int tb = min(rt - start, n - 1);
+      tab[rt] = make_int4(b, tb, n, 0);
+      return;
+    }
+    start += n;
+  }
+}
+
+// rows [end, min(T, end + rows)) of item blockIdx.x, end = its last row tile's end, zeroed in slab blockIdx.y (a or b)
+static __global__ void varlen_zero_tail_kernel(const int* __restrict__ len, int T, int rows, int C, uint16_t* a, uint16_t* b) {
+  const int item = blockIdx.x;
+  const int end = (min(max(len[item], 1), T) + 2 * TC_BM - 1) / (2 * TC_BM) * (2 * TC_BM);
+  const int n = min(T, end + rows) - end;
+  if (n <= 0) return;
+  uint16_t* slab = blockIdx.y ? b : a;
+  uint4* p = reinterpret_cast<uint4*>(slab + ((size_t)item * T + end) * C);
+  const long long nv = (long long)n * C / 8;
+  for (long long i = threadIdx.x; i < nv; i += blockDim.x) p[i] = make_uint4(0u, 0u, 0u, 0u);
+}
+
 static int wn_forward_mega(const WnDims& d, const PackedLayout& PL, const FwdLayout& FL, const uint8_t* pk, uint8_t* ws,
                            const void* ycl, int B, int T, bool save, bool fold0, int f16, void* const* hin, void* const* hlo,
-                           void* const* gop, void* const* sb, float* skip32, float* lst, cudaStream_t st) {
+                           void* const* gop, void* const* sb, float* skip32, float* lst, cudaStream_t st,
+                           const VarLen& vl = VarLen()) {
   MegaParams p;
   memset(&p, 0, sizeof(p));
   const bool res_lo = fwd_res_lo(d);
@@ -307,6 +360,24 @@ static int wn_forward_mega(const WnDims& d, const PackedLayout& PL, const FwdLay
   p.depth = d.depth; p.B = B; p.T = T;
   p.tiles_per_batch = ceil_div(T, 2 * TC_BM);
   p.RT = B * p.tiles_per_batch;
+  if (vl.on()) {
+    // only the row tiles that hold valid rows are tasks; rt -> (item, tile, tiles of the item) comes from a table on the device
+    int4* tab = reinterpret_cast<int4*>(ws + varlen_tab_offset(d, B, T));
+    p.RT = varlen_row_tiles(vl.host, B);
+    p.rt_tab = tab;
+    p.row_len = vl.dev;
+    varlen_tiles_kernel<<<ceil_div(p.RT, 256), 256, 0, st>>>(vl.dev, B, T, p.RT, tab);
+    CMWG_COUNT_LAUNCH();
+    CMWG_LAUNCH_CHECK();
+    // The taps of the last tile of an item reach up to max_dil rows past it: rows of the slab that no task of this call
+    // writes and that hold whatever an earlier call left in these per-stream slabs.  Zero them in every layer-input slab.
+    const int max_dil = ((d.radix - 1) / 2) << (d.depth - 1);
+    dim3 zg(B, 2);
+    varlen_zero_tail_kernel<<<zg, 256, 0, st>>>(vl.dev, T, max_dil, d.Cr, reinterpret_cast<uint16_t*>(hin[0]),
+                                                reinterpret_cast<uint16_t*>(hin[d.depth > 1 ? 1 : 0]));
+    CMWG_COUNT_LAUNCH();
+    CMWG_LAUNCH_CHECK();
+  }
   p.ngt = d.npadA / MEGA_BN;
   p.taps = d.R; p.kb_h = d.Crp / TC_BK; p.kb_c = d.auxp / TC_BK; p.kb_g = d.Cdp / TC_BK;
   p.Cd = d.Cd; p.f16 = f16;
@@ -370,6 +441,7 @@ static int wn_forward_mega(const WnDims& d, const PackedLayout& PL, const FwdLay
   }
   p.flags = reinterpret_cast<uint32_t*>(ws + FL.flags);
   CMWG_CHECK_CUDA(cudaMemsetAsync(p.flags, 0, (size_t)d.depth * 2 * p.RT * 4, st));
+  if (vl.on()) return mega_launch<false, true>(p, st);   // inference only: no saves
   return save ? mega_launch<true>(p, st) : mega_launch<false>(p, st);
 }
 
@@ -445,7 +517,8 @@ static int wn_backward_mega(const WnDims& d, const PackedLayout& PL, const BwdLa
 
 template <typename OpT>
 static int wn_forward_impl(const WnDims& d, const void* packed, const float* x, long long x_bs, const void* ycl, int B,
-                           int T, void* workspace, void* saved, float* lst, cudaStream_t st, LineWin lw = LineWin()) {
+                           int T, void* workspace, void* saved, float* lst, cudaStream_t st, LineWin lw = LineWin(),
+                           const VarLen& vl = VarLen()) {
   using E = EngineSel<OpT>;
   constexpr bool TC = E::kTc;
   const int f16 = d.prec == CMWG_PREC_FP16;
@@ -491,7 +564,7 @@ static int wn_forward_impl(const WnDims& d, const void* packed, const float* x, 
     const long long n = (long long)B * T * d.R * d.cin;
     const int nb_aug = (int)std::min<long long>(ceil_div_ll(n, 256), 4 * 148 * 8);
     CMWG_CHECK_CUDA(launch_pdl(cond_aug_kernel, dim3(nb_aug), dim3(256), 0, st, x, x_bs, d.cin, d.R, B, T,
-                               reinterpret_cast<uint16_t*>(const_cast<void*>(ycl)), d.aux, d.auxp, f16));
+                               reinterpret_cast<uint16_t*>(const_cast<void*>(ycl)), d.aux, d.auxp, f16, vl.dev));
     CMWG_COUNT_LAUNCH();
     CMWG_LAUNCH_CHECK();
   } else {
@@ -501,7 +574,7 @@ static int wn_forward_impl(const WnDims& d, const void* packed, const float* x, 
     OpT* olo = (TC && fwd_res_lo(d)) ? hlo_op(0) : nullptr;
     CMWG_PROPAGATE(smallk_to_slab<OpT>(x, x_bs, reinterpret_cast<const float*>(pk + PL.wStart), d.cin, 1,
                                        d.bias ? reinterpret_cast<const float*>(pk + PL.biasStart) : nullptr, d.cin,
-                                       d.Cr, B, d.H * T, o32, oop, olo, f16, st, t_off, t_n));
+                                       d.Cr, B, d.H * T, o32, oop, olo, f16, st, t_off, t_n, nullptr, vl.dev));
   }
 
   bool fused = false;
@@ -512,7 +585,7 @@ static int wn_forward_impl(const WnDims& d, const void* packed, const float* x, 
         hin[i] = hin_op(i); hlo[i] = hlo_op(i); gop[i] = g_op(i);
         sb[i] = save ? sv + FL.s_b[i] : nullptr;
       }
-      CMWG_PROPAGATE(wn_forward_mega(d, PL, FL, pk, ws, ycl, B, T, save, fold0, f16, hin, hlo, gop, sb, skip32, lst, st));
+      CMWG_PROPAGATE(wn_forward_mega(d, PL, FL, pk, ws, ycl, B, T, save, fold0, f16, hin, hlo, gop, sb, skip32, lst, st, vl));
       fused = true;
     }
   }
@@ -567,6 +640,7 @@ static int wn_forward_impl(const WnDims& d, const void* packed, const float* x, 
         g.nseg = 1;
         g.w = pk + PL.PB[i]; g.ldw = d.ldPB; g.N = d.Cr; g.n_rows_w = d.nb(i);
         g.B = B; g.T = T; g.H = d.H; g.h0 = lw.h0; g.nh = lw.nh; g.bn = pick_bn(d.Cr); g.is_fp16 = f16; g.tag = CMWG_KCLASS_RESSKIP;
+        g.row_len = vl.dev;
         TcIo io;
         memset(&io, 0, sizeof(io));
         const float* biasB = d.bias ? reinterpret_cast<const float*>(pk + PL.biasB[i]) : nullptr;
@@ -600,6 +674,7 @@ static int wn_forward_impl(const WnDims& d, const void* packed, const float* x, 
       epi.skip = skip32;
       epi.bias = d.bias ? reinterpret_cast<const float*>(pk + PL.biasB[i]) : nullptr;
       epi.Cr = d.Cr; epi.Cs = d.Cs; epi.cr_eff = d.cr_eff(i); epi.first_layer = (i == 0); epi.f16 = f16;
+      epi.row_len = vl.dev; epi.T = T;
       CMWG_PROPAGATE((E::template gemm<false>(g, epi, st)));
     }
   }
@@ -743,7 +818,7 @@ static int wn_backward_impl(const WnDims& d, const cmwg_wn_params* prm, const vo
     const long long n = (long long)B * T * d.R * d.cin;
     const int nb_aug = (int)std::min<long long>(ceil_div_ll(n, 256), 4 * 148 * 8);
     CMWG_CHECK_CUDA(launch_pdl(cond_aug_kernel, dim3(nb_aug), dim3(256), 0, st, x, x_bs, d.cin, d.R, B, T,
-                               reinterpret_cast<uint16_t*>(const_cast<void*>(ycl)), d.aux, d.auxp, f16));
+                               reinterpret_cast<uint16_t*>(const_cast<void*>(ycl)), d.aux, d.auxp, f16, (const int*)nullptr));
     CMWG_COUNT_LAUNCH();
     CMWG_LAUNCH_CHECK();
   }
@@ -1316,6 +1391,67 @@ int cmwg_wn_forward(const cmwg_wn_config* cfg, const void* packed, const float* 
   if (B == 0 || T == 0) return CMWG_OK;
   if (d.tc) return wn_forward_impl<uint16_t>(d, packed, x, x_bstride, ycl, B, T, workspace, saved, lst, (cudaStream_t)stream);
   return wn_forward_impl<float>(d, packed, x, x_bstride, ycl, B, T, workspace, saved, lst, (cudaStream_t)stream);
+}
+
+size_t cmwg_wn_varlen_workspace_bytes(const cmwg_wn_config* cfg, int B, int T) {
+  WnDims d;
+  if (make_dims(cfg, &d) != CMWG_OK || B < 1 || T < 1) return 0;
+  return varlen_tab_offset(d, B, T) + align_up((size_t)B * ceil_div(T, 2 * TC_BM) * sizeof(int4), 1024) + 1024;
+}
+
+int cmwg_wn_forward_varlen(const cmwg_wn_config* cfg, const void* packed, const float* x, long long x_bstride,
+                           const void* ycl, int B, int T, const int* lengths_host, const int* lengths_dev, void* workspace,
+                           float* lst, void* stream) {
+  WnDims d;
+  CMWG_PROPAGATE(make_dims(cfg, &d));
+  CMWG_REQUIRE(packed && x && ycl && workspace && lst && lengths_host && lengths_dev, "cmwg_wn_forward_varlen: null argument");
+  if (B == 0 || T == 0) return CMWG_OK;
+  for (int b = 0; b < B; ++b)
+    CMWG_REQUIRE(lengths_host[b] >= 1 && lengths_host[b] <= T, "cmwg_wn_forward_varlen: length %d of item %d outside [1, %d]",
+                 lengths_host[b], b, T);
+  if (d.H != 1) {
+    set_error("cmwg_wn_forward_varlen: per-item lengths are implemented for the 1-D WN only");
+    return CMWG_ERR_UNSUPPORTED;
+  }
+  if (d.tc && fwd_res_lo(d)) {
+    const char* e = getenv("CMWG_MEGA_RDIRECT");
+    if (e && e[0] == '1' && mega_enabled() && mega_shapes_ok(d, B, T)) {
+      set_error("cmwg_wn_forward_varlen: CMWG_MEGA_RDIRECT=1 residual tiles do not mask rows past an item's end");
+      return CMWG_ERR_UNSUPPORTED;
+    }
+  }
+  VarLen vl;
+  vl.host = lengths_host; vl.dev = lengths_dev;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (d.tc) return wn_forward_impl<uint16_t>(d, packed, x, x_bstride, ycl, B, T, workspace, nullptr, lst, st, LineWin(), vl);
+  return wn_forward_impl<float>(d, packed, x, x_bstride, ycl, B, T, workspace, nullptr, lst, st, LineWin(), vl);
+}
+
+int cmwg_mega_task_list_varlen(int depth, int B, int T, const int* lengths, int* out, int cap, int* total, int* lag, int* tiles,
+                               int tiles_cap, int* row_tiles) {
+  CMWG_REQUIRE(depth >= 1 && depth <= cmwg::MEGA_D && B >= 1 && T >= 1 && lengths && out && total && lag && tiles && row_tiles,
+               "cmwg_mega_task_list_varlen: bad arguments");
+  for (int b = 0; b < B; ++b)
+    CMWG_REQUIRE(lengths[b] >= 1 && lengths[b] <= T, "cmwg_mega_task_list_varlen: length %d of item %d outside [1, %d]",
+                 lengths[b], b, T);
+  cmwg::MegaParams p;
+  memset(&p, 0, sizeof(p));
+  p.depth = depth; p.B = B; p.T = T; p.tiles_per_batch = cmwg::ceil_div(T, 2 * cmwg::TC_BM);
+  p.RT = varlen_row_tiles(lengths, B);
+  p.ngt = 2;
+  p.lag = cmwg::mega_fwd_lag(p.RT);
+  p.total_tasks = (depth * p.RT + p.lag) * (p.ngt + 1) + p.RT;
+  *total = p.total_tasks; *lag = p.lag; *row_tiles = p.RT;
+  for (int i = 0; i < p.total_tasks && i < cap; ++i) {
+    const cmwg::MegaTask t = cmwg::mega_decode(p, i);
+    out[4 * i] = t.type; out[4 * i + 1] = t.layer; out[4 * i + 2] = t.rt; out[4 * i + 3] = t.nt;
+  }
+  for (int b = 0, rt = 0; b < B; ++b) {   // the table varlen_tiles_kernel builds on the device
+    const int n = cmwg::ceil_div(lengths[b], 2 * cmwg::TC_BM);
+    for (int k = 0; k < n; ++k, ++rt)
+      if (rt < tiles_cap) { tiles[3 * rt] = b; tiles[3 * rt + 1] = k; tiles[3 * rt + 2] = n; }
+  }
+  return CMWG_OK;
 }
 
 size_t cmwg_wn_line_state_bytes(const cmwg_wn_config* cfg, int B, int T) {

@@ -118,6 +118,20 @@ def coupling_apply(x: torch.Tensor, lst: torch.Tensor, inverse: bool) -> Tuple[t
     return z, neg
 
 
+def coupling_apply_varlen(x: torch.Tensor, lst: torch.Tensor, lengths_dev: torch.Tensor,
+                          inverse: bool) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
+    """coupling_apply on a padded batch: columns t >= lengths_dev[b] of z and -log_s are 0."""
+    x = _ncl(x)
+    B, c, T = x.shape
+    cin = c // 2
+    z = torch.empty((B, c, T), device=x.device, dtype=torch.float32)
+    neg = torch.empty((B, cin, T), device=x.device, dtype=torch.float32) if inverse else None
+    L.check(L.load().cmwg_coupling_apply_varlen(x.data_ptr(), _bstride(x), lst.data_ptr(), z.data_ptr(), _bstride(z),
+                                                L.ptr(neg), B, cin, T, lengths_dev.data_ptr(), int(inverse),
+                                                L.stream_ptr(x.device)), "coupling_apply_varlen")
+    return z, neg
+
+
 def coupling_bwd(out: torch.Tensor, lst: torch.Tensor, dout: torch.Tensor, dls: torch.Tensor,
                  restored: torch.Tensor, inverse: bool) -> Tuple[torch.Tensor, torch.Tensor]:
     """Writes the re-materialised input into `restored` (contiguous (B, c, T)); returns (dlst, din)."""
@@ -177,6 +191,22 @@ def logdet_accumulate(log_s: torch.Tensor, prev, log_det_w) -> torch.Tensor:
         prev = prev.detach().float().contiguous()
     L.check(L.load().cmwg_logdet_accumulate(a.data_ptr(), a.stride(0) if B > 1 else N, B, N, L.ptr(prev), L.ptr(log_det_w),
                                             out.data_ptr(), L.stream_ptr(a.device)), "logdet_accumulate")
+    return out
+
+
+def logdet_accumulate_varlen(a: torch.Tensor, lengths_dev: torch.Tensor, prev, log_det_w_col) -> torch.Tensor:
+    """prev (B,) or None + log_det_w_col (0-dim: the log-det of one column) * len_b + a[b, :, :len_b].sum()."""
+    if a.dim() != 3 or a.stride(2) != 1 or (a.shape[1] > 1 and a.stride(1) != a.shape[2]):
+        a = a.contiguous()
+    B, Cc, T = a.shape
+    out = torch.empty((B,), device=a.device, dtype=torch.float32)
+    if log_det_w_col is not None:
+        log_det_w_col = log_det_w_col.detach().reshape(()).float().contiguous()
+    if prev is not None:
+        prev = prev.detach().float().contiguous()
+    L.check(L.load().cmwg_logdet_accumulate_varlen(a.data_ptr(), a.stride(0) if B > 1 else Cc * T, B, Cc, T,
+                                                   lengths_dev.data_ptr(), L.ptr(prev), L.ptr(log_det_w_col),
+                                                   out.data_ptr(), L.stream_ptr(a.device)), "logdet_accumulate_varlen")
     return out
 
 

@@ -21,7 +21,7 @@ from torch import Tensor
 
 from . import _lib as L
 from . import ops, precision
-from .base import FlowBase
+from .base import FlowBase, Lengths, lengths_list
 from .efficient_modules import AffineCouplingBlock, InvertibleConv1x1, grad_hint, graph_possible
 from .parallel import grad_buffer
 from .utils import add_weight_norms
@@ -279,6 +279,24 @@ class WN(nn.Module):
         st.cfg, st.packed, st.params, st.ycl, st.saved, st.B, st.T, st.prec = cfg, packed, ps, ycl, saved, B, T, prec
         return lst, st
 
+    def _cmwg_forward_varlen(self, x: Tensor, y: Tensor, lengths_host, lengths_dev: Tensor, prec: str) -> Tensor:
+        """Inference over a padded batch: lst (B, 2cin, T) whose columns t < lengths[b] equal the WN of item b alone
+        (cmwg_wn_forward_varlen); lengths_host is a ctypes int array, lengths_dev the same values as a device int32 tensor."""
+        L.require_cuda(x, y, op="WN.forward")
+        cfg, packed, _ = self._prepare(prec, x.device)
+        lib = L.load()
+        x = ops._ncl(x)
+        B, _, T = x.shape
+        if y.shape[0] != B or y.shape[1] != self.aux_chs or y.shape[2] != T:
+            raise RuntimeError(f"WN: conditioning shape {tuple(y.shape)} does not match input {(B, self.aux_chs, T)}")
+        ycl = _cond_cache.get(y if y.dtype == torch.float32 else y.float(), cfg)
+        ws = self._scratch_buf(int(lib.cmwg_wn_varlen_workspace_bytes(C.byref(cfg), B, T)), x.device, "ws")
+        lst = torch.empty((B, 2 * self.in_chs, T), device=x.device, dtype=torch.float32)
+        L.check(lib.cmwg_wn_forward_varlen(C.byref(cfg), packed.data_ptr(), x.data_ptr(), ops._bstride(x), ycl.data_ptr(),
+                                           B, T, lengths_host, lengths_dev.data_ptr(), ws.data_ptr(), lst.data_ptr(),
+                                           L.stream_ptr(x.device)), "wn_forward_varlen")
+        return lst
+
     def _grads_struct(self):
         """(cmwg_wn_grads, {id(param): destination tensor}); destinations are views of the data-parallel
         communication buffers when available."""
@@ -423,7 +441,13 @@ class _LogdetAccumulate(torch.autograd.Function):
 
 class WaveGlow(FlowBase):
     """Reference ``model/waveglow.py:108-212``: upsampler, squeeze, ``flows`` x (invertible 1x1 conv ->
-    affine coupling with WN), early outputs every ``n_early_every`` flows."""
+    affine coupling with WN), early outputs every ``n_early_every`` flows.
+
+    ``forward(x, h, lengths=...)`` / ``reverse(z, h, lengths=...)`` run a zero-padded batch of different-length items in one
+    call (inference only): ``lengths`` are valid SAMPLES per item, multiples of ``n_group``.  Item b then gets exactly what
+    the call on ``(x[b, :len_b], h[b, :, :ceil(len_b / hop)])`` alone gives on its valid samples (bit for bit in fp32 and
+    fp16), zeros after them, and a log-det over its valid samples only."""
+    _supports_lengths = True
 
     def __init__(self, flows, n_group, n_early_every, n_early_size, hop_size, n_mels, memory_efficient,
                  reverse_mode=False, **kwargs):
@@ -459,7 +483,99 @@ class WaveGlow(FlowBase):
         g, v, b = WN._gvb(up)
         return _UpsampleFunction.apply(h, g, v, b, up.stride[0], up.padding[0])
 
-    def forward_computation(self, x: Tensor, h: Tensor) -> Tuple[Tensor, Tensor]:
+    # ---- per-item lengths (inference on a padded batch) -------------------------------------------------------------
+    def _check_lengths(self, x: Tensor, h: Tensor, lengths: Lengths, what: str) -> List[int]:
+        if x.dim() != 2 or h.dim() != 3 or h.shape[0] != x.shape[0]:
+            raise ValueError(f"{what}: expected x (B, T) and h (B, n_mels, frames), got {tuple(x.shape)} and {tuple(h.shape)}")
+        B, T = x.shape
+        lens = lengths_list(lengths, B, what, "samples")
+        for n in lens:
+            if not 1 <= n <= T or n % self.n_group:
+                raise ValueError(f"{what}: length {n} must be a multiple of n_group={self.n_group} in [1, {T}] "
+                                 "(lengths are in samples here; FlowBase.infer takes mel frames)")
+        if torch.is_grad_enabled() and (x.requires_grad or h.requires_grad or any(p.requires_grad for p in self.parameters())):
+            raise NotImplementedError(f"{what}: per-item lengths are inference only; run under torch.no_grad() "
+                                      "(training on variable-length batches is not supported)")
+        return lens
+
+    def _varlen_prepare(self, x: Tensor, h: Tensor, lens: List[int]):
+        """x and h with their padding zeroed -> the squeezed input, the upsampled conditioning and the per-item lengths in
+        squeezed columns (host ctypes array and device int32 tensor)."""
+        L.require_cuda(x, h, op="WaveGlow")
+        B, T = x.shape
+        hop = self._hop_length
+        frames = [-(-n // hop) for n in lens]
+        t_idx = torch.arange(T, device=x.device)
+        f_idx = torch.arange(h.shape[2], device=h.device)
+        len_t = torch.tensor(lens, device=x.device)
+        x = torch.where(t_idx[None, :] < len_t[:, None], x.float(), 0.)
+        # a zero frame adds nothing to the transposed conv, so the upsampled conditioning equals the item's own on its samples
+        h = torch.where(f_idx[None, None, :] < torch.tensor(frames, device=h.device)[:, None, None], h.float(), 0.)
+        up = self.upsampler
+        g, v, b = WN._gvb(up)
+        y = ops.upsample_fwd(h, g, v, b, up.stride[0], up.padding[0])
+        xs = ops.squeeze(x, self.n_group, False)
+        assert xs.size(2) <= y.size(2)
+        y = y[..., :xs.size(2)]
+        cols = [n // self.n_group for n in lens]
+        cols_host = (C.c_int * B)(*cols)
+        cols_dev = torch.tensor(cols, dtype=torch.int32).to(x.device)
+        return xs, y, cols_host, cols_dev
+
+    # One flow's two steps on a padded batch.  `inverse` is the direction the model asks for; a module built with
+    # reverse_mode=True swaps it (Reversible._direction), exactly as the ordinary path's module calls do.
+    def _varlen_conv(self, k: int, x: Tensor, inverse: bool) -> Tuple[Tensor, Tensor]:
+        conv = self.invconv1x1[k]
+        inv = inverse != bool(conv._reverse_mode)
+        w2 = conv.weight.detach().reshape(conv.weight.shape[0], -1).float().contiguous()
+        winv, ld = ops.small_inverse_logdet(w2)
+        return ops.conv1x1_apply(winv if inv else w2, x), (-ld if inv else ld)
+
+    def _varlen_coupling(self, k: int, x: Tensor, y: Tensor, cols_host, cols_dev: Tensor,
+                         inverse: bool) -> Tuple[Tensor, Tensor]:
+        coup = self.WNs[k]
+        inv = inverse != bool(coup._reverse_mode)
+        F = coup.F
+        lst = F._cmwg_forward_varlen(x, y, cols_host, cols_dev, precision.resolve(F._tc_supported(), training=False))
+        z, neg_log_s = ops.coupling_apply_varlen(x, lst, cols_dev, inverse=inv)
+        return z, (neg_log_s if inv else lst[:, :F.in_chs])
+
+    def _forward_varlen(self, x: Tensor, h: Tensor, lens: List[int]) -> Tuple[Tensor, Tensor]:
+        batch = x.size(0)
+        x, y, cols_host, cols_dev = self._varlen_prepare(x, h, lens)
+        early: List[Tensor] = []
+        logdet = None
+        for k in range(len(self.WNs)):
+            if k % self.n_early_every == 0 and k:
+                e, x = x.split([self.n_early_size, x.size(1) - self.n_early_size], 1)
+                early.append(e)
+            x, ldw = self._varlen_conv(k, x, False)
+            x, log_s = self._varlen_coupling(k, x, y, cols_host, cols_dev, False)
+            logdet = ops.logdet_accumulate_varlen(log_s, cols_dev, logdet, ldw)
+        early.append(x)
+        z = ops.squeeze(torch.cat(early, 1), self.n_group, True)
+        return z.view(batch, -1), logdet
+
+    def _reverse_varlen(self, z: Tensor, h: Tensor, lens: List[int]) -> Tuple[Tensor, Tensor]:
+        batch = z.size(0)
+        z, y, cols_host, cols_dev = self._varlen_prepare(z, h, lens)
+        parts = list(z.split(self.z_split_sizes, 1))
+        z = parts.pop()
+        logdet = None
+        for k in range(len(self.WNs) - 1, -1, -1):
+            z, log_s = self._varlen_coupling(k, z, y, cols_host, cols_dev, True)
+            z, ldw = self._varlen_conv(k, z, True)
+            logdet = ops.logdet_accumulate_varlen(log_s, cols_dev, logdet, ldw)
+            if k % self.n_early_every == 0 and k:
+                z = torch.cat((parts.pop(), z), 1)
+        x = ops.squeeze(z, self.n_group, True)
+        return x.view(batch, -1), logdet
+
+    def forward_computation(self, x: Tensor, h: Tensor, lengths: Optional[Lengths] = None) -> Tuple[Tensor, Tensor]:
+        if lengths is not None:
+            lens = self._check_lengths(x, h, lengths, "WaveGlow.forward")
+            if any(n != x.shape[1] for n in lens):   # all lengths == T: the ordinary call, same bits
+                return self._forward_varlen(x, h, lens)
         L.require_cuda(x, h, op="WaveGlow.forward")
         y = self._upsample_h(h)
         batch = x.size(0)
@@ -482,7 +598,11 @@ class WaveGlow(FlowBase):
         z = _SqueezeFunction.apply(torch.cat(early, 1), self.n_group, True)
         return z.view(batch, -1), logdet
 
-    def reverse_computation(self, z: Tensor, h: Tensor) -> Tuple[Tensor, Tensor]:
+    def reverse_computation(self, z: Tensor, h: Tensor, lengths: Optional[Lengths] = None) -> Tuple[Tensor, Tensor]:
+        if lengths is not None:
+            lens = self._check_lengths(z, h, lengths, "WaveGlow.reverse")
+            if any(n != z.shape[1] for n in lens):
+                return self._reverse_varlen(z, h, lens)
         L.require_cuda(z, h, op="WaveGlow.reverse")
         y = self._upsample_h(h)
         batch = z.size(0)

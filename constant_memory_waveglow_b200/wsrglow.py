@@ -92,6 +92,7 @@ class MuLawEncoding(nn.Module):
 class WSRGlow(WaveGlow):
     """Reference ``model/wsrglow.py:21-56`` (same constructor, attributes and state-dict keys:
     ``mu_enc.1.weight``, ``angle_embed.embed.weight``, buffer ``window``)."""
+    _supports_lengths = False   # WaveGlow's per-item lengths do not cover the low-rate conditioning front end
 
     def __init__(self, upsample_rate: int = 2, memory_efficient: bool = False, **kwargs) -> None:
         super().__init__(12, 8 * upsample_rate, 4, 2, 8 * upsample_rate, 8 * 400 + 51 * 9,

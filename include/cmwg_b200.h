@@ -99,6 +99,11 @@ int cmwg_conv1x1_backward(const float* w, const float* w_inv, int inverse_mode, 
 int cmwg_coupling_apply(const float* x, long long x_bstride, const float* lst, float* z, long long z_bstride,
                         float* neg_log_s, int B, int cin, int T, int inverse, void* stream);
 
+/* cmwg_coupling_apply for a padded batch with per-item lengths (lengths_dev: B device ints, in columns of T): the same
+ * values at columns t < lengths_dev[b]; z (both halves) and neg_log_s are written as 0 at t >= lengths_dev[b]. */
+int cmwg_coupling_apply_varlen(const float* x, long long x_bstride, const float* lst, float* z, long long z_bstride,
+                               float* neg_log_s, int B, int cin, int T, const int* lengths_dev, int inverse, void* stream);
+
 /* The elementwise half of AffineCouplingFunc.backward (:132-148, inverse = 0) and of
  * InvAffineCouplingFunc.backward (:190-207, inverse = 1).  Given the saved OUTPUT `out` of the
  * forward call, the recomputed `lst`, and the incoming cotangents (dout for the tensor output,
@@ -197,6 +202,23 @@ unsigned long long cmwg_debug_counter(int which);
 int cmwg_mega_clk_read(long long* host, int n);
 /* bytes of per-layer activations kept between cmwg_wn_forward(save != NULL) and cmwg_wn_backward */
 size_t cmwg_wn_saved_bytes(const cmwg_wn_config* cfg, int B, int T);
+
+/* Inference over a padded batch with per-item lengths: item b of (x, ycl, lst) holds lengths_host[b] valid time steps of T,
+ * 1 <= lengths_host[b] <= T.  lst[b, :, t] for t < lengths_host[b] is bit-identical to cmwg_wn_forward on that item alone
+ * with T = lengths_host[b]; lst at t >= lengths_host[b] is unspecified (the single-kernel forward does not compute row tiles
+ * that hold no valid step).  lengths_host plans the work on the host; lengths_dev is a device int[B] holding the SAME values,
+ * uploaded by the caller (the library never allocates or copies it).  workspace: cmwg_wn_varlen_workspace_bytes(cfg, B, T).
+ * No `saved` (training on per-item lengths is not supported).  Returns CMWG_ERR_ARG for a length outside [1, T] and
+ * CMWG_ERR_UNSUPPORTED for the 2-D WN (height > 1) and for CMWG_MEGA_RDIRECT=1 residual tiles. */
+size_t cmwg_wn_varlen_workspace_bytes(const cmwg_wn_config* cfg, int B, int T);
+int cmwg_wn_forward_varlen(const cmwg_wn_config* cfg, const void* packed, const float* x, long long x_bstride,
+                           const void* ycl, int B, int T, const int* lengths_host, const int* lengths_dev, void* workspace,
+                           float* lst, void* stream);
+/* host-side listing of the single-kernel WN forward's task list for per-item lengths (host array `lengths`): out / total / lag as
+ * cmwg_mega_task_list(0, ...); *row_tiles = sum_b ceil(lengths[b] / 256) compacted row tiles and tiles[3 rt .. 3 rt + 2] =
+ * (item, tile within the item, tiles of the item) for rt < min(*row_tiles, tiles_cap) */
+int cmwg_mega_task_list_varlen(int depth, int B, int T, const int* lengths, int* out, int cap, int* total, int* lag, int* tiles,
+                               int tiles_cap, int* row_tiles);
 
 /* (log_s, t) = WN(xa, y)   (model/waveglow.py:98-105 with NonCausalLayer.forward :41-46 and
  * fused_gate :13-15).  xa = first cin channels of x (NCL, batch stride x_bstride);
@@ -345,6 +367,12 @@ int cmwg_sum_per_batch(const float* a, long long a_bstride, int B, int N, float*
  * float) may be NULL (= 0); out may alias prev.  Deterministic. */
 int cmwg_logdet_accumulate(const float* a, long long a_bstride, int B, int N, const float* prev, const float* log_det_w,
                            float* out, void* stream);
+
+/* Per-item lengths: out[b] = prev[b] + *log_det_w * len_b + sum over channels c < C and columns t < len_b of a[b, c, t],
+ * len_b = lengths_dev[b] (device ints).  a: (C, T) rows per item at batch stride a_bstride.  log_det_w here is the log-det
+ * of ONE column (the 1x1 conv's log|det W|), scaled by each item's own length.  The padded columns are not read. */
+int cmwg_logdet_accumulate_varlen(const float* a, long long a_bstride, int B, int C, int T, const int* lengths_dev,
+                                  const float* prev, const float* log_det_w, float* out, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Per-kernel-class device timing (CUDA events recorded on the launching stream around each GEMM
