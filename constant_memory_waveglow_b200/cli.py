@@ -5,6 +5,8 @@ repository root; its ``inference.py`` cannot in this image (``torchaudio.load`` 
 so the two entry points exist here with the reference's flags (``train.py:81-93``, ``inference.py:62-70``) on top of the
 RIFF reader/writer of ``datasets.py``.  Multi-GPU: launch ``train`` under ``torchrun --nproc-per-node N``.  ``synth-batch``
 re-synthesises many files, batching utterances of different lengths into one call each (``WaveGlow.infer(lengths=...)``).
+``-d/--denoiser-strength`` on ``synth`` and ``synth-batch`` runs the bias-spectrum ``Denoiser`` on the output (one call per
+batch, with the per-item lengths); at 0, the default, it is skipped.
 """
 from __future__ import annotations
 
@@ -74,7 +76,9 @@ def synth(argv) -> None:
     p.add_argument("outfile", type=str)
     p.add_argument("-s", "--sigma", type=float, default=0.6)
     p.add_argument("-n", "--n-group", type=int, default=None)
+    _add_denoiser_arg(p)
     args = p.parse_args(argv)
+    _check_denoiser_arg(p, args)
     lit = TR.LightModel.load_from_checkpoint(args.ckpt, map_location="cpu")
     model, conditioner = lit.model, lit.conditioner
     model.apply(remove_weight_norms)
@@ -95,8 +99,30 @@ def synth(argv) -> None:
         print("Time cost: {:.4f}, Speed: {:.4f} kHz".format(cost, z.numel() / cost / 1000))
         x, cost = _timed(lambda: model.infer(cond, args.sigma))
     print("Time cost: {:.4f}, Speed: {:.4f} kHz".format(cost, x.numel() / cost / 1000))
+    if args.denoiser_strength > 0:
+        x = _denoiser(model, x.numel(), p)(x, args.denoiser_strength)
     print(x.max().item(), x.min().item())
     wav_write(args.outfile, x.reshape(1, -1), sr)
+
+
+def _add_denoiser_arg(p: argparse.ArgumentParser) -> None:
+    p.add_argument("-d", "--denoiser-strength", type=float, default=0.0,
+                   help="subtract this multiple of the model's bias spectrum from the output (Denoiser); 0 = off")
+
+
+def _check_denoiser_arg(p: argparse.ArgumentParser, args) -> None:
+    if not 0 <= args.denoiser_strength < math.inf:
+        p.error("--denoiser-strength must be a finite number >= 0")
+
+
+def _denoiser(model, shortest: int, p: argparse.ArgumentParser):
+    """The Denoiser of `model` for outputs of at least `shortest` samples (its STFT needs more than filter_length / 2)."""
+    from .denoiser import Denoiser
+    d = Denoiser(model)
+    if shortest <= d.filter_length // 2:
+        p.error(f"--denoiser-strength: an output of {shortest} samples is too short to denoise "
+                f"(more than {d.filter_length // 2} needed)")
+    return d
 
 
 def _load_for_synthesis(ckpt: str):
@@ -123,7 +149,9 @@ def synth_batch(argv) -> None:
     p.add_argument("-s", "--sigma", type=float, default=0.6)
     p.add_argument("--max-batch", type=int, default=16, help="utterances per synthesis call")
     p.add_argument("--seed", type=int, default=0, help="noise seed; file i draws from a generator seeded by (seed, i)")
+    _add_denoiser_arg(p)
     args = p.parse_args(argv)
+    _check_denoiser_arg(p, args)
     if args.max_batch < 1:
         p.error("--max-batch must be >= 1")
     stems = [os.path.splitext(os.path.basename(f))[0] for f in args.infiles]
@@ -140,6 +168,9 @@ def synth_batch(argv) -> None:
             rates.append(wav_info(f).sample_rate)
             conds.append(conditioner(wav_read(f).mean(0, keepdim=True).to(dev))[0])
         order = sorted(range(len(conds)), key=lambda i: conds[i].shape[-1])
+        denoiser = None
+        if args.denoiser_strength > 0:
+            denoiser = _denoiser(model, conds[order[0]].shape[-1] * hop, p)
         total, cost = 0, 0.0
         for s0 in range(0, len(order), args.max_batch):
             idx = order[s0:s0 + args.max_batch]
@@ -150,6 +181,8 @@ def synth_batch(argv) -> None:
             z = z.to(dev)
             x, dt = _timed(lambda: model.infer(h, args.sigma, z=z, lengths=frames))
             cost += dt
+            if denoiser is not None:
+                x = denoiser(x, args.denoiser_strength, lengths=[f * hop for f in frames])
             for j, i in enumerate(idx):
                 n = frames[j] * hop
                 total += n

@@ -6,19 +6,12 @@
 //
 // One CTA per (batch, frame).  The n_fft real samples are packed as n_fft/2 complex numbers z[n] = x[2n] + i x[2n+1]
 // (window applied, reflected indices resolved while loading), transformed by an in-shared-memory radix-2 FFT of half
-// the length, and split back into the n_fft/2+1 one-sided bins.  A thread per mel band then runs over that band's
-// support [lo, hi) of the triangular filter.  The real workloads are small (24 x 63 training frames, 863 frames per
+// the length, and split back into the n_fft/2+1 one-sided bins (fft.cuh, shared with the denoiser).  A thread per mel
+// band then runs over that band's support [lo, hi) of the triangular filter.  The real workloads are small (24 x 63 training frames, 863 frames per
 // 10 s utterance), so the kernel is latency bound and a CTA per frame -- the widest decomposition -- is the fast one.
-#include "common.cuh"
+#include "fft.cuh"
 
 namespace cmwg {
-
-__device__ __forceinline__ int reflect_index(int i, int T) {
-  // ReflectionPad1d semantics (edge sample not repeated); valid for pads < T
-  if (i < 0) i = -i;
-  if (i >= T) i = 2 * (T - 1) - i;
-  return i;
-}
 
 template <int NFFT>
 __global__ void __launch_bounds__(256) melspec_kernel(const float* __restrict__ x, long long x_bstride, int T,
@@ -27,16 +20,11 @@ __global__ void __launch_bounds__(256) melspec_kernel(const float* __restrict__ 
                                                       const int* __restrict__ fb_hi, int n_mels, int hop,
                                                       int pad_left, int frames, int power_is_one, float eps,
                                                       int take_log, float* __restrict__ out) {
-  constexpr int M = NFFT / 2;  // complex FFT length
-  constexpr int LOGM = (M == 64) ? 6 : (M == 128) ? 7 : (M == 256) ? 8 : (M == 512) ? 9 : (M == 1024) ? 10 : 11;
+  constexpr int M = FftShape<NFFT>::M;
   constexpr int NT = 256;
-  // one pad slot per 16 entries: the bit-reversed scatter (stride M/2) and the strided twiddle reads of the late
-  // stages (stride NFFT >> (s+1)) would otherwise hit a single bank 32 ways
-  constexpr int MP = M + M / 16;
-#define CMWG_PADI(i) ((i) + ((i) >> 4))
-  __shared__ float2 z[MP];
-  __shared__ float2 tw[MP];      // tw[PAD(k)] = exp(-2 pi i k / NFFT), k < NFFT/2
-  __shared__ float pw[M + 1];    // |X[k]|^power, k <= NFFT/2
+  __shared__ float2 z[FftShape<NFFT>::MP];
+  __shared__ float2 tw[FftShape<NFFT>::MP];   // tw[padi(k)] = exp(-2 pi i k / NFFT), k < NFFT/2
+  __shared__ float pw[M + 1];                  // |X[k]|^power, k <= NFFT/2
 
   const int b = blockIdx.x / frames, fr = blockIdx.x % frames;
   const float* xb = x + (long long)b * x_bstride;
@@ -47,47 +35,18 @@ __global__ void __launch_bounds__(256) melspec_kernel(const float* __restrict__ 
     my_hi = fb_hi[threadIdx.x];
   }
 
-  for (int k = threadIdx.x; k < M; k += NT) {
-    float s, c;
-    sincospif(-2.f * (float)k / (float)NFFT, &s, &c);
-    tw[CMWG_PADI(k)] = make_float2(c, s);
-  }
+  fft_twiddles<NFFT, NT>(tw);
   // bit-reversed scatter of the packed, windowed frame
   for (int n = threadIdx.x; n < M; n += NT) {
     int i0 = reflect_index(start + 2 * n, T), i1 = reflect_index(start + 2 * n + 1, T);
     float a = xb[i0] * window[2 * n], c = xb[i1] * window[2 * n + 1];
-    int r = (int)(__brev((unsigned)n) >> (32 - LOGM));
-    z[CMWG_PADI(r)] = make_float2(a, c);
+    z[fft_bitrev_slot<NFFT>(n)] = make_float2(a, c);
   }
   __syncthreads();
-  // radix-2 decimation-in-time stages on M points; twiddle exp(-2 pi i pos / (2 half)) = tw[pos * (NFFT / (2 half))]
-#pragma unroll 1
-  for (int s = 0; s < LOGM; ++s) {
-    const int half = 1 << s;
-    const int tstep = NFFT >> (s + 1);
-    for (int j = threadIdx.x; j < M / 2; j += NT) {
-      int pos = j & (half - 1);
-      int i0 = ((j >> s) << (s + 1)) + pos, i1 = i0 + half;
-      float2 w = tw[CMWG_PADI(pos * tstep)];
-      i0 = CMWG_PADI(i0);
-      i1 = CMWG_PADI(i1);
-      float2 u = z[i0], v = z[i1];
-      float2 t = make_float2(fmaf(v.x, w.x, -v.y * w.y), fmaf(v.x, w.y, v.y * w.x));
-      z[i0] = make_float2(u.x + t.x, u.y + t.y);
-      z[i1] = make_float2(u.x - t.x, u.y - t.y);
-    }
-    __syncthreads();
-  }
-  // split: X[k] = (Z[k] + conj Z[M-k]) / 2 - (i/2) exp(-2 pi i k / NFFT) (Z[k] - conj Z[M-k]),  k = 0..M  (Z[M] = Z[0])
+  fft_radix2<NFFT, NT>(z, tw);
   for (int k = threadIdx.x; k <= M; k += NT) {
-    float2 a = z[CMWG_PADI(k & (M - 1))], c = z[CMWG_PADI((M - k) & (M - 1))];
-    float er = 0.5f * (a.x + c.x), ei = 0.5f * (a.y - c.y);   // even part
-    float dr = 0.5f * (a.x - c.x), di = 0.5f * (a.y + c.y);   // (Z[k] - conj Z[M-k]) / 2
-    float2 w = (k < M) ? tw[CMWG_PADI(k)] : make_float2(-1.f, 0.f);
-    // -i * w * d
-    float pr = w.x * dr - w.y * di, pi = w.x * di + w.y * dr;
-    float xr = er + pi, xi = ei - pr;
-    float p = fmaf(xr, xr, xi * xi);
+    float2 X = rfft_split(z[fft_padi(k & (M - 1))], z[fft_padi((M - k) & (M - 1))], fft_split_twiddle<NFFT>(tw, k));
+    float p = fmaf(X.x, X.x, X.y * X.y);
     pw[k] = power_is_one ? sqrtf(p) : p;
   }
   __syncthreads();
@@ -108,7 +67,6 @@ __global__ void __launch_bounds__(256) melspec_kernel(const float* __restrict__ 
     float v = (a0 + a1) + (a2 + a3) + eps;
     out[((long long)b * n_mels + m) * frames + fr] = take_log ? logf(v) : v;
   }
-#undef CMWG_PADI
 }
 
 }  // namespace cmwg

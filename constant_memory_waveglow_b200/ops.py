@@ -7,7 +7,9 @@ batch stride is free so channel slices of a wider tensor are passed without copi
 from __future__ import annotations
 
 import ctypes as C
-from typing import Optional, Tuple
+import math
+import numbers
+from typing import List, Optional, Tuple
 
 import torch
 
@@ -270,6 +272,70 @@ def upsample_bwd_input(g, v, dy, F: int, stride: int, pad: int) -> torch.Tensor:
                                              F, K, stride, pad, Tv, dh.data_ptr(), L.stream_ptr(dy.device)),
             "upsample_bwd_input")
     return dh
+
+
+# ---------------------------------------------------------------------------------------------
+# denoiser (bias-spectrum subtraction)
+# ---------------------------------------------------------------------------------------------
+def stft_frame_magnitude(x: torch.Tensor, window: torch.Tensor, hop: int, frame: int = 0) -> torch.Tensor:
+    """|torch.stft(x, n_fft, hop, window, center=True, pad_mode="reflect")[:, frame]| of a 1-D signal, n_fft = len(window)."""
+    L.require_cuda(x, window, op="stft_frame_magnitude")
+    x = x.detach().reshape(-1).float().contiguous()
+    n_fft = window.numel()
+    mag = torch.empty((n_fft // 2 + 1,), device=x.device, dtype=torch.float32)
+    L.check(L.load().cmwg_stft_frame_magnitude(x.data_ptr(), x.numel(), window.data_ptr(), n_fft, int(hop), int(frame),
+                                               mag.data_ptr(), L.stream_ptr(x.device)), "stft_frame_magnitude")
+    return mag
+
+
+def denoise_lengths(audio: torch.Tensor, n_fft: int, strength: float, lengths) -> Optional[List[int]]:
+    """The argument checks of denoise() (no device needed): audio (T,) or (B, T), strength >= 0, each length in
+    (n_fft // 2, T].  Returns the lengths as a list of ints, or None."""
+    from .base import lengths_list
+    if audio.dim() not in (1, 2):
+        raise ValueError(f"denoise: expected audio (T,) or (B, T), got {tuple(audio.shape)}")
+    if isinstance(strength, bool) or not isinstance(strength, numbers.Real) or not 0 <= strength < math.inf:
+        raise ValueError(f"denoise: strength must be a finite number >= 0, got {strength!r}")
+    B = 1 if audio.dim() == 1 else audio.shape[0]
+    T = audio.shape[-1]
+    lens = None if lengths is None else lengths_list(lengths, B, "denoise", "samples")
+    for n in (lens if lens is not None else ([T] if B else [])):
+        if not n_fft // 2 < n <= T:
+            raise ValueError(f"denoise: length {n} outside ({n_fft // 2}, {T}]: reflect padding by n_fft/2 needs more "
+                             "samples than the pad (lengths are in samples)")
+    return lens
+
+
+def denoise(audio: torch.Tensor, window: torch.Tensor, bias_mag: torch.Tensor, strength: float, hop: int,
+            lengths=None, workspace: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Bias-spectrum subtraction (cmwg_denoise) of audio (T,) or (B, T) with optional per-item `lengths` in samples; returns
+    a tensor of audio's shape, 0 after each item's length.  `workspace`: uint8 tensor of at least
+    cmwg_denoise_workspace_bytes bytes (allocated here when None)."""
+    n_fft = window.numel()
+    lens = denoise_lengths(audio, n_fft, strength, lengths)
+    L.require_cuda(audio, window, bias_mag, op="denoise")
+    x = audio.detach()
+    squeeze = x.dim() == 1
+    if squeeze:
+        x = x.unsqueeze(0)
+    if x.dtype != torch.float32 or x.stride(1) != 1:
+        x = x.float().contiguous()
+    B, T = x.shape
+    out = torch.empty((B, T), device=x.device, dtype=torch.float32)
+    lib = L.load()
+    need = int(lib.cmwg_denoise_workspace_bytes(B, T, n_fft, int(hop)))
+    if workspace is None:
+        workspace = torch.empty((max(need, 4),), device=x.device, dtype=torch.uint8)
+    elif workspace.numel() * workspace.element_size() < need:
+        raise ValueError(f"denoise: workspace of {workspace.numel() * workspace.element_size()} bytes, {need} needed")
+    lens_host = lens_dev = None
+    if lens is not None:
+        lens_host = (C.c_int * B)(*lens)
+        lens_dev = torch.tensor(lens, dtype=torch.int32).to(x.device)
+    L.check(lib.cmwg_denoise(x.data_ptr(), x.stride(0) if B > 1 else T, B, T, lens_host, L.ptr(lens_dev),
+                             window.data_ptr(), bias_mag.data_ptr(), float(strength), n_fft, int(hop),
+                             workspace.data_ptr(), out.data_ptr(), L.stream_ptr(x.device)), "denoise")
+    return out[0] if squeeze else out
 
 
 def selftest_tc_gemm(a: torch.Tensor, b: torch.Tensor, M: int, N: int, K: int, variant: int) -> torch.Tensor:

@@ -283,6 +283,30 @@ int cmwg_melspec_fwd(const float* x, long long x_bstride, int B, int T, const fl
                      int take_log, float* out, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Denoiser of synthesised audio: bias-spectrum subtraction, the `Denoiser` of NVIDIA's WaveGlow (denoiser.py, mode 'zeros',
+ * used by its inference.py --denoiser_strength).  With w the window (n_fft floats; a window shorter than n_fft zero-padded and
+ * centred, as torch.stft does), STFT(x) = torch.stft(x, n_fft, hop, window=w, center=True, pad_mode="reflect",
+ * onesided=True): len / hop + 1 frames of n_fft/2 + 1 bins.  n_fft: power of two in [128, 4096]; 1 <= hop <= n_fft/2; the
+ * window's squared overlap-add must not vanish (true for a Hann window of win_length >= 2 hop).  Lengths: n_fft/2 < len <= T
+ * (reflect padding needs more samples than the pad).  Deterministic; the caller owns all memory.
+ * ------------------------------------------------------------------------------------------- */
+/* mag (n_fft/2 + 1 floats) <- |STFT(x)[:, frame]| of one signal x (T floats), 0 <= frame <= T / hop.  The denoiser's bias
+ * spectrum is this at frame 0 of the model's output for an all-zero mel spectrogram. */
+int cmwg_stft_frame_magnitude(const float* x, int T, const float* window, int n_fft, int hop, int frame, float* mag,
+                              void* stream);
+/* bytes of the workspace of cmwg_denoise: B * (T / hop + 1) * n_fft floats (the windowed time-domain frames) */
+size_t cmwg_denoise_workspace_bytes(int B, int T, int n_fft, int hop);
+/* out (B, T) contiguous <- per item b, over its first len_b samples (len_b = lengths[b], or T when both length pointers are
+ * NULL): S = STFT(x_b), M = max(|S| - strength * bias_mag[:, None], 0), out_b = torch.istft(M * S / |S|, n_fft, hop, w,
+ * center=True, length=len_b), with the term 0 where |S| = 0; out[b, t] = 0 for t >= len_b.  Each item's output is
+ * bit-identical to a call on that item alone.  x: (B, T) at batch stride x_bstride; bias_mag: n_fft/2 + 1 floats;
+ * strength >= 0.  lengths_host (host) and lengths_dev (device) hold the same B ints, or are both NULL.  workspace:
+ * cmwg_denoise_workspace_bytes(B, T, n_fft, hop) bytes.  Bad sizes, lengths or strength: CMWG_ERR_ARG. */
+int cmwg_denoise(const float* x, long long x_bstride, int B, int T, const int* lengths_host, const int* lengths_dev,
+                 const float* window, const float* bias_mag, float strength, int n_fft, int hop, void* workspace, float* out,
+                 void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * WSRGlow conditioning front end (model/wsrglow.py:37-50, `_get_cond`), one kernel:
  *   c (B, Tc) fp32 low-rate signal, CLIPPED TO [-1, 1] IN PLACE like the reference's c.clip_(-1, 1) (:38);
  *   out (B, 8E + 9 + 9P, Tc/8) fp32 NCL = cat(mu-law code embedding rows (emb: n_codes x E, :39), the 9 magnitudes of
