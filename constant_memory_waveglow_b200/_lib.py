@@ -102,6 +102,10 @@ SIGNATURES = {
     "cmwg_upsample_bwd_workspace": (_SZ, [_I, _I, _I]),
     "cmwg_upsample_bwd": (_I, [_VP, _VP, _VP, _VP, _LL, _LL, _I, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP]),
     "cmwg_upsample_bwd_input": (_I, [_VP, _VP, _VP, _LL, _LL, _I, _I, _I, _I, _I, _I, _I, _VP, _VP]),
+    "cmwg_nvidia_upsample_packed_bytes": (_SZ, [_I, _I, _I]),
+    "cmwg_nvidia_upsample_pack": (_I, [_VP, _I, _I, _I, _I, _I, _VP, _VP]),
+    "cmwg_nvidia_upsample_workspace_bytes": (_SZ, [_I, _I, _I, _I, _I, _I]),
+    "cmwg_nvidia_upsample_slab": (_I, [_VP, _VP, _VP, _LL, _LL, _I, _I, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP]),
     "cmwg_squeeze": (_I, [_VP, _VP, _I, _I, _I, _I, _VP]),
     "cmwg_nll_loss": (_I, [_VP, _VP, _I, _I, C.c_float, _I, _VP, _VP, _VP, _VP]),
     "cmwg_sum_per_batch": (_I, [_VP, _LL, _I, _I, _VP, _I, C.c_float, _VP]),

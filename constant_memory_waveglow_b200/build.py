@@ -18,7 +18,7 @@ LIBDIR = os.path.join(HERE, "lib")
 OBJDIR = os.path.join(LIBDIR, "obj")
 LIB = os.path.join(LIBDIR, "libcmwg_b200.so")
 SOURCES = ["flow_elementwise.cu", "upsample.cu", "melspec.cu", "denoise.cu", "waveflow.cu", "wsrglow_cond.cu", "lvc.cu",
-           "engine_tc.cu", "wn_pipeline.cu"]
+           "engine_tc.cu", "wn_pipeline.cu", "nvidia_upsample.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 

@@ -1,4 +1,4 @@
-"""Command line of the harness: ``python -m constant_memory_waveglow_b200.cli {train,synth,synth-batch} ...``.
+"""Command line of the harness: ``python -m constant_memory_waveglow_b200.cli {train,synth,synth-batch,vocode} ...``.
 
 The reference's own ``train.py`` runs unchanged on the ``pytorch_lightning`` / ``model`` / ``datasets`` shims at the
 repository root; its ``inference.py`` cannot in this image (``torchaudio.load`` / ``save`` need the absent TorchCodec),
@@ -6,7 +6,8 @@ so the two entry points exist here with the reference's flags (``train.py:81-93`
 RIFF reader/writer of ``datasets.py``.  Multi-GPU: launch ``train`` under ``torchrun --nproc-per-node N``.  ``synth-batch``
 re-synthesises many files, batching utterances of different lengths into one call each (``WaveGlow.infer(lengths=...)``).
 ``-d/--denoiser-strength`` on ``synth`` and ``synth-batch`` runs the bias-spectrum ``Denoiser`` on the output (one call per
-batch, with the per-item lengths); at 0, the default, it is skipped.
+batch, with the per-item lengths); at 0, the default, it is skipped.  ``vocode`` synthesises mel spectrogram files (.pt /
+.npy, as NVIDIA's ``inference.py`` reads them) with an NVIDIA WaveGlow checkpoint or this package's, batched the same way.
 """
 from __future__ import annotations
 
@@ -190,11 +191,101 @@ def synth_batch(argv) -> None:
     print("{} files, {} samples, synthesis {:.4f} s, {:.4f} kHz".format(len(conds), total, cost, total / max(cost, 1e-9) / 1e3))
 
 
+def _read_mel(path: str, n_mels: int, p: argparse.ArgumentParser) -> torch.Tensor:
+    """A mel spectrogram file as NVIDIA's inference.py reads them: .pt (a tensor) or .npy, (n_mels, frames) or
+    (1, n_mels, frames)."""
+    if path.endswith(".npy"):
+        import numpy as np
+        m = torch.from_numpy(np.load(path, allow_pickle=False))
+    elif path.endswith(".pt"):
+        m = torch.load(path, map_location="cpu", weights_only=True)
+    else:
+        p.error(f"{path}: mel files must be .pt or .npy")
+    if not isinstance(m, torch.Tensor) or m.dim() not in (2, 3) or (m.dim() == 3 and m.shape[0] != 1) \
+            or not m.is_floating_point():
+        p.error(f"{path}: expected a floating-point mel of shape (n_mels, frames) or (1, n_mels, frames), got "
+                f"{tuple(m.shape) if isinstance(m, torch.Tensor) else type(m).__name__}")
+    m = m.reshape(m.shape[-2], m.shape[-1])
+    if m.shape[0] != n_mels or m.shape[1] < 1:
+        p.error(f"{path}: mel of shape {tuple(m.shape)} does not fit the model ({n_mels} mel channels, >= 1 frame)")
+    return m.float()
+
+
+def _load_vocoder(ckpt: str, p: argparse.ArgumentParser):
+    """(model on the CPU, default sampling rate) of an NVIDIA WaveGlow checkpoint or of this package's Lightning
+    checkpoint, told apart by their contents (read with weights_only=True first either way)."""
+    from . import nvidia
+    try:
+        obj = nvidia._read_checkpoint(ckpt)
+    except Exception as e:
+        p.error(f"{ckpt}: not a checkpoint this command reads ({e})")
+    if isinstance(obj, dict) and "hyper_parameters" in obj and isinstance(obj.get("state_dict"), dict) \
+            and any(k.startswith("model.") for k in obj["state_dict"]):
+        lit = TR.LightModel.load_from_checkpoint(ckpt, map_location="cpu")
+        lit.model.apply(remove_weight_norms)
+        return lit.model, int(lit.conditioner.sample_rate)
+    return nvidia.load_nvidia_waveglow(obj, device="cpu"), 22050
+
+
+def vocode(argv) -> None:
+    p = argparse.ArgumentParser(prog="cli vocode", description="synthesis from mel spectrograms (.pt / .npy), batched by "
+                                "length; NVIDIA WaveGlow or this package's checkpoints")
+    p.add_argument("ckpt", type=str)
+    p.add_argument("outdir", type=str)
+    p.add_argument("mels", type=str, nargs="+")
+    p.add_argument("-s", "--sigma", type=float, default=0.6)
+    p.add_argument("--max-batch", type=int, default=16, help="utterances per synthesis call")
+    p.add_argument("--seed", type=int, default=0, help="noise seed; file i draws from a generator seeded by (seed, i)")
+    p.add_argument("--sampling-rate", type=int, default=None,
+                   help="of the written WAVs (default: 22050 for NVIDIA checkpoints, else the conditioner's)")
+    _add_denoiser_arg(p)
+    args = p.parse_args(argv)
+    _check_denoiser_arg(p, args)
+    if args.max_batch < 1:
+        p.error("--max-batch must be >= 1")
+    if args.sampling_rate is not None and args.sampling_rate < 1:
+        p.error("--sampling-rate must be >= 1")
+    stems = [os.path.splitext(os.path.basename(f))[0] for f in args.mels]
+    if len(set(stems)) != len(stems):
+        p.error("mel files must have distinct names: outputs are written as OUTDIR/<name>.wav")
+    model, sr = _load_vocoder(args.ckpt, p)
+    sr = args.sampling_rate or sr
+    mels = [_read_mel(f, model.n_mels, p) for f in args.mels]
+    from .base import pad_batch
+    dev = torch.device("cuda")
+    model = model.to(dev).eval()
+    hop = model._hop_length
+    os.makedirs(args.outdir, exist_ok=True)
+    order = sorted(range(len(mels)), key=lambda i: mels[i].shape[-1])
+    # families without per-item lengths (WaveFlow, WSRGlow, ...) synthesise one utterance per call
+    max_batch = args.max_batch if model._supports_lengths else 1
+    with torch.no_grad():
+        denoiser = _denoiser(model, mels[order[0]].shape[-1] * hop, p) if args.denoiser_strength > 0 else None
+        total, cost = 0, 0.0
+        for s0 in range(0, len(order), max_batch):
+            idx = order[s0:s0 + max_batch]
+            h, frames = pad_batch([mels[i] for i in idx])
+            z = torch.zeros((len(idx), h.shape[-1] * hop))
+            for j, i in enumerate(idx):
+                z[j, :frames[j] * hop] = item_noise(args.seed, i, frames[j] * hop, args.sigma)
+            h, z = h.to(dev), z.to(dev)
+            lengths = frames if model._supports_lengths else None
+            x, dt = _timed(lambda: model.infer(h, args.sigma, z=z, lengths=lengths).reshape(len(idx), -1))
+            cost += dt
+            if denoiser is not None:
+                x = denoiser(x, args.denoiser_strength, lengths=[f * hop for f in frames] if lengths else None)
+            for j, i in enumerate(idx):
+                n = frames[j] * hop
+                total += n
+                wav_write(os.path.join(args.outdir, stems[i] + ".wav"), x[j, :n].reshape(1, -1).cpu(), sr)
+    print("{} files, {} samples, synthesis {:.4f} s, {:.4f} kHz".format(len(mels), total, cost, total / max(cost, 1e-9) / 1e3))
+
+
 def main(argv=None) -> None:
     argv = list(sys.argv[1:] if argv is None else argv)
-    verbs = {"train": train, "synth": synth, "synth-batch": synth_batch}
+    verbs = {"train": train, "synth": synth, "synth-batch": synth_batch, "vocode": vocode}
     if not argv or argv[0] not in verbs:
-        raise SystemExit("usage: python -m constant_memory_waveglow_b200.cli {train,synth,synth-batch} [flags]  "
+        raise SystemExit("usage: python -m constant_memory_waveglow_b200.cli {train,synth,synth-batch,vocode} [flags]  "
                          "(-h after the verb)")
     verbs[argv[0]](argv[1:])
 

@@ -61,6 +61,16 @@ class NonCausalLayer(nn.Module):
 # ---------------------------------------------------------------------------------------------
 # conditioning cache: the slab-layout copy of y is built once and reused by all flows / recomputes
 # ---------------------------------------------------------------------------------------------
+class CondSlab:
+    """Conditioning already in the slab layout ``cmwg_cond_pack`` writes ([B*T][auxp], the operand type of `prec`), for a
+    model that produces it directly (NvidiaWaveGlow's upsampler GEMM).  The WN entry points take it in place of the
+    (B, aux, T) fp32 tensor; `shape` is that tensor's shape."""
+    __slots__ = ("data", "shape", "prec")
+
+    def __init__(self, data: Tensor, shape: Tuple[int, int, int], prec: str):
+        self.data, self.shape, self.prec = data, tuple(shape), prec
+
+
 class _CondCache:
     def __init__(self, capacity: int = 3):
         self.capacity = capacity
@@ -68,6 +78,11 @@ class _CondCache:
 
     def get(self, y: Tensor, cfg: L.WnConfig) -> Tensor:
         auxp = L.load().cmwg_wn_aux_padded(C.byref(cfg))
+        if isinstance(y, CondSlab):
+            if L.PREC_NAMES[y.prec] != cfg.precision or y.data.numel() != y.shape[0] * y.shape[2] * auxp:
+                raise RuntimeError(f"WN: conditioning slab of precision {y.prec} and {y.data.numel()} elements does not "
+                                   f"match this WN ({auxp} padded channels, precision code {cfg.precision})")
+            return y.data
         key = (y.untyped_storage().data_ptr(), y.storage_offset(), tuple(y.shape), tuple(y.stride()), y._version,
                auxp, cfg.precision, y.device.index)
         hit = self.entries.get(key)
@@ -254,7 +269,7 @@ class WN(nn.Module):
         """x: (B, >=cin, T) NCL whose first `cin` channels are the WN input.  Returns (lst, state):
         lst (B, 2cin, T) = [log_s ; t].  `transient`: the saved activations are consumed by a `_cmwg_backward` call that
         follows immediately (the constant-memory recompute), so they may live in the per-stream scratch buffer."""
-        L.require_cuda(x, y, op="WN.forward")
+        L.require_cuda(x, y.data if isinstance(y, CondSlab) else y, op="WN.forward")
         if prec is None:
             prec = precision.resolve(self._tc_supported(), training=save)
         cfg, packed, ps = self._prepare(prec, x.device)
@@ -263,7 +278,7 @@ class WN(nn.Module):
         B, _, T = x.shape
         if y.shape[0] != B or y.shape[1] != self.aux_chs or y.shape[2] != T:
             raise RuntimeError(f"WN: conditioning shape {tuple(y.shape)} does not match input {(B, self.aux_chs, T)}")
-        if y.dtype != torch.float32:
+        if not isinstance(y, CondSlab) and y.dtype != torch.float32:
             y = y.float()
         ycl = _cond_cache.get(y, cfg)
         ws = self._scratch_buf(int(lib.cmwg_wn_workspace_bytes(C.byref(cfg), B, T)), x.device, "ws")
@@ -282,14 +297,14 @@ class WN(nn.Module):
     def _cmwg_forward_varlen(self, x: Tensor, y: Tensor, lengths_host, lengths_dev: Tensor, prec: str) -> Tensor:
         """Inference over a padded batch: lst (B, 2cin, T) whose columns t < lengths[b] equal the WN of item b alone
         (cmwg_wn_forward_varlen); lengths_host is a ctypes int array, lengths_dev the same values as a device int32 tensor."""
-        L.require_cuda(x, y, op="WN.forward")
+        L.require_cuda(x, y.data if isinstance(y, CondSlab) else y, op="WN.forward")
         cfg, packed, _ = self._prepare(prec, x.device)
         lib = L.load()
         x = ops._ncl(x)
         B, _, T = x.shape
         if y.shape[0] != B or y.shape[1] != self.aux_chs or y.shape[2] != T:
             raise RuntimeError(f"WN: conditioning shape {tuple(y.shape)} does not match input {(B, self.aux_chs, T)}")
-        ycl = _cond_cache.get(y if y.dtype == torch.float32 else y.float(), cfg)
+        ycl = _cond_cache.get(y if isinstance(y, CondSlab) or y.dtype == torch.float32 else y.float(), cfg)
         ws = self._scratch_buf(int(lib.cmwg_wn_varlen_workspace_bytes(C.byref(cfg), B, T)), x.device, "ws")
         lst = torch.empty((B, 2 * self.in_chs, T), device=x.device, dtype=torch.float32)
         L.check(lib.cmwg_wn_forward_varlen(C.byref(cfg), packed.data_ptr(), x.data_ptr(), ops._bstride(x), ycl.data_ptr(),

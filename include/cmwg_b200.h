@@ -371,6 +371,24 @@ int cmwg_upsample_dense_bwd(const float* h, const float* g, const float* v, cons
                             int C, int F, int K, int stride, int pad, int rpad, float slope, float* dg, float* dv,
                             float* dbias, void* workspace, void* stream);
 
+/* Conditioning of NVIDIA's WaveGlow (NVIDIA/waveglow glow.py): ConvTranspose1d(C, C, taps * hop, stride = hop) with
+ * bias, no weight norm, then unfolded by n_group, computed as one tcgen05 GEMM that writes the 16-bit WN conditioning
+ * slab (the layout cmwg_cond_pack writes, C * n_group channels) directly:
+ *   slab[b][t][c] = up[b, c / n_group, n_group t + c % n_group],
+ *   up[b, o, hop q + r] = bias[o] + sum_{j < taps} sum_i w[i, o, r + hop j] * mel[b, i, q - j]   (mel = 0 outside [0, F)).
+ * w is the (C, C, taps * hop) fp32 weight; `packed` (cmwg_nvidia_upsample_packed_bytes) is its GEMM operand, written by
+ * cmwg_nvidia_upsample_pack once per weight version.  mel (B, C, F) fp32 with unit frame stride; T squeezed steps per
+ * item (any T >= 0: frames past F contribute nothing, rows past T are not written); precision CMWG_PREC_FP16 / _BF16.
+ * C * n_group must be a multiple of 64 (else CMWG_ERR_UNSUPPORTED) and n_group must divide hop.
+ * workspace: cmwg_nvidia_upsample_workspace_bytes(B, T, C, hop, taps, n_group) bytes. */
+size_t cmwg_nvidia_upsample_packed_bytes(int C, int hop, int taps);
+int cmwg_nvidia_upsample_pack(const float* w, int C, int hop, int taps, int n_group, int precision, void* packed,
+                              void* stream);
+size_t cmwg_nvidia_upsample_workspace_bytes(int B, int T, int C, int hop, int taps, int n_group);
+int cmwg_nvidia_upsample_slab(const void* packed, const float* bias, const float* mel, long long mel_bstride,
+                              long long mel_cstride, int B, int C, int F, int hop, int taps, int n_group, int T,
+                              int precision, void* slab, void* workspace, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Model glue (model/waveglow.py:153,179; model/loss.py:10-15)
  * ------------------------------------------------------------------------------------------- */
