@@ -16,10 +16,11 @@ from .wsrglow import WSRGlow
 from .mr_waveglow import MRWaveGlow
 from .melglow import MelGlow, WN_LVC
 from .denoiser import Denoiser
+from .condition import MelSpec, TacotronSTFT
 from .nvidia import NvidiaWaveGlow, load_nvidia_waveglow
 
 __all__ = ["FlowBase", "Reversible", "AffineCouplingBlock", "InvertibleConv1x1", "AffineCouplingFunc",
            "InvAffineCouplingFunc", "Conv1x1Func", "InvConv1x1Func", "WaveGlowLoss", "WN", "NonCausalLayer",
            "WaveGlow", "WSRGlow", "MRWaveGlow", "MelGlow", "WN_LVC", "WaveFlow", "WN2D", "NonCausalLayer2D", "fused_gate", "add_weight_norms", "remove_weight_norms", "get_instance", "set_precision",
            "get_precision", "invalidate_packs", "pad_batch", "Denoiser",
-           "NvidiaWaveGlow", "load_nvidia_waveglow"]
+           "NvidiaWaveGlow", "load_nvidia_waveglow", "MelSpec", "TacotronSTFT"]

@@ -92,6 +92,8 @@ SIGNATURES = {
                               _VP, _VP, _LL, _VP, C.POINTER(WnGrads), _VP]),
     "cmwg_melspec_frames": (_I, [_I, _I, _I]),
     "cmwg_melspec_fwd": (_I, [_VP, _LL, _I, _I, _VP, _VP, _VP, _VP, _I, _I, _I, _I, C.c_float, _I, _VP, _VP]),
+    "cmwg_melspec_fwd_varlen": (_I, [_VP, _LL, _I, _I, C.POINTER(C.c_int), _VP, _VP, _VP, _VP, _VP, _I, _I, _I, _I, _I,
+                                     _I, C.c_float, _VP, _VP]),
     "cmwg_denoise_workspace_bytes": (_SZ, [_I, _I, _I, _I]),
     "cmwg_stft_frame_magnitude": (_I, [_VP, _I, _VP, _I, _I, _I, _VP, _VP]),
     "cmwg_denoise": (_I, [_VP, _LL, _I, _I, C.POINTER(C.c_int), _VP, _VP, _VP, C.c_float, _I, _I, _VP, _VP, _VP]),

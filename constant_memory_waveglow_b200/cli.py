@@ -1,4 +1,4 @@
-"""Command line of the harness: ``python -m constant_memory_waveglow_b200.cli {train,synth,synth-batch,vocode} ...``.
+"""Command line of the harness: ``python -m constant_memory_waveglow_b200.cli {train,synth,synth-batch,vocode,score} ...``.
 
 The reference's own ``train.py`` runs unchanged on the ``pytorch_lightning`` / ``model`` / ``datasets`` shims at the
 repository root; its ``inference.py`` cannot in this image (``torchaudio.load`` / ``save`` need the absent TorchCodec),
@@ -7,7 +7,10 @@ RIFF reader/writer of ``datasets.py``.  Multi-GPU: launch ``train`` under ``torc
 re-synthesises many files, batching utterances of different lengths into one call each (``WaveGlow.infer(lengths=...)``).
 ``-d/--denoiser-strength`` on ``synth`` and ``synth-batch`` runs the bias-spectrum ``Denoiser`` on the output (one call per
 batch, with the per-item lengths); at 0, the default, it is skipped.  ``vocode`` synthesises mel spectrogram files (.pt /
-.npy, as NVIDIA's ``inference.py`` reads them) with an NVIDIA WaveGlow checkpoint or this package's, batched the same way.
+.npy, as NVIDIA's ``inference.py`` reads them) with an NVIDIA WaveGlow checkpoint or this package's, batched the same way;
+given ``.wav`` files it computes their mels first (Tacotron2's ``TacotronSTFT`` for NVIDIA checkpoints, the checkpoint's
+conditioner otherwise): copy synthesis.  ``score`` prints the per-file negative log-likelihood of WAV files under a
+checkpoint, in the convention of the training loss (``WaveGlowLoss``).
 """
 from __future__ import annotations
 
@@ -214,7 +217,15 @@ def _read_mel(path: str, n_mels: int, p: argparse.ArgumentParser) -> torch.Tenso
 def _load_vocoder(ckpt: str, p: argparse.ArgumentParser):
     """(model on the CPU, default sampling rate) of an NVIDIA WaveGlow checkpoint or of this package's Lightning
     checkpoint, told apart by their contents (read with weights_only=True first either way)."""
+    model, sr, _ = _load_vocoder_frontend(ckpt, p)
+    return model, sr
+
+
+def _load_vocoder_frontend(ckpt: str, p: argparse.ArgumentParser):
+    """(model, default sampling rate, mel front end), on the CPU.  The front end maps audio to the model's mels:
+    Tacotron2's TacotronSTFT for an NVIDIA checkpoint, the checkpoint's conditioner for this package's."""
     from . import nvidia
+    from .condition import TacotronSTFT
     try:
         obj = nvidia._read_checkpoint(ckpt)
     except Exception as e:
@@ -223,16 +234,53 @@ def _load_vocoder(ckpt: str, p: argparse.ArgumentParser):
             and any(k.startswith("model.") for k in obj["state_dict"]):
         lit = TR.LightModel.load_from_checkpoint(ckpt, map_location="cpu")
         lit.model.apply(remove_weight_norms)
-        return lit.model, int(lit.conditioner.sample_rate)
-    return nvidia.load_nvidia_waveglow(obj, device="cpu"), 22050
+        return lit.model, int(lit.conditioner.sample_rate), lit.conditioner
+    model = nvidia.load_nvidia_waveglow(obj, device="cpu")
+    return model, 22050, TacotronSTFT(n_mel_channels=model.n_mels, sampling_rate=22050)
+
+
+def _frontend_rate(frontend) -> int:
+    return int(getattr(frontend, "sampling_rate", None) or frontend.sample_rate)
+
+
+def _read_wav_mono(path: str, rate: int, p: argparse.ArgumentParser) -> torch.Tensor:
+    """A WAV file as one channel (the mean of its channels); its sampling rate must be `rate` (there is no resampler)."""
+    from .datasets import wav_info
+    sr = wav_info(path).sample_rate
+    if sr != rate:
+        p.error(f"{path}: sampled at {sr} Hz; the model's mel front end expects {rate} Hz (resample it first)")
+    return wav_read(path).mean(0)
+
+
+def _frontend_mels(frontend, signals, names, max_batch: int, dev, p: argparse.ArgumentParser):
+    """Mels of 1-D signals (on the CPU), one front-end call per length-sorted group of `max_batch` with per-item
+    lengths; item i gets signals[i].numel() // hop + 1 frames.  Returns CPU tensors (n_mels, frames) in input order."""
+    from .base import pad_batch
+    from .condition import MelSpec, TacotronSTFT
+    batched = isinstance(frontend, (MelSpec, TacotronSTFT))
+    step = max_batch if batched else 1
+    order = sorted(range(len(signals)), key=lambda i: signals[i].numel())
+    hop = frontend.hop_length
+    out = [None] * len(signals)
+    for s0 in range(0, len(order), step):
+        idx = order[s0:s0 + step]
+        x, lens = pad_batch([signals[i] for i in idx])
+        try:
+            m = frontend(x.to(dev), lengths=lens) if batched else frontend(x.to(dev))
+        except ValueError as e:
+            p.error(f"{', '.join(names[i] for i in idx)}: {e}")
+        for j, i in enumerate(idx):
+            out[i] = m[j, :, :lens[j] // hop + 1].cpu()
+    return out
 
 
 def vocode(argv) -> None:
-    p = argparse.ArgumentParser(prog="cli vocode", description="synthesis from mel spectrograms (.pt / .npy), batched by "
-                                "length; NVIDIA WaveGlow or this package's checkpoints")
+    p = argparse.ArgumentParser(prog="cli vocode", description="synthesis from mel spectrograms (.pt / .npy) or from the "
+                                "mels of WAV files (copy synthesis), batched by length; NVIDIA WaveGlow or this package's "
+                                "checkpoints")
     p.add_argument("ckpt", type=str)
     p.add_argument("outdir", type=str)
-    p.add_argument("mels", type=str, nargs="+")
+    p.add_argument("mels", type=str, nargs="+", help=".pt / .npy mel spectrograms or .wav files (at the front end's rate)")
     p.add_argument("-s", "--sigma", type=float, default=0.6)
     p.add_argument("--max-batch", type=int, default=16, help="utterances per synthesis call")
     p.add_argument("--seed", type=int, default=0, help="noise seed; file i draws from a generator seeded by (seed, i)")
@@ -248,13 +296,24 @@ def vocode(argv) -> None:
     stems = [os.path.splitext(os.path.basename(f))[0] for f in args.mels]
     if len(set(stems)) != len(stems):
         p.error("mel files must have distinct names: outputs are written as OUTDIR/<name>.wav")
-    model, sr = _load_vocoder(args.ckpt, p)
+    model, sr, frontend = _load_vocoder_frontend(args.ckpt, p)
     sr = args.sampling_rate or sr
-    mels = [_read_mel(f, model.n_mels, p) for f in args.mels]
+    is_wav = [f.lower().endswith(".wav") for f in args.mels]
+    mels = [None if w else _read_mel(f, model.n_mels, p) for f, w in zip(args.mels, is_wav)]
+    wav_idx = [i for i, w in enumerate(is_wav) if w]
+    signals = [_read_wav_mono(args.mels[i], _frontend_rate(frontend), p) for i in wav_idx]
     from .base import pad_batch
     dev = torch.device("cuda")
     model = model.to(dev).eval()
     hop = model._hop_length
+    # WAV inputs: mels from the front end, one call per batch with the per-item lengths; the output keeps each file's
+    # sample count (the model gives frames * hop >= samples + 1)
+    n_out = {}
+    if wav_idx:
+        with torch.no_grad():
+            wav_mels = _frontend_mels(frontend.to(dev), signals, [args.mels[i] for i in wav_idx], args.max_batch, dev, p)
+        for i, m, x in zip(wav_idx, wav_mels, signals):
+            mels[i], n_out[i] = m, x.numel()
     os.makedirs(args.outdir, exist_ok=True)
     order = sorted(range(len(mels)), key=lambda i: mels[i].shape[-1])
     # families without per-item lengths (WaveFlow, WSRGlow, ...) synthesise one utterance per call
@@ -275,17 +334,75 @@ def vocode(argv) -> None:
             if denoiser is not None:
                 x = denoiser(x, args.denoiser_strength, lengths=[f * hop for f in frames] if lengths else None)
             for j, i in enumerate(idx):
-                n = frames[j] * hop
+                n = n_out.get(i, frames[j] * hop)
                 total += n
                 wav_write(os.path.join(args.outdir, stems[i] + ".wav"), x[j, :n].reshape(1, -1).cpu(), sr)
     print("{} files, {} samples, synthesis {:.4f} s, {:.4f} kHz".format(len(mels), total, cost, total / max(cost, 1e-9) / 1e3))
 
 
+def score(argv) -> None:
+    p = argparse.ArgumentParser(prog="cli score", description="per-file negative log-likelihood of WAV files under an NVIDIA "
+                                "WaveGlow or a package checkpoint, per sample as the training loss (WaveGlowLoss) gives it")
+    p.add_argument("ckpt", type=str)
+    p.add_argument("wavs", type=str, nargs="+")
+    p.add_argument("-s", "--sigma", type=float, default=1.0, help="of the loss (NVIDIA trains with 1.0)")
+    p.add_argument("--max-batch", type=int, default=16, help="files per forward call")
+    args = p.parse_args(argv)
+    if args.max_batch < 1:
+        p.error("--max-batch must be >= 1")
+    if not 0 < args.sigma < math.inf:
+        p.error("--sigma must be a finite number > 0")
+    for path, n, nll in score_files(args.ckpt, args.wavs, args.sigma, args.max_batch, p):
+        print(f"{path}\t{n}\t{nll:.6f}")
+
+
+def score_files(ckpt: str, paths, sigma: float, max_batch: int, p: argparse.ArgumentParser):
+    """[(path, samples, NLL)] in input order.  Each file, cut to a multiple of n_group, gets WaveGlowLoss(sigma) of its own
+    forward call: 0.5 sum z^2 / sigma^2 - log-det, over its samples.  Files run in length-sorted batches through
+    forward(x, mel, lengths=...), which gives every item its own call's z and log-det bit for bit; families without
+    per-item lengths run one file per call."""
+    from .base import pad_batch
+    from .loss import WaveGlowLoss
+    from .nvidia import NvidiaWaveGlow
+    model, _, frontend = _load_vocoder_frontend(ckpt, p)
+    g, hop = getattr(model, "n_group", 1), model._hop_length
+    signals = []
+    for f in paths:
+        x = _read_wav_mono(f, _frontend_rate(frontend), p)
+        signals.append(x[:x.numel() - x.numel() % g])
+    dev = torch.device("cuda")
+    model, frontend = model.to(dev).eval(), frontend.to(dev)
+    with torch.no_grad():
+        mels = _frontend_mels(frontend, signals, list(paths), max_batch, dev, p)
+    # The batched path conditions item b on its first ceil(n_b / hop) mel frames (the frames infer() synthesises from).
+    # The front end gives n / hop + 1 frames, one more when hop divides n, and this package's upsampler reaches back from
+    # that frame into the item's last samples; such files run alone.  NVIDIA's upsampler only reaches forward.
+    alone = [not model._supports_lengths or (x.numel() % hop == 0 and not isinstance(model, NvidiaWaveGlow)) for x in signals]
+    order = sorted((i for i in range(len(paths)) if not alone[i]), key=lambda i: signals[i].numel())
+    groups = [order[s0:s0 + max_batch] for s0 in range(0, len(order), max_batch)] + [[i] for i in range(len(paths)) if alone[i]]
+    loss = WaveGlowLoss(sigma)
+    nll = [None] * len(paths)
+    with torch.no_grad():
+        for idx in groups:
+            x, lens = pad_batch([signals[i] for i in idx])
+            h, _ = pad_batch([mels[i] for i in idx])
+            x, h = x.to(dev), h.to(dev)
+            if len(idx) == 1:
+                z, logdet = model(x, h)
+            else:
+                z, logdet = model(x, h, lengths=lens)
+            z = z.reshape(len(idx), -1)
+            logdet = logdet.reshape(len(idx))
+            for j, i in enumerate(idx):
+                nll[i] = float(loss(z[j:j + 1, :lens[j]].clone(), logdet[j:j + 1].clone()))
+    return [(f, signals[i].numel(), nll[i]) for i, f in enumerate(paths)]
+
+
 def main(argv=None) -> None:
     argv = list(sys.argv[1:] if argv is None else argv)
-    verbs = {"train": train, "synth": synth, "synth-batch": synth_batch, "vocode": vocode}
+    verbs = {"train": train, "synth": synth, "synth-batch": synth_batch, "vocode": vocode, "score": score}
     if not argv or argv[0] not in verbs:
-        raise SystemExit("usage: python -m constant_memory_waveglow_b200.cli {train,synth,synth-batch,vocode} [flags]  "
+        raise SystemExit("usage: python -m constant_memory_waveglow_b200.cli {train,synth,synth-batch,vocode,score} [flags]  "
                          "(-h after the verb)")
     verbs[argv[0]](argv[1:])
 

@@ -281,6 +281,20 @@ int cmwg_melspec_frames(int T, int n_fft, int hop);
 int cmwg_melspec_fwd(const float* x, long long x_bstride, int B, int T, const float* window, const float* fbt,
                      const int* fb_lo, const int* fb_hi, int n_fft, int hop, int n_mels, int power_is_one, float eps,
                      int take_log, float* out, void* stream);
+/* The same transform over a zero-padded batch with per-item lengths, a free left pad and a choice of log; serves MelSpec
+ * with lengths and TacotronSTFT.mel_spectrogram (Tacotron2's layers.py / stft.py: reflect pad n_fft/2, |STFT|, mel,
+ * log(clamp(., 1e-5))).  Item b is framed over its own len_b samples (len_b = lengths[b], or T when both length pointers
+ * are NULL) with reflection at its own end: frame f starts at sample f * hop - pad_left, and item b has len_b / hop + 1
+ * frames; out (B, n_mels, T / hop + 1) holds 0 in the frames after them.  Nothing past len_b is read, so every item equals
+ * its own call (B = 1, T = len_b) bit for bit.
+ *   pad_left: n_fft/2 - hop/2 for MelSpec, n_fft/2 for Tacotron2; lengths in (max(pad_left, n_fft - pad_left), T].
+ *   log_mode: 0 -> v, 1 -> log(v + eps) (then equal to cmwg_melspec_fwd bit for bit when pad_left = n_fft/2 - hop/2),
+ *   2 -> log(max(v, eps)); v the mel value.  eps finite and >= 0.  Other arguments as cmwg_melspec_fwd.
+ *   CMWG_ERR_ARG for a bad length, log_mode, eps or n_fft. */
+int cmwg_melspec_fwd_varlen(const float* x, long long x_bstride, int B, int T, const int* lengths_host,
+                            const int* lengths_dev, const float* window, const float* fbt, const int* fb_lo,
+                            const int* fb_hi, int n_fft, int hop, int n_mels, int pad_left, int power_is_one,
+                            int log_mode, float eps, float* out, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Denoiser of synthesised audio: bias-spectrum subtraction, the `Denoiser` of NVIDIA's WaveGlow (denoiser.py, mode 'zeros',
