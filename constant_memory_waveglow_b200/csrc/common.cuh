@@ -147,26 +147,11 @@ __device__ __forceinline__ float sigmoid_ex2(float x) { return __fdividef(1.f, 1
 // tanh(x), sigmoid(y) and their product with ONE reciprocal:  E1 = e^(2x), E2 = e^(-y), r = 1 / ((E1 + 1)(1 + E2));
 //   tanh = (E1 - 1)(1 + E2) r,  sigmoid = (E1 + 1) r,  tanh * sigmoid = (E1 - 1) r.
 // x is clamped above at 15 (tanh = 1 to fp32 precision beyond 9.1) and y below at -30 so that the product stays finite.
-// 2^t on the FMA / integer pipes, no MUFU: t = n + f with n the nearest integer (magic-number rounding), a degree-4 polynomial
-// for 2^f on [-0.5, 0.5] (max relative error 3.1e-6), the exponent patched in by integer addition.  |t| <= 125.
-__device__ __forceinline__ float exp2_fma(float t) {
-  const float r = t + 12582912.f;            // 1.5 * 2^23: the low mantissa bits of r hold n
-  const float f = t - (r - 12582912.f);
-  float p = fmaf(0.00960039534f, f, 0.0559168942f);
-  p = fmaf(p, f, 0.240237191f);
-  p = fmaf(p, f, 0.69312197f);
-  p = fmaf(p, f, 1.0f);
-  return __int_as_float(__float_as_int(p) + (__float_as_int(r) << 23));   // (bits of r) << 23 == n << 23 (mod 2^32)
-}
-// POLY: e^(-y) by exp2_fma instead of MUFU.EX2.  The gate epilogue of the task kernels is bound by the MUFU pipe (16 lanes per
-// clock per SM: 3 operations x 128 x 128 gate values = 3072 cycles per tile against 7168 of MMA, with the residual tiles'
-// epilogues on top); giving every second value's sigmoid exponential to the FMA pipe balances the two pipes (~2500 cycles each).
-template <bool WANT_AB, bool POLY = false>
+template <bool WANT_AB>
 __device__ __forceinline__ void gate_ex2(float x, float y, float& a, float& b, float& g) {
   float e1, e2, r;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e1) : "f"(fminf(x, 15.f) * 2.885390082f));   // 2 log2(e)
-  if (POLY) e2 = exp2_fma(fminf(fmaxf(y, -30.f), 86.f) * -1.442695041f);
-  else asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e2) : "f"(fmaxf(y, -30.f) * -1.442695041f));
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e2) : "f"(fmaxf(y, -30.f) * -1.442695041f));
   const float p = e1 + 1.f, q = 1.f + e2, m = e1 - 1.f;
   asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(p * q));
   g = m * r;

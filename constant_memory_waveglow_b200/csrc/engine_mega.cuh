@@ -12,8 +12,8 @@
 // and CTA pair p runs tasks p, p + P, p + 2P, ... (P pairs, all co-resident).  Dependencies are per ROW TILE, not per
 // layer: R(i, rt) needs G(i, rt, *); G(i, rt, *) needs R(i-1, rt-1 .. rt+1) (the dilated taps reach at most one
 // 256-row tile away); S(rt) needs G(depth-1, rt, *).  They are tracked by counters in global memory: every epilogue warp
-// adds 1 (release) to its task's counter once its TMA stores have COMPLETED, and the TMA producer (and, for R, the
-// epilogue's input loader) polls (acquire) before it issues loads.  The list is in dependency order and a pair executes
+// adds 1 (release) to its task's counter once its TMA stores have COMPLETED, and the scout warp (for the TMA producer) and,
+// for R, the epilogue's input loader poll (acquire) before loads are issued.  The list is in dependency order and a pair executes
 // its tasks in list order, so the lowest unfinished task is always runnable: no deadlock as long as all pairs are
 // resident (grid <= SM count / 2, one CTA per SM).  A wait that exceeds ~2 s traps instead of hanging the device.
 //
@@ -81,21 +81,10 @@ struct alignas(64) MegaParams {
   uint32_t idesc, desc_lbo, desc_sbo;
   int lag;                      // residual tiles trail their gate tiles by `lag` row-tile slots (< RT - 1)
   int total_tasks;
-  int lagged;                   // signal a unit's completion one unit later (its stores complete behind the next unit's work)
   long long* clk;               // nullptr, or [CTAs][18 warps][16] cycle accumulators (CMWG_MEGA_CLK: where the roles wait)
-  int dbg;                      // timing experiments only (CMWG_MEGA_DBG): 1 no producer waits, 2 no signals, 4 no wait_all
-  int dual;                     // 1: warp MEGA_BWARP issues the weight tiles (default), 0: warp 0 issues both operands
+  int res_lo;                   // 1: the residual stream is a (hi, lo) pair of 16-bit slabs; 0: the operand slab alone (AddTcEpi)
   // `end` conv fused into the skip tiles' epilogue (model/waveglow.py:92,105): lst[b][o][t] = sum_c w_end[o][c] * cum_skip[b][t][c].
   // lst == nullptr: off (the fp32 skip slab is written and a separate kernel reads it back).
-  // Residual tiles with DIRECT global loads / stores of the (hi, lo) pairs (row-per-thread 32-byte vectors) instead of TMA
-  // chunks through the staging buffers: the small epilogue transfers no longer queue behind the operand stream in the SM's
-  // TMA unit (res_direct = 0: the TMA path).
-  const uint16_t* hi_ptr[MEGA_D];   // layer inputs, hi halves  [rows][Cr]
-  uint16_t* lo_ptr[MEGA_D];         // layer inputs, lo halves
-  uint16_t* hi_out_ptr[MEGA_D];     // same slabs, writable view (hi_out_ptr[i] = hi_ptr[i])
-  int res_direct;
-  int res_lo;                   // 1: the residual stream is a (hi, lo) pair of 16-bit slabs; 0: the operand slab alone (AddTcEpi)
-  int gate_mix;                 // GateTcEpi::mix
   float* lst;                   // (B, cout, T) fp32 NCL
   const float* w_end;           // [MEGA_END_MAXC][Cs] fp32, rows >= cout zero
   int cout;
@@ -139,10 +128,6 @@ __device__ __forceinline__ void red_release_add_u32(uint32_t* p, uint32_t v) {
 // the producer ~700 cycles per task with five TMA stages in flight.
 __device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void bulk_wait_complete() {  // all but the N most recent bulk groups of this thread are COMPLETE
-  asm volatile("cp.async.bulk.wait_group %0;" ::"n"(N) : "memory");
-}
 // completion signal of one unit (one TMEM buffer's worth of epilogue) of one warp
 struct MegaSig {
   uint32_t* flag;     // global dependency counter (nullptr: nothing depends on this unit)
@@ -182,8 +167,7 @@ __device__ __forceinline__ uint32_t ld_relaxed_u32(const uint32_t* p) {
   return v;
 }
 // up to three counters polled with independent relaxed loads (one L2 round trip), then one acquire fence
-__device__ __forceinline__ void mega_wait_flags3(const uint32_t* a, const uint32_t* b, const uint32_t* c, uint32_t target,
-                                                 bool fence = true) {
+__device__ __forceinline__ void mega_wait_flags3(const uint32_t* a, const uint32_t* b, const uint32_t* c, uint32_t target) {
   const long long t0 = clock64();
   while (true) {
     const uint32_t va = ld_relaxed_u32(a), vb = ld_relaxed_u32(b), vc = ld_relaxed_u32(c);
@@ -191,7 +175,7 @@ __device__ __forceinline__ void mega_wait_flags3(const uint32_t* a, const uint32
     __nanosleep(40);
     if (clock64() - t0 > MEGA_WAIT_LIMIT) mega_timeout(b, target);
   }
-  if (fence) asm volatile("fence.acq_rel.gpu;" ::: "memory");
+  asm volatile("fence.acq_rel.gpu;" ::: "memory");
 }
 
 struct MegaTask {
@@ -229,15 +213,14 @@ __device__ __forceinline__ uint32_t* mega_rflag(const MegaParams& p, int layer, 
 
 // Epilogue of ONE task for one warp: GW epilogue columns per tile, four column groups (one per warp of the lane quadrant).
 // kIn > 0: in-place staging -- chunk inputs are TMA-loaded into the buffers the outputs are later stored from; the
-// caller has already issued chunk 0's inputs and made sure the staging buffers are free.  Immediate mode: ends with ALL
-// of this warp's stores complete, then signals `flag`.  Lagged mode (`prev` != nullptr): waits only for the PREVIOUS unit's
-// stores (which completed behind this unit's work), signals that unit and leaves this one pending in `prev`.
+// caller has already issued chunk 0's inputs and made sure the staging buffers are free.  Ends with ALL of this warp's
+// stores complete, then signals `sig`.
 template <class Epi, int GW>
 __device__ __forceinline__ void mega_epilogue_task(const Epi& epi, uint32_t tmem_tile, uint64_t* tmem_full, uint32_t full_phase,
                                                    uint32_t tmem_empty_remote, int q, int cg, int lane, uint32_t wbuf,
                                                    uint64_t* ibar, uint32_t& it, const CUtensorMap* om0,
                                                    const CUtensorMap* om1, const CUtensorMap* om2, const CUtensorMap* im0,
-                                                   const CUtensorMap* im1, int b, int r0, int cbase, MegaSig sig, MegaSig* prev, int dbg, uint32_t* tt,
+                                                   const CUtensorMap* im1, int b, int r0, int cbase, MegaSig sig, uint32_t* tt,
                                                    bool dead = false) {
   constexpr int NCH = GW / 128;                      // 32-column chunks per warp
   constexpr int OUTW = Epi::kOutF32 ? 16 : 8;
@@ -345,89 +328,13 @@ __device__ __forceinline__ void mega_epilogue_task(const Epi& epi, uint32_t tmem
   }
   const uint32_t c_c = (uint32_t)clock();
   if (lane == 0) {
-    if (dbg & 2) sig.flag = nullptr;
-    if (prev != nullptr) {
-      bulk_wait_complete<NCH * (Epi::kOut > 2 ? 2 : 1)>();  // this unit's own groups may be pending, everything older is complete
-      mega_signal(*prev);
-      *prev = sig;
-    } else {
-      bulk_wait_all();            // stores COMPLETE (not just read): the results are in global memory
-      mega_signal(sig);
-    }
+    bulk_wait_all();            // stores COMPLETE (not just read): the results are in global memory
+    mega_signal(sig);
   }
   __syncwarp();
   tt[0] += c_b - c_a;            // waiting for the accumulator
   tt[1] += c_c - c_b;            // drain + functor + staging + store issue (+ input waits)
   tt[2] += (uint32_t)clock() - c_c;  // store completion + signal
-  tt[3] += 1;
-}
-
-__device__ __forceinline__ void ldg256_cg(const void* p, uint32_t (&r)[8]) {   // L2 only: the slabs are rewritten by other SMs
-  asm volatile("ld.global.cg.v8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-               : "l"(p)
-               : "memory");
-}
-__device__ __forceinline__ void stg256(void* p, const uint32_t (&r)[8]) {
-  asm volatile("st.global.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(p), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]),
-               "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
-               : "memory");
-}
-
-// In-place tile (two 16-bit input streams, two output streams, 256 columns) without TMA: thread = accumulator row, a warp owns
-// 64 columns = four 16-column steps of one 32-byte vector per stream; the loads of step k + 2 are in flight while step k is
-// computed.  in0 / in1 / out0 / out1 point at this thread's row (element offset of the warp's first column included) or are
-// nullptr for rows beyond T.  Ends with every lane's stores fenced and ONE release by lane 0.
-template <class Epi>
-__device__ __forceinline__ void mega_inplace_direct(const Epi& epi, uint32_t taddr, uint64_t* tmem_full, uint32_t full_phase,
-                                                    uint32_t tmem_empty_remote, int lane, int col0, const uint16_t* in0,
-                                                    const uint16_t* in1, uint16_t* out0, uint16_t* out1, MegaSig sig,
-                                                    uint32_t* tt) {
-  uint32_t buf[2][2][8];   // [step parity][stream][8]
-  const bool valid = out0 != nullptr;
-#pragma unroll
-  for (int k = 0; k < 2; ++k) {
-    if (Epi::kIn > 0 && valid) {
-      ldg256_cg(in0 + 16 * k, buf[k][0]);
-      ldg256_cg(in1 + 16 * k, buf[k][1]);
-    } else {
-#pragma unroll
-      for (int j = 0; j < 8; ++j) buf[k][0][j] = buf[k][1][j] = 0u;
-    }
-  }
-  const uint32_t c_a = (uint32_t)clock();
-  mbar_wait(tmem_full, full_phase);
-  tc_fence_after();
-  const uint32_t c_b = (uint32_t)clock();
-#pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    float v[16];
-    tmem_ld16(taddr + 16 * k, v);
-    if (k == 3) {
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive_cluster(tmem_empty_remote);
-    }
-    uint32_t o[2][8];
-    if constexpr (Epi::kIn > 0) epi.compute(col0 + 16 * k, v, buf[k & 1], o);
-    else epi.compute(col0 + 16 * k, v, o);
-    if (Epi::kIn > 0 && k + 2 < 4 && valid) {
-      ldg256_cg(in0 + 16 * (k + 2), buf[k & 1][0]);
-      ldg256_cg(in1 + 16 * (k + 2), buf[k & 1][1]);
-    }
-    if (valid) {
-      stg256(out0 + 16 * k, o[0]);
-      stg256(out1 + 16 * k, o[1]);
-    }
-  }
-  const uint32_t c_c = (uint32_t)clock();
-  __threadfence();          // this lane's stores are visible device-wide ...
-  __syncwarp();             // ... before lane 0 publishes the tile
-  if (lane == 0) mega_signal(sig);
-  __syncwarp();
-  tt[0] += c_b - c_a;
-  tt[1] += c_c - c_b;
-  tt[2] += (uint32_t)clock() - c_c;
   tt[3] += 1;
 }
 
@@ -601,7 +508,6 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
   tc_setup<STAGES>(s, warp, lane, 2 * MEGA_BN, TC_EPI_WARPS);
   const uint32_t tmem_base = *s.tmem_ptr;
   pdl_wait();
-  const int Crp = p.kb_h * TC_BK;
   const uint32_t gtarget = (uint32_t)p.ngt * 2u * TC_EPI_WARPS, rtarget = 2u * TC_EPI_WARPS;
 
   if (warp == 0) {
@@ -612,8 +518,8 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
       uint32_t ntask = 0;
       const long long c_start = clock64();
       const uint32_t full0 = mapa_shared(smem_u32(&s.full[0]), 0);
-      const bool both = p.dual == 0;
-      auto load = [&](const CUtensorMap* am, int ak, int at, int ab, const CUtensorMap* bm, int bk, int bn) {
+      // activation (A) tiles; warp MEGA_BWARP fills the weight half of the same stage
+      auto load = [&](const CUtensorMap* am, int ak, int at, int ab) {
         if (p.clk) {
           const long long c0 = clock64();
           mbar_wait(&s.empty[stage], phase ^ 1);
@@ -623,9 +529,7 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
         }
         const uint32_t sa = smem_u32(s.stages + stage * MEGA_STAGE_BYTES);
         if (rank == 0) mbar_arrive_expect_tx(&s.full[stage], 2 * MEGA_STAGE_BYTES);
-        const uint32_t bar = full0 + 8 * stage;
-        tma_load_4d(sa, am, bar, ak, at, 0, ab);
-        if (both) tma_load_2d(sa + TC_A_BYTES, bm, bar, bk, bn);
+        tma_load_4d(sa, am, full0 + 8 * stage, ak, at, 0, ab);
         if (++stage == STAGES) { stage = 0; phase ^= 1; }
       };
       for (int task = pair; task < p.total_tasks; task += npairs) {
@@ -634,43 +538,26 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
         const MegaTile mt = mega_tile(VARLEN ? p.rt_tab : nullptr, p.tiles_per_batch, t.rt);
         const int b = mt.b, tb = mt.tb;
         const int t0 = tb * (2 * TC_BM) + rank * TC_BM;
-        const int nrow = rank * (MEGA_BN / 2);
         const long long cf = clock64();
-        if (p.dual) {
-          mega_wait_cleared(cleared, ++ntask);       // the scout (warp MEGA_SWARP) has done the waiting
-        } else if (t.type == MEGA_G) {
-          if (t.layer > 0 && !(p.dbg & 1)) {
-            const uint32_t* f1 = mega_rflag(p, t.layer - 1, t.rt);
-            mega_wait_flags3(tb > 0 ? f1 - 1 : f1, f1, tb + 1 < mt.ntb ? f1 + 1 : f1, rtarget, !(p.dbg & 32));
-            if (!(p.dbg & 16)) fence_proxy_async_all();
-          }
-        } else {
-          if (!(p.dbg & 1)) mega_wait_flag(mega_gflag(p, t.type == MEGA_R ? t.layer : p.depth - 1, t.rt), gtarget);
-          if (!(p.dbg & 16)) fence_proxy_async_all();
-        }
+        mega_wait_cleared(cleared, ++ntask);       // the scout (warp MEGA_SWARP) has done the waiting
         w_flag += clock64() - cf;
         const bool f0 = p.fold0 && t.layer == 0;
         if (t.type == MEGA_G) {
-          const int n0 = t.nt * MEGA_BN + nrow;
           if (f0) {
-            for (int kb = 0; kb < p.kb_c; ++kb) load(&p.cond_op, kb * TC_BK, t0, b, &p.pa0f, kb * TC_BK, n0);
+            for (int kb = 0; kb < p.kb_c; ++kb) load(&p.cond_op, kb * TC_BK, t0, b);
           } else {
             for (int sg = 0; sg < p.taps; ++sg) {
               const int shift = (sg - (p.taps - 1) / 2) * (1 << t.layer);
-              for (int kb = 0; kb < p.kb_h; ++kb)
-                load(&p.hin_op[t.layer], kb * TC_BK, t0 + shift, b, &p.pa[t.layer], sg * Crp + kb * TC_BK, n0);
+              for (int kb = 0; kb < p.kb_h; ++kb) load(&p.hin_op[t.layer], kb * TC_BK, t0 + shift, b);
             }
-            for (int kb = 0; kb < p.kb_c; ++kb)
-              load(&p.cond_op, kb * TC_BK, t0, b, &p.pa[t.layer], p.taps * Crp + kb * TC_BK, n0);
+            for (int kb = 0; kb < p.kb_c; ++kb) load(&p.cond_op, kb * TC_BK, t0, b);
           }
         } else if (t.type == MEGA_R) {
-          const CUtensorMap* bm = f0 ? &p.pb0f : &p.pb[t.layer];
-          for (int kb = 0; kb < p.kb_g; ++kb) load(&p.g_op[t.layer], kb * TC_BK, t0, b, bm, kb * TC_BK, nrow);
-          if (f0) load(&p.cond_op, (p.kb_c - 1) * TC_BK, t0, b, bm, p.kb_g * TC_BK, nrow);
+          for (int kb = 0; kb < p.kb_g; ++kb) load(&p.g_op[t.layer], kb * TC_BK, t0, b);
+          if (f0) load(&p.cond_op, (p.kb_c - 1) * TC_BK, t0, b);
         } else {
           for (int j = 0; j < p.depth; ++j)
-            for (int kb = 0; kb < p.kb_g; ++kb)
-              load(&p.g_op[j], kb * TC_BK, t0, b, &p.ps, (j * p.kb_g + kb) * TC_BK, nrow);
+            for (int kb = 0; kb < p.kb_g; ++kb) load(&p.g_op[j], kb * TC_BK, t0, b);
         }
       }
       if (p.clk) {
@@ -679,7 +566,7 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
       }
     }
   } else if (warp == MEGA_SWARP) {
-    if (lane == 0 && p.dual) {
+    if (lane == 0) {
       uint32_t n = 0;
       for (int task = pair; task < p.total_tasks; task += npairs) {
         const MegaTask t = mega_decode(p, task);
@@ -697,7 +584,7 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
       }
     }
   } else if (warp == MEGA_BWARP) {
-    if (lane == 0 && p.dual) {
+    if (lane == 0) {
       // weight tiles of the same task sequence: no dependencies, only free ring slots
       int stage = 0;
       uint32_t phase = 0;
@@ -779,7 +666,7 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
     const uint32_t wbuf = smem_u32(s.epi + e * WB);
     uint64_t* ibar = s.in_bar + e;
     const uint32_t tmem_empty_addr = mapa_shared(smem_u32(&s.tmem_empty[0]), 0);
-    const GateTcEpi<SAVE> gate_epi{nullptr, p.Cd, p.f16, p.gate_mix};
+    const GateTcEpi<SAVE> gate_epi{nullptr, p.Cd, p.f16};
     const SplitTcEpi<true> split_epi{nullptr, p.f16};
     const AddTcEpi add_epi{nullptr, p.f16};
     const RoundTcEpi round_epi{p.f16};
@@ -790,9 +677,6 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
     uint32_t seq = 0;  // units done by this pair; warps of a CTA are never more than two units apart (TMEM double buffer)
     uint32_t tt[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};   // 32-bit cycle counters: a launch is far below 2^32 cycles
     const uint32_t c_start = (uint32_t)clock();
-    MegaSig pending{nullptr, 0};
-    MegaSig* prev = p.lagged ? &pending : nullptr;
-    bool prev_alt = false;  // the previous unit staged through ONE of the two 2 KB buffers (gate tile without saves)
     for (int task = pair; task < p.total_tasks; task += npairs) {
       const MegaTask t = mega_decode(p, task);
       if (t.type == MEGA_NONE) continue;
@@ -806,44 +690,16 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
       const bool alt = !SAVE && t.type == MEGA_G;
       const uint32_t ubuf = wbuf + (alt ? (seq & 1) * TC_CHUNK16_BYTES : 0);
       ++seq;
-      if (p.dbg & 8) {  // timing experiment: no epilogue work at all
-        mbar_wait(&s.tmem_full[acc], acc_phase);
-        tc_fence_after();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(te);
-        acc ^= 1;
-        if (acc == 0) acc_phase ^= 1;
-        continue;
-      }
-      // lagged mode: the previous unit's stores may still be reading its staging (not if both use alternate buffers)
-      if (p.lagged && !(alt && prev_alt)) {
-        if (lane == 0) bulk_wait_read<0>();
-        __syncwarp();
-      }
-      prev_alt = alt;
       if (t.type == MEGA_G) {
         mega_epilogue_task<GateTcEpi<SAVE>, MEGA_BN / 2>(gate_epi, tile, &s.tmem_full[acc], acc_phase, te, q, cg, lane, ubuf,
                                                          ibar, it, &p.g_c16[t.layer], &p.b_c16[t.layer], nullptr,
                                                          nullptr, nullptr, b, r0, t.nt * (MEGA_BN / 2),
-                                                         MegaSig{mega_gflag(p, t.layer, t.rt), dcnt}, prev, p.dbg, tt);
-      } else if (t.type == MEGA_R && p.res_direct && p.res_lo) {
-        if (lane == 0 && !(p.dbg & 1)) mega_wait_flag(mega_gflag(p, t.layer, t.rt), gtarget);  // implies R(layer-1, rt) is complete
-        __syncwarp();
-        const int trow = r0 + lane;                      // row within the batch item
-        const bool ok = trow < p.T;
-        const size_t off = ((size_t)b * p.T + trow) * MEGA_BN + cg * (MEGA_BN / 4);
-        mega_inplace_direct<SplitTcEpi<true>>(split_epi, tile + ((uint32_t)(q * 32) << 16) + cg * (MEGA_BN / 4), &s.tmem_full[acc],
-                                              acc_phase, te, lane, cg * (MEGA_BN / 4), ok ? p.hi_ptr[t.layer] + off : nullptr,
-                                              ok ? p.lo_ptr[t.layer] + off : nullptr,
-                                              ok ? p.hi_out_ptr[t.layer + 1] + off : nullptr,
-                                              ok ? p.lo_ptr[t.layer + 1] + off : nullptr,
-                                              MegaSig{mega_rflag(p, t.layer, t.rt), dcnt}, tt + 4);
+                                                         MegaSig{mega_gflag(p, t.layer, t.rt), dcnt}, tt);
       } else if (t.type == MEGA_R && p.fold0 && t.layer == 0) {
         // h_1 = W_res g_0 + W_start x_a, all of it from the tensor core: nothing to load, one 16-bit stream to store
         mega_epilogue_task<RoundTcEpi, MEGA_BN>(round_epi, tile, &s.tmem_full[acc], acc_phase, te, q, cg, lane, wbuf, ibar, it,
                                                 &p.hi_c16[1], nullptr, nullptr, nullptr, nullptr, b, r0, 0,
-                                                MegaSig{mega_rflag(p, 0, t.rt), dcnt}, prev, p.dbg, tt + 4, dead);
+                                                MegaSig{mega_rflag(p, 0, t.rt), dcnt}, tt + 4, dead);
       } else if (t.type == MEGA_R && !p.res_lo) {
         if (lane == 0) {  // the warp's whole share of the layer input (two chunks), ahead of the accumulator
           mega_wait_flag(mega_gflag(p, t.layer, t.rt), gtarget);  // implies R(layer-1, rt) is complete
@@ -858,7 +714,7 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
                        MegaSig{mega_rflag(p, t.layer, t.rt), dcnt}, tt + 4, dead);
       } else if (t.type == MEGA_R) {
         if (lane == 0) {  // chunk 0 of the layer input's (hi, lo) pair, ahead of the accumulator
-          if (!(p.dbg & 1)) mega_wait_flag(mega_gflag(p, t.layer, t.rt), gtarget);  // implies R(layer-1, rt) is complete
+          mega_wait_flag(mega_gflag(p, t.layer, t.rt), gtarget);  // implies R(layer-1, rt) is complete
           fence_proxy_async_all();
           mbar_arrive_expect_tx(ibar, 2 * TC_CHUNK16_BYTES);
           const int c0 = cg * (MEGA_BN / 4);
@@ -869,25 +725,20 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_fwd_mega_kernel(const __gr
         mega_epilogue_task<SplitTcEpi<true>, MEGA_BN>(split_epi, tile, &s.tmem_full[acc], acc_phase, te, q, cg, lane, ubuf, ibar,
                                                       it, &p.hi_c16[t.layer + 1], &p.lo_c16[t.layer + 1], nullptr,
                                                       &p.hi_c16[t.layer], &p.lo_c16[t.layer], b, r0, 0,
-                                                      MegaSig{mega_rflag(p, t.layer, t.rt), dcnt}, prev, p.dbg, tt + 4, dead);
+                                                      MegaSig{mega_rflag(p, t.layer, t.rt), dcnt}, tt + 4, dead);
       } else if (p.lst != nullptr) {
-        if (p.lagged) {   // staging is about to be used as plain memory: no store may still be reading it
-          if (lane == 0) bulk_wait_read<0>();
-          __syncwarp();
-        }
         if (p.cout <= 8) mega_end_task<8>(p, tile, &s.tmem_full[acc], acc_phase, te, q, cg, lane, s.epi, WB, b, r0);
         else mega_end_task<MEGA_END_MAXC>(p, tile, &s.tmem_full[acc], acc_phase, te, q, cg, lane, s.epi, WB, b, r0);
       } else {
         mega_epilogue_task<StoreTcEpi, MEGA_BN>(store_epi, tile, &s.tmem_full[acc], acc_phase, te, q, cg, lane, ubuf, ibar, it,
                                                 &p.skip_c32, nullptr, nullptr, nullptr, nullptr, b, r0, 0,
-                                                MegaSig{nullptr, dcnt}, prev, p.dbg, tt + 8);
+                                                MegaSig{nullptr, dcnt}, tt + 8);
       }
       acc ^= 1;
       if (acc == 0) acc_phase ^= 1;
     }
-    if (lane == 0) {  // flush: the last unit's stores, and its signal in lagged mode
+    if (lane == 0) {  // flush: the last unit's stores
       bulk_wait_all();
-      if (p.lagged) mega_signal(pending);
       if (p.clk) {
         long long* o = p.clk + ((size_t)blockIdx.x * 18 + warp) * 16;
         for (int i = 0; i < 12; ++i) o[i] = tt[i];
@@ -925,14 +776,6 @@ struct alignas(64) MegaBwdParams {
   int f16;
   uint32_t idesc, desc_lbo, desc_sbo;
   int lag, total_tasks;
-  int dual;                       // see MegaParams::dual
-  // direct global loads / stores in the epilogues (see MegaParams::res_direct)
-  const uint16_t* sa_ptr[MEGA_D];   // gate output g  [rows][Cd]
-  const uint16_t* sb_ptr[MEGA_D];   // saved sigmoid  [rows][Cd]
-  uint16_t* dpre_ptr[MEGA_D];       // dpre_i         [rows][2Cd]
-  uint16_t* dhi_ptr[MEGA_D];        // dh_i hi halves [rows][Cr]
-  uint16_t* dlo_ptr[MEGA_D];        // dh_i lo halves [rows][Cr]
-  int direct;
   int res_lo;                       // see MegaParams::res_lo (here: the residual GRADIENT stream)
   // `end` conv folded into the dgate GEMM (PackedLayout::Q1f): instead of the kb_s k-blocks of dskip = W_end^T d(log_s, t), a
   // dgate tile reads ONE k-block of the slab dl = S * d(log_s, t) (2 in_channels real columns) against (W_end W_skip)^T
@@ -1000,7 +843,6 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_bwd_mega_kernel(const __gr
   pdl_wait();
   const uint32_t target = 2u * TC_EPI_WARPS;
   const int rounds = (p.total_tasks + npairs - 1) / npairs;
-  const int Crp = p.kb_r * TC_BK, Cd2p = p.kb_d2 * TC_BK;
 
   if (warp == 0) {
     if (lane == 0) {
@@ -1008,14 +850,12 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_bwd_mega_kernel(const __gr
       int stage = 0;
       uint32_t phase = 0;
       const uint32_t full0 = mapa_shared(smem_u32(&s.full[0]), 0);
-      const bool both = p.dual == 0;
-      auto load = [&](const CUtensorMap* am, int ak, int at, int ab, const CUtensorMap* bm, int bk, int bn) {
+      // activation (A) tiles; warp MEGA_BWARP fills the weight half of the same stage
+      auto load = [&](const CUtensorMap* am, int ak, int at, int ab) {
         mbar_wait(&s.empty[stage], phase ^ 1);
         const uint32_t sa = smem_u32(s.stages + stage * MEGA_STAGE_BYTES);
         if (rank == 0) mbar_arrive_expect_tx(&s.full[stage], 2 * MEGA_STAGE_BYTES);
-        const uint32_t bar = full0 + 8 * stage;
-        tma_load_4d(sa, am, bar, ak, at, 0, ab);
-        if (both) tma_load_2d(sa + TC_A_BYTES, bm, bar, bk, bn);
+        tma_load_4d(sa, am, full0 + 8 * stage, ak, at, 0, ab);
         if (++stage == STAGES) { stage = 0; phase ^= 1; }
       };
       for (int k = 0; k < rounds; ++k) {
@@ -1025,40 +865,25 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_bwd_mega_kernel(const __gr
         if (t.type == MEGA_NONE) continue;
         const int b = t.rt / p.tiles_per_batch, tb = t.rt - b * p.tiles_per_batch;
         const int t0 = tb * (2 * TC_BM) + rank * TC_BM;
-        const int nrow = rank * (MEGA_BN / 2);
-        const bool last = t.layer == p.depth - 1;
-        if (p.dual) {
-          mega_wait_cleared(cleared, ++ntask);
-        } else if (t.type == MEGA_DG) {
-          if (!last) {
-            mega_wait_flag(mega_bwd_xflag(p, t.layer + 1, t.rt), target);
-            fence_proxy_async_all();
-          }
-        } else {
-          const uint32_t* f1 = mega_bwd_gflag(p, t.layer, t.rt);
-          mega_wait_flags3(tb > 0 ? f1 - 1 : f1, f1, tb + 1 < p.tiles_per_batch ? f1 + 1 : f1, target);
-          fence_proxy_async_all();
-        }
+        mega_wait_cleared(cleared, ++ntask);       // the scout (warp MEGA_SWARP) has done the waiting
         if (t.type == MEGA_DG) {
-          const CUtensorMap* bm = p.fold_end ? &p.q1f[t.layer] : &p.q1[t.layer];
-          if (!last)
-            for (int kb = 0; kb < p.kb_r; ++kb) load(&p.dh_op[t.layer + 1], kb * TC_BK, t0, b, bm, kb * TC_BK, nrow);
+          if (t.layer != p.depth - 1)
+            for (int kb = 0; kb < p.kb_r; ++kb) load(&p.dh_op[t.layer + 1], kb * TC_BK, t0, b);
           if (p.fold_end) {
-            load(&p.dl_op, 0, t0, b, bm, last ? 0 : Crp, nrow);
+            load(&p.dl_op, 0, t0, b);
           } else {
-            for (int kb = 0; kb < p.kb_s; ++kb) load(&p.dskip_op, kb * TC_BK, t0, b, bm, (last ? 0 : Crp) + kb * TC_BK, nrow);
+            for (int kb = 0; kb < p.kb_s; ++kb) load(&p.dskip_op, kb * TC_BK, t0, b);
           }
         } else {
           for (int sg = 0; sg < p.taps; ++sg) {
             const int shift = -(sg - (p.taps - 1) / 2) * (1 << t.layer);
-            for (int kb = 0; kb < p.kb_d2; ++kb)
-              load(&p.dpre_op[t.layer], kb * TC_BK, t0 + shift, b, &p.q2[t.layer], sg * Cd2p + kb * TC_BK, nrow);
+            for (int kb = 0; kb < p.kb_d2; ++kb) load(&p.dpre_op[t.layer], kb * TC_BK, t0 + shift, b);
           }
         }
       }
     }
   } else if (warp == MEGA_SWARP) {
-    if (lane == 0 && p.dual) {
+    if (lane == 0) {
       uint32_t n = 0;
       for (int k = 0; k < rounds; ++k) {
         const int task = mega_bwd_entry(p.total_tasks, k, pair, npairs);
@@ -1076,7 +901,7 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_bwd_mega_kernel(const __gr
       }
     }
   } else if (warp == MEGA_BWARP) {
-    if (lane == 0 && p.dual) {
+    if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
       const uint32_t full0 = mapa_shared(smem_u32(&s.full[0]), 0);
@@ -1164,36 +989,6 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_bwd_mega_kernel(const __gr
       const uint32_t dcnt = smem_u32(done_cnt + (seq++ & 3));
       const bool last = t.layer == p.depth - 1;
       const int c0 = cg * (MEGA_BN / 4);
-      if (p.direct && p.res_lo) {
-        const int trow = r0 + lane;
-        const bool ok = trow < p.T;
-        const size_t row = (size_t)b * p.T + trow;
-        const uint32_t ta = tile + ((uint32_t)(q * 32) << 16) + c0;
-        if (t.type == MEGA_DG) {
-          const size_t oi = row * MEGA_BN + c0, oo = row * (2 * MEGA_BN) + c0;
-          mega_inplace_direct<GateBwdTcEpi>(gbwd_epi, ta, &s.tmem_full[acc], acc_phase, te, lane, c0,
-                                            ok ? p.sa_ptr[t.layer] + oi : nullptr, ok ? p.sb_ptr[t.layer] + oi : nullptr,
-                                            ok ? p.dpre_ptr[t.layer] + oo : nullptr,
-                                            ok ? p.dpre_ptr[t.layer] + oo + MEGA_BN : nullptr,
-                                            MegaSig{mega_bwd_gflag(p, t.layer, t.rt), dcnt}, tt);
-        } else if (!last) {
-          if (lane == 0) mega_wait_flag(mega_bwd_xflag(p, t.layer + 1, t.rt), target);   // the upstream (hi, lo) pair is complete
-          __syncwarp();
-          const size_t o = row * MEGA_BN + c0;
-          mega_inplace_direct<SplitTcEpi<true>>(add_epi, ta, &s.tmem_full[acc], acc_phase, te, lane, c0,
-                                                ok ? p.dhi_ptr[t.layer + 1] + o : nullptr, ok ? p.dlo_ptr[t.layer + 1] + o : nullptr,
-                                                ok ? p.dhi_ptr[t.layer] + o : nullptr, ok ? p.dlo_ptr[t.layer] + o : nullptr,
-                                                MegaSig{mega_bwd_xflag(p, t.layer, t.rt), dcnt}, tt);
-        } else {
-          const size_t o = row * MEGA_BN + c0;
-          mega_inplace_direct<SplitTcEpi<false>>(first_epi, ta, &s.tmem_full[acc], acc_phase, te, lane, c0, nullptr, nullptr,
-                                                 ok ? p.dhi_ptr[t.layer] + o : nullptr, ok ? p.dlo_ptr[t.layer] + o : nullptr,
-                                                 MegaSig{mega_bwd_xflag(p, t.layer, t.rt), dcnt}, tt);
-        }
-        acc ^= 1;
-        if (acc == 0) acc_phase ^= 1;
-        continue;
-      }
       if (t.type == MEGA_DG) {
         if (lane == 0) {  // chunk 0 of the gate output / saved sigmoid (written by the forward: always ready)
           fence_proxy_async_all();
@@ -1205,7 +1000,7 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_bwd_mega_kernel(const __gr
         mega_epilogue_task<GateBwdTcEpi, MEGA_BN>(gbwd_epi, tile, &s.tmem_full[acc], acc_phase, te, q, cg, lane, wbuf, ibar, it,
                                                   &p.dpt_c16[t.layer], &p.dps_c16[t.layer], nullptr, &p.sa_c16[t.layer],
                                                   &p.sb_c16[t.layer], b, r0, 0,
-                                                  MegaSig{mega_bwd_gflag(p, t.layer, t.rt), dcnt}, nullptr, 0, tt);
+                                                  MegaSig{mega_bwd_gflag(p, t.layer, t.rt), dcnt}, tt);
       } else if (!last && !p.res_lo) {
         if (lane == 0) {  // the warp's whole share of the upstream residual gradient (two chunks of one stream)
           mega_wait_flag(mega_bwd_xflag(p, t.layer + 1, t.rt), target);
@@ -1220,7 +1015,7 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_bwd_mega_kernel(const __gr
       } else if (!p.res_lo) {
         mega_epilogue_task<RoundTcEpi, MEGA_BN>(round_epi, tile, &s.tmem_full[acc], acc_phase, te, q, cg, lane, wbuf, ibar, it,
                                                 &p.dhi_c16[t.layer], nullptr, nullptr, nullptr, nullptr, b, r0, 0,
-                                                MegaSig{mega_bwd_xflag(p, t.layer, t.rt), dcnt}, nullptr, 0, tt);
+                                                MegaSig{mega_bwd_xflag(p, t.layer, t.rt), dcnt}, tt);
       } else if (!last) {
         if (lane == 0) {  // chunk 0 of the upstream residual gradient's (hi, lo) pair
           mega_wait_flag(mega_bwd_xflag(p, t.layer + 1, t.rt), target);
@@ -1233,12 +1028,11 @@ __global__ void __launch_bounds__(MEGA_THREADS, 1) wn_bwd_mega_kernel(const __gr
         mega_epilogue_task<SplitTcEpi<true>, MEGA_BN>(add_epi, tile, &s.tmem_full[acc], acc_phase, te, q, cg, lane, wbuf, ibar, it,
                                                       &p.dhi_c16[t.layer], &p.dlo_c16[t.layer], nullptr,
                                                       &p.dhi_c16[t.layer + 1], &p.dlo_c16[t.layer + 1], b, r0, 0,
-                                                      MegaSig{mega_bwd_xflag(p, t.layer, t.rt), dcnt}, nullptr, 0, tt);
+                                                      MegaSig{mega_bwd_xflag(p, t.layer, t.rt), dcnt}, tt);
       } else {
         mega_epilogue_task<SplitTcEpi<false>, MEGA_BN>(first_epi, tile, &s.tmem_full[acc], acc_phase, te, q, cg, lane, wbuf, ibar,
                                                        it, &p.dhi_c16[t.layer], &p.dlo_c16[t.layer], nullptr, nullptr, nullptr,
-                                                       b, r0, 0, MegaSig{mega_bwd_xflag(p, t.layer, t.rt), dcnt}, nullptr, 0,
-                                                       tt);
+                                                       b, r0, 0, MegaSig{mega_bwd_xflag(p, t.layer, t.rt), dcnt}, tt);
       }
       acc ^= 1;
       if (acc == 0) acc_phase ^= 1;

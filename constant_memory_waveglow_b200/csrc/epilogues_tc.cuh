@@ -28,7 +28,6 @@ struct GateTcEpi {
   static constexpr int kOut = SAVE ? 2 : 1, kIn = 0, kOutBufs = 1, kColGroups = 4;
   const float* bias;  // nullptr or [2][Cd]
   int Cd, f16;
-  int mix;            // fp16 path: odd columns take e^(-y) from the FMA pipe (exp2_fma), even columns from MUFU.EX2
   __device__ __forceinline__ int out_col(int, int c0) const { return c0; }
   __device__ __forceinline__ int in_col(int, int c0) const { return c0; }
   __device__ __forceinline__ void compute(int ch0, float (&lo)[16], float (&hi)[16], uint32_t (&o)[kOut][8]) const {
@@ -40,24 +39,13 @@ struct GateTcEpi {
       // fp16's 11-bit mantissa deserves better than tanh.approx (2^-11 relative error): exact-to-1e-7 forms on
       // MUFU.EX2 / MUFU.RCP, three MUFU operations per gate value (the MUFU pipe runs 16 lanes per clock per SM, a
       // quarter of an epilogue's budget at four) -- see gate_ex2()
-      if (mix) {
 #pragma unroll
-        for (int j = 0; j < 16; j += 2) {
-          float a0, b0, g0, a1, b1, g1;
-          gate_ex2<SAVE, false>(lo[j], hi[j], a0, b0, g0);
-          gate_ex2<SAVE, true>(lo[j + 1], hi[j + 1], a1, b1, g1);
-          o[0][j >> 1] = pack2(g0, g1, 1);
-          if constexpr (SAVE) o[1][j >> 1] = pack2(b0, b1, 1);
-        }
-      } else {
-#pragma unroll
-        for (int j = 0; j < 16; j += 2) {
-          float a0, b0, g0, a1, b1, g1;
-          gate_ex2<SAVE>(lo[j], hi[j], a0, b0, g0);
-          gate_ex2<SAVE>(lo[j + 1], hi[j + 1], a1, b1, g1);
-          o[0][j >> 1] = pack2(g0, g1, 1);
-          if constexpr (SAVE) o[1][j >> 1] = pack2(b0, b1, 1);
-        }
+      for (int j = 0; j < 16; j += 2) {
+        float a0, b0, g0, a1, b1, g1;
+        gate_ex2<SAVE>(lo[j], hi[j], a0, b0, g0);
+        gate_ex2<SAVE>(lo[j + 1], hi[j + 1], a1, b1, g1);
+        o[0][j >> 1] = pack2(g0, g1, 1);
+        if constexpr (SAVE) o[1][j >> 1] = pack2(b0, b1, 1);
       }
     } else {
 #pragma unroll

@@ -211,27 +211,8 @@ static bool mega_enabled() {  // read at every call: tests flip CMWG_MEGA inside
 
 // residual (forward) / dgate (backward) tiles trail their gate / dx tiles by `lag` row-tile slots; lag <= RT - 2 keeps the
 // list in dependency order (tests/test_host.py::test_task_lists_are_in_dependency_order)
-static inline int mega_fwd_lag(int RT) {
-  static const int lag_env = [] { const char* v = getenv("CMWG_MEGA_LAG"); return v ? atoi(v) : 64; }();
-  return std::max(0, std::min(lag_env, RT - 2));
-}
-static inline int mega_bwd_lag(int RT) {
-  static const int lag_env = [] { const char* v = getenv("CMWG_MEGA_LAG_BWD"); return v ? atoi(v) : 96; }();
-  return std::max(0, std::min(lag_env, RT - 2));
-}
-
-static inline int mega_dual() {  // CMWG_MEGA_DUAL=0: one TMA producer thread for both operands (the round-1 arrangement)
-  static const int v = [] { const char* e = getenv("CMWG_MEGA_DUAL"); return (e && e[0] == '0') ? 0 : 1; }();
-  return v;
-}
-
-// CMWG_GATE_MIX=1: every second gate value takes its sigmoid exponential from the FMA pipe (exp2_fma) instead of MUFU.EX2.
-// Measured: the gate epilogue gets 11 % shorter (3559 -> 3177 cycles per tile) and the kernel does not get faster (0.504 ms
-// either way: the residual tiles' epilogue and the operand feed bound it), so it stays off.
-static inline int gate_mix() {
-  static const int v = [] { const char* e = getenv("CMWG_GATE_MIX"); return (e && e[0] == '1') ? 1 : 0; }();
-  return v;
-}
+static inline int mega_fwd_lag(int RT) { return std::max(0, std::min(64, RT - 2)); }
+static inline int mega_bwd_lag(int RT) { return std::max(0, std::min(96, RT - 2)); }
 
 // Residual stream of the tcgen05 engine (forward) and its gradient (backward): (hi, lo) pair of 16-bit slabs, or the operand
 // slab alone (AddTcEpi: fp16 operands only -- bf16's 8 mantissa bits need the pair).  CMWG_RES_LO=1 keeps the pair with fp16
@@ -265,16 +246,14 @@ static inline bool mega_shapes_ok(const WnDims& d, int B, int T);
 // The backward will run the single-kernel chain / batch all weight-gradient GEMMs / fold the `end` conv completely
 // (wn_backward_impl); the saving forward asks the last one to know whether anything will read the fp32 skip sum.
 static inline bool bwd_fused_chain(const WnDims& d, int B, int T) {
-  const char* e = getenv("CMWG_MEGA_BWD");
-  return d.tc && mega_enabled() && mega_shapes_ok(d, B, T) && d.Cd == 256 && !(e && e[0] == '0');
+  return d.tc && mega_enabled() && mega_shapes_ok(d, B, T) && d.Cd == 256;
 }
 static inline bool bwd_wgrad_batched(const WnDims& d, int B, int T) {
   const char* e = getenv("CMWG_WGRAD_BATCH");
   return bwd_fused_chain(d, B, T) && d.depth * (d.R + 3) <= TC_MAX_WG && !(e && e[0] == '0');
 }
 static inline bool bwd_foldend_full(const WnDims& d, int B, int T) {
-  const char* e = getenv("CMWG_FOLD_END_W");
-  return bwd_wgrad_batched(d, B, T) && foldend_enabled(d) && !(e && e[0] == '0');
+  return bwd_wgrad_batched(d, B, T) && foldend_enabled(d);
 }
 
 static inline bool mega_shapes_ok(const WnDims& d, int B, int T) {
@@ -381,15 +360,12 @@ static int wn_forward_mega(const WnDims& d, const PackedLayout& PL, const FwdLay
   p.ngt = d.npadA / MEGA_BN;
   p.taps = d.R; p.kb_h = d.Crp / TC_BK; p.kb_c = d.auxp / TC_BK; p.kb_g = d.Cdp / TC_BK;
   p.Cd = d.Cd; p.f16 = f16;
-  {
-    const char* e = getenv("CMWG_MEGA_KTRIM");   // CMWG_MEGA_KTRIM=0: issue the padded K steps too (A/B timing)
-    const int real_last = d.aux - (p.kb_c - 1) * TC_BK;
-    p.kc_last = (e && e[0] == '0') ? TC_BK / 16 : std::max(1, std::min(TC_BK / 16, ceil_div(real_last, 16)));
-  }
+  const int real_last = d.aux - (p.kb_c - 1) * TC_BK;
+  p.kc_last = std::max(1, std::min(TC_BK / 16, ceil_div(real_last, 16)));
   if (fold0) {
     p.fold0 = 1;
     const int real_last0 = d.aux + d.R * d.cin - (p.kb_c - 1) * TC_BK;
-    p.kc_last0 = p.kc_last == TC_BK / 16 ? p.kc_last : std::max(1, std::min(TC_BK / 16, ceil_div(real_last0, 16)));
+    p.kc_last0 = std::max(1, std::min(TC_BK / 16, ceil_div(real_last0, 16)));
     CMWG_PROPAGATE(get_matrix_map(&p.pa0f, pk + PL.PA0f, d.auxp, d.npadA, MEGA_BN / 2, f16));
     CMWG_PROPAGATE(get_matrix_map(&p.pb0f, pk + PL.PB0f, d.Cdp + d.kb, d.Cr, MEGA_BN / 2, f16));
   }
@@ -397,19 +373,6 @@ static int wn_forward_mega(const WnDims& d, const PackedLayout& PL, const FwdLay
   p.desc_lbo = 1u; p.desc_sbo = 1024u >> 4;
   // R(u) must come after G(u) and before G(u + RT - 1) (its right-hand neighbour one layer up): lag <= RT - 2
   p.lag = mega_fwd_lag(p.RT);
-  p.dual = mega_dual();
-  p.gate_mix = gate_mix();
-  {
-    // measured SLOWER than the TMA chunks (whole WN forward 0.540 vs 0.503 ms, saving 0.598 vs 0.560: row-per-thread 32-byte
-    // accesses and a device-scope fence per lane cost more than the queueing they avoid): opt-in, kept for the comparison
-    const char* e = getenv("CMWG_MEGA_RDIRECT");
-    p.res_direct = (e && e[0] == '1') ? 1 : 0;
-    for (int i = 0; i < d.depth; ++i) {
-      p.hi_ptr[i] = reinterpret_cast<const uint16_t*>(hin[i]);
-      p.hi_out_ptr[i] = reinterpret_cast<uint16_t*>(hin[i]);
-      p.lo_ptr[i] = reinterpret_cast<uint16_t*>(hlo[i]);
-    }
-  }
   if (mega_end_fused(d)) {
     p.lst = lst;
     p.w_end = reinterpret_cast<const float*>(pk + PL.wEnd);
@@ -418,18 +381,6 @@ static int wn_forward_mega(const WnDims& d, const PackedLayout& PL, const FwdLay
     p.store_skip = (save && !bwd_foldend_full(d, B, T)) ? 1 : 0;
   }
   p.total_tasks = (d.depth * p.RT + p.lag) * (p.ngt + 1) + p.RT;
-  // timing experiments that SKIP synchronisation or epilogue work (wrong results by design) exist only in builds made
-  // with -DCMWG_MEGA_EXPERIMENTS; the shipped library ignores CMWG_MEGA_DBG
-#ifdef CMWG_MEGA_EXPERIMENTS
-  static const int dbg_env = [] { const char* v = getenv("CMWG_MEGA_DBG"); return v ? atoi(v) : 0; }();
-  p.dbg = dbg_env;
-#else
-  p.dbg = 0;
-#endif
-  // "lagged" completion signals (a unit's stores complete behind the next unit's work, its dependency counter is released one
-  // unit later) were measured slower in round 1 (0.51 vs 0.476 ms at the LJ shape: consumers wait longer than the epilogue
-  // warps save) and are not maintained with the scout / fused-epilogue arrangement: always immediate.
-  p.lagged = 0;
   {
     // CMWG_MEGA_CLK=1: per-role cycle accumulators of the LAST launch, read back with cmwg_mega_clk_read (tools only)
     const char* v = getenv("CMWG_MEGA_CLK");
@@ -484,18 +435,6 @@ static int wn_backward_mega(const WnDims& d, const PackedLayout& PL, const BwdLa
   p.idesc = make_idesc(f16, 2 * TC_BM, MEGA_BN, 0, 0);
   p.desc_lbo = 1u; p.desc_sbo = 1024u >> 4;
   p.lag = mega_bwd_lag(p.RT);
-  p.dual = mega_dual();
-  {
-    const char* e = getenv("CMWG_MEGA_RDIRECT");   // see wn_forward_mega: opt-in, measured slower
-    p.direct = (e && e[0] == '1') ? 1 : 0;
-    for (int i = 0; i < d.depth; ++i) {
-      p.sa_ptr[i] = reinterpret_cast<const uint16_t*>(sa[i]);
-      p.sb_ptr[i] = reinterpret_cast<const uint16_t*>(sb[i]);
-      p.dpre_ptr[i] = reinterpret_cast<uint16_t*>(dpre[i]);
-      p.dhi_ptr[i] = reinterpret_cast<uint16_t*>(dh_hi[i]);
-      p.dlo_ptr[i] = reinterpret_cast<uint16_t*>(dh_lo[i]);
-    }
-  }
   p.total_tasks = p.RT + 2 * (d.depth * p.RT + p.lag);
   p.flags = reinterpret_cast<uint32_t*>(ws + BL.flags);
   CMWG_CHECK_CUDA(cudaMemsetAsync(p.flags, 0, (size_t)d.depth * 2 * p.RT * 4, st));
@@ -614,10 +553,10 @@ static int wn_forward_impl(const WnDims& d, const void* packed, const float* x, 
         io.out[0] = op_stream(g_op(i), d.Cd);
         if (save) {
           io.out[1] = op_stream(sv + FL.s_b[i], d.Cd);   // the backward recovers tanh as g / sigmoid (GateBwdTcEpi)
-          GateTcEpi<true> epi{biasA, d.Cd, f16, gate_mix()};
+          GateTcEpi<true> epi{biasA, d.Cd, f16};
           CMWG_PROPAGATE(tc_gemm_launch(g, io, epi, st));
         } else {
-          GateTcEpi<false> epi{biasA, d.Cd, f16, gate_mix()};
+          GateTcEpi<false> epi{biasA, d.Cd, f16};
           CMWG_PROPAGATE(tc_gemm_launch(g, io, epi, st));
         }
       } else {
@@ -850,8 +789,7 @@ static int wn_backward_impl(const WnDims& d, const cmwg_wn_params* prm, const vo
   const bool wg_batched = TC && bwd_wgrad_batched(d, B, T);
   // `end` conv folded into the backward: fe_dg -- the dgate tiles of the chain read S * dlst (one k-block) against
   // (W_end W_skip)^T instead of the 256-channel dskip slab; fe_full -- the weight gradients that dskip feeds (skip rows of every
-  // W_o, the `end` weight) go through the fold as well (foldend_dw_kernel), so dskip is never formed.  CMWG_FOLD_END_W=0
-  // keeps the slab for the weight gradients.
+  // W_o, the `end` weight) go through the fold as well (foldend_dw_kernel), so dskip is never formed.
   const bool fe_dg = fusedb && foldend_enabled(d);
   const bool fe_full = TC && bwd_foldend_full(d, B, T);
   uint16_t* dl16 = nullptr;
@@ -937,7 +875,6 @@ static int wn_backward_impl(const WnDims& d, const cmwg_wn_params* prm, const vo
   GatherSpec gather[TC_MAX_WG];
   int np = 0, nr = 0, ngather = 0;
   bool pending_gather = false;
-  const bool deferred_gather = wg_batched && !(getenv("CMWG_WGRAD_GATHER") && getenv("CMWG_WGRAD_GATHER")[0] == '0');
   auto flush_wgrad = [&](int group) -> int {
     for (int g0 = 0; g0 < np; g0 += group) {
       const int gn = std::min(group, np - g0);
@@ -963,7 +900,7 @@ static int wn_backward_impl(const WnDims& d, const cmwg_wn_params* prm, const vo
       for (int k = 0; k < nr; ++k) {
         if (rs[k].pi < g0 || rs[k].pi >= g0 + gn) continue;
         const WgradProblem& q = pr[rs[k].pi];
-        if (deferred_gather && splits[rs[k].pi - g0] == 1 && !rs[k].no_gather) {
+        if (wg_batched && splits[rs[k].pi - g0] == 1 && !rs[k].no_gather) {
           pending_gather = true;
           gather[ngather++] = GatherSpec{rs[k].out, q.partial, q.M, q.N, rs[k].n_valid, rs[k].sm, rs[k].sn, rs[k].off};
           rs[k].pi = -1;   // taken
@@ -1412,13 +1349,6 @@ int cmwg_wn_forward_varlen(const cmwg_wn_config* cfg, const void* packed, const 
   if (d.H != 1) {
     set_error("cmwg_wn_forward_varlen: per-item lengths are implemented for the 1-D WN only");
     return CMWG_ERR_UNSUPPORTED;
-  }
-  if (d.tc && fwd_res_lo(d)) {
-    const char* e = getenv("CMWG_MEGA_RDIRECT");
-    if (e && e[0] == '1' && mega_enabled() && mega_shapes_ok(d, B, T)) {
-      set_error("cmwg_wn_forward_varlen: CMWG_MEGA_RDIRECT=1 residual tiles do not mask rows past an item's end");
-      return CMWG_ERR_UNSUPPORTED;
-    }
   }
   VarLen vl;
   vl.host = lengths_host; vl.dev = lengths_dev;

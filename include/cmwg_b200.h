@@ -209,7 +209,7 @@ size_t cmwg_wn_saved_bytes(const cmwg_wn_config* cfg, int B, int T);
  * that hold no valid step).  lengths_host plans the work on the host; lengths_dev is a device int[B] holding the SAME values,
  * uploaded by the caller (the library never allocates or copies it).  workspace: cmwg_wn_varlen_workspace_bytes(cfg, B, T).
  * No `saved` (training on per-item lengths is not supported).  Returns CMWG_ERR_ARG for a length outside [1, T] and
- * CMWG_ERR_UNSUPPORTED for the 2-D WN (height > 1) and for CMWG_MEGA_RDIRECT=1 residual tiles. */
+ * CMWG_ERR_UNSUPPORTED for the 2-D WN (height > 1). */
 size_t cmwg_wn_varlen_workspace_bytes(const cmwg_wn_config* cfg, int B, int T);
 int cmwg_wn_forward_varlen(const cmwg_wn_config* cfg, const void* packed, const float* x, long long x_bstride,
                            const void* ycl, int B, int T, const int* lengths_host, const int* lengths_dev, void* workspace,

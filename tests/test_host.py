@@ -134,6 +134,20 @@ def test_fused_optimizer_step_invalidates_weight_packs():
     assert W.pack_generation() == g2 + 1
 
 
+def test_every_native_switch_is_documented():
+    """Every CMWG_* environment variable the native library reads (getenv, or engine_tc.cu's dbg_flag) is described in
+    INTEGRATION.md, so a switch cannot be added without saying what it selects."""
+    csrc = os.path.join(ROOT, "constant_memory_waveglow_b200", "csrc")
+    names = set()
+    for f in os.listdir(csrc):
+        if f.endswith((".cu", ".cuh")):
+            names |= set(re.findall(r'\b(?:getenv|dbg_flag)\("(CMWG_[A-Z0-9_]+)"\)', open(os.path.join(csrc, f)).read()))
+    assert "CMWG_MEGA" in names and "CMWG_DEBUG_NOCACHE" in names
+    doc = open(os.path.join(ROOT, "INTEGRATION.md")).read()
+    missing = sorted(n for n in names if not re.search(r"`" + n + r"\b", doc))
+    assert not missing, f"switches read in csrc/ but not documented in INTEGRATION.md: {missing}"
+
+
 def test_no_product_import_of_oracle():
     pkg = os.path.join(ROOT, "constant_memory_waveglow_b200")
     for dirpath, _, files in os.walk(pkg):
