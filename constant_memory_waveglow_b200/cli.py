@@ -10,7 +10,9 @@ batch, with the per-item lengths); at 0, the default, it is skipped.  ``vocode``
 .npy, as NVIDIA's ``inference.py`` reads them) with an NVIDIA WaveGlow checkpoint or this package's, batched the same way;
 given ``.wav`` files it computes their mels first (Tacotron2's ``TacotronSTFT`` for NVIDIA checkpoints, the checkpoint's
 conditioner otherwise): copy synthesis.  ``score`` prints the per-file negative log-likelihood of WAV files under a
-checkpoint, in the convention of the training loss (``WaveGlowLoss``).
+checkpoint, in the convention of the training loss (``WaveGlowLoss``).  WAV inputs must be at the front end's rate unless
+``--resample`` is given (``vocode``, ``score``): files at other rates are then resampled on the GPU (``Resample``, in
+length-sorted batches per source rate).  ``vocode --output-rate HZ`` resamples the synthesised audio to HZ.
 """
 from __future__ import annotations
 
@@ -243,13 +245,35 @@ def _frontend_rate(frontend) -> int:
     return int(getattr(frontend, "sampling_rate", None) or frontend.sample_rate)
 
 
-def _read_wav_mono(path: str, rate: int, p: argparse.ArgumentParser) -> torch.Tensor:
-    """A WAV file as one channel (the mean of its channels); its sampling rate must be `rate` (there is no resampler)."""
+def _read_wav_mono(path: str, rate: int, p: argparse.ArgumentParser, resample: bool = False):
+    """A WAV file as one channel (the mean of its channels), and its sampling rate.  Unless `resample`, the rate must be
+    `rate`."""
     from .datasets import wav_info
     sr = wav_info(path).sample_rate
-    if sr != rate:
-        p.error(f"{path}: sampled at {sr} Hz; the model's mel front end expects {rate} Hz (resample it first)")
-    return wav_read(path).mean(0)
+    if sr != rate and not resample:
+        p.error(f"{path}: sampled at {sr} Hz; the model's mel front end expects {rate} Hz (resample it first, or pass "
+                "--resample)")
+    return wav_read(path).mean(0), sr
+
+
+def _resample_batches(signals, rates, rate: int, max_batch: int, dev) -> list:
+    """Each 1-D signal (on the CPU) at `rate`: signals already there are kept, the others are grouped by source rate and
+    resampled in length-sorted batches of `max_batch`, one Resample call with the per-item lengths each.  Item i gets
+    ceil(N n_i / O) samples, bit for bit what a call on it alone gives.  Returns CPU tensors in input order."""
+    from .base import pad_batch
+    from .resample import Resample
+    out = list(signals)
+    for sr in sorted(set(rates) - {rate}):
+        rs = Resample(sr, rate).to(dev)
+        order = sorted((i for i, r in enumerate(rates) if r == sr), key=lambda i: signals[i].numel())
+        for s0 in range(0, len(order), max_batch):
+            idx = order[s0:s0 + max_batch]
+            x, lens = pad_batch([signals[i] for i in idx])
+            with torch.no_grad():
+                y = rs(x.to(dev), lengths=lens)
+            for j, (i, n) in enumerate(zip(idx, rs.output_lengths(lens))):
+                out[i] = y[j, :n].cpu()
+    return out
 
 
 def _frontend_mels(frontend, signals, names, max_batch: int, dev, p: argparse.ArgumentParser):
@@ -280,12 +304,19 @@ def vocode(argv) -> None:
                                 "checkpoints")
     p.add_argument("ckpt", type=str)
     p.add_argument("outdir", type=str)
-    p.add_argument("mels", type=str, nargs="+", help=".pt / .npy mel spectrograms or .wav files (at the front end's rate)")
+    p.add_argument("mels", type=str, nargs="+", help=".pt / .npy mel spectrograms or .wav files (at the front end's rate, "
+                   "or any rate with --resample)")
     p.add_argument("-s", "--sigma", type=float, default=0.6)
     p.add_argument("--max-batch", type=int, default=16, help="utterances per synthesis call")
     p.add_argument("--seed", type=int, default=0, help="noise seed; file i draws from a generator seeded by (seed, i)")
     p.add_argument("--sampling-rate", type=int, default=None,
-                   help="of the written WAVs (default: 22050 for NVIDIA checkpoints, else the conditioner's)")
+                   help="the model's output rate, declared: it labels the written WAVs and is the rate --output-rate "
+                   "converts from; no samples change (default: 22050 for NVIDIA checkpoints, else the conditioner's)")
+    p.add_argument("--output-rate", type=int, default=None, metavar="HZ",
+                   help="resample the synthesised audio (after the denoiser) from the model's rate to HZ on the GPU and "
+                   "write it at HZ; an utterance of n samples becomes ceil(n * HZ / model rate) samples")
+    p.add_argument("--resample", action="store_true",
+                   help="accept .wav files at any rate: they are resampled on the GPU to the front end's rate first")
     _add_denoiser_arg(p)
     args = p.parse_args(argv)
     _check_denoiser_arg(p, args)
@@ -293,6 +324,8 @@ def vocode(argv) -> None:
         p.error("--max-batch must be >= 1")
     if args.sampling_rate is not None and args.sampling_rate < 1:
         p.error("--sampling-rate must be >= 1")
+    if args.output_rate is not None and args.output_rate < 1:
+        p.error("--output-rate must be >= 1")
     stems = [os.path.splitext(os.path.basename(f))[0] for f in args.mels]
     if len(set(stems)) != len(stems):
         p.error("mel files must have distinct names: outputs are written as OUTDIR/<name>.wav")
@@ -301,9 +334,13 @@ def vocode(argv) -> None:
     is_wav = [f.lower().endswith(".wav") for f in args.mels]
     mels = [None if w else _read_mel(f, model.n_mels, p) for f, w in zip(args.mels, is_wav)]
     wav_idx = [i for i, w in enumerate(is_wav) if w]
-    signals = [_read_wav_mono(args.mels[i], _frontend_rate(frontend), p) for i in wav_idx]
+    read = [_read_wav_mono(args.mels[i], _frontend_rate(frontend), p, args.resample) for i in wav_idx]
     from .base import pad_batch
+    from .resample import Resample
     dev = torch.device("cuda")
+    # WAVs at other rates (--resample): the model-rate signal replaces the file
+    signals = _resample_batches([x for x, _ in read], [r for _, r in read], _frontend_rate(frontend), args.max_batch, dev)
+    out_rs = Resample(sr, args.output_rate).to(dev) if args.output_rate is not None else None
     model = model.to(dev).eval()
     hop = model._hop_length
     # WAV inputs: mels from the front end, one call per batch with the per-item lengths; the output keeps each file's
@@ -333,10 +370,13 @@ def vocode(argv) -> None:
             cost += dt
             if denoiser is not None:
                 x = denoiser(x, args.denoiser_strength, lengths=[f * hop for f in frames] if lengths else None)
+            ns = [n_out.get(i, frames[j] * hop) for j, i in enumerate(idx)]
+            total += sum(ns)
+            if out_rs is not None:
+                x, ns = out_rs(x, lengths=ns), out_rs.output_lengths(ns)
             for j, i in enumerate(idx):
-                n = n_out.get(i, frames[j] * hop)
-                total += n
-                wav_write(os.path.join(args.outdir, stems[i] + ".wav"), x[j, :n].reshape(1, -1).cpu(), sr)
+                wav_write(os.path.join(args.outdir, stems[i] + ".wav"), x[j, :ns[j]].reshape(1, -1).cpu(),
+                          args.output_rate or sr)
     print("{} files, {} samples, synthesis {:.4f} s, {:.4f} kHz".format(len(mels), total, cost, total / max(cost, 1e-9) / 1e3))
 
 
@@ -347,17 +387,22 @@ def score(argv) -> None:
     p.add_argument("wavs", type=str, nargs="+")
     p.add_argument("-s", "--sigma", type=float, default=1.0, help="of the loss (NVIDIA trains with 1.0)")
     p.add_argument("--max-batch", type=int, default=16, help="files per forward call")
+    p.add_argument("--resample", action="store_true",
+                   help="accept files at any rate: they are resampled on the GPU to the front end's rate, and the "
+                   "printed sample count and the NLL are those of the resampled signal")
     args = p.parse_args(argv)
     if args.max_batch < 1:
         p.error("--max-batch must be >= 1")
     if not 0 < args.sigma < math.inf:
         p.error("--sigma must be a finite number > 0")
-    for path, n, nll in score_files(args.ckpt, args.wavs, args.sigma, args.max_batch, p):
+    for path, n, nll in score_files(args.ckpt, args.wavs, args.sigma, args.max_batch, p, args.resample):
         print(f"{path}\t{n}\t{nll:.6f}")
 
 
-def score_files(ckpt: str, paths, sigma: float, max_batch: int, p: argparse.ArgumentParser):
-    """[(path, samples, NLL)] in input order.  Each file, cut to a multiple of n_group, gets WaveGlowLoss(sigma) of its own
+def score_files(ckpt: str, paths, sigma: float, max_batch: int, p: argparse.ArgumentParser, resample: bool = False):
+    """[(path, samples, NLL)] in input order.  With `resample`, files at other rates are first resampled to the front end's
+    rate (in batches, as _resample_batches does), and samples and NLL are those of that signal.  Each file, cut to a
+    multiple of n_group, gets WaveGlowLoss(sigma) of its own
     forward call: 0.5 sum z^2 / sigma^2 - log-det, over its samples.  Files run in length-sorted batches through
     forward(x, mel, lengths=...), which gives every item its own call's z and log-det bit for bit; families without
     per-item lengths run one file per call."""
@@ -366,11 +411,10 @@ def score_files(ckpt: str, paths, sigma: float, max_batch: int, p: argparse.Argu
     from .nvidia import NvidiaWaveGlow
     model, _, frontend = _load_vocoder_frontend(ckpt, p)
     g, hop = getattr(model, "n_group", 1), model._hop_length
-    signals = []
-    for f in paths:
-        x = _read_wav_mono(f, _frontend_rate(frontend), p)
-        signals.append(x[:x.numel() - x.numel() % g])
+    read = [_read_wav_mono(f, _frontend_rate(frontend), p, resample) for f in paths]
     dev = torch.device("cuda")
+    signals = _resample_batches([x for x, _ in read], [r for _, r in read], _frontend_rate(frontend), max_batch, dev)
+    signals = [x[:x.numel() - x.numel() % g] for x in signals]
     model, frontend = model.to(dev).eval(), frontend.to(dev)
     with torch.no_grad():
         mels = _frontend_mels(frontend, signals, list(paths), max_batch, dev, p)

@@ -338,6 +338,60 @@ def denoise(audio: torch.Tensor, window: torch.Tensor, bias_mag: torch.Tensor, s
     return out[0] if squeeze else out
 
 
+# ---------------------------------------------------------------------------------------------
+# band-limited resampling
+# ---------------------------------------------------------------------------------------------
+def resample_lengths(x: Tensor, lengths) -> Optional[List[int]]:
+    """The argument checks of resample (no device needed): x (T,) or (B, T), each length in [1, T].  Returns the lengths
+    as a list of ints, or None."""
+    from .base import lengths_list
+    if x.dim() not in (1, 2):
+        raise ValueError(f"Resample expects (B, T) or (T,), got {tuple(x.shape)}")
+    if lengths is None:
+        return None
+    B = 1 if x.dim() == 1 else x.shape[0]
+    T = x.shape[-1]
+    lens = lengths_list(lengths, B, "Resample", "samples")
+    for n in lens:
+        if not 1 <= n <= T:
+            raise ValueError(f"Resample: length {n} outside [1, {T}] (lengths are in samples)")
+    return lens
+
+
+def resample(x: Tensor, table: Tensor, first: Tensor, O: int, N: int, w: int, lengths=None) -> Tensor:
+    """cmwg_resample (band-limited resampling, resample.py) of x (B, T) or (T,) on the GPU -> (B, ceil(N T / O)) or (ceil(N T / O),) float32; item b (len_b
+    samples) holds its ceil(N len_b / O) resampled samples, then zeros.  table (L, N) float32 and first (N,) int32 on x's
+    device come from resample_table."""
+    lens = resample_lengths(x, lengths)
+    T = x.shape[-1]
+    if (N * T + O - 1) // O > 2 ** 31 - 1:
+        raise ValueError(f"resample: {T} samples give {(N * T + O - 1) // O} output samples, more than the 2**31 - 1 a "
+                         "call can write")
+    L.require_cuda(x, table, first, op="resample")
+    if table.dtype != torch.float32 or table.dim() != 2 or table.shape[1] != N or first.dtype != torch.int32 \
+            or first.shape != (N,):
+        raise ValueError(f"resample: expected table (L, {N}) float32 and first ({N},) int32, got {tuple(table.shape)} "
+                         f"{table.dtype} and {tuple(first.shape)} {first.dtype}")
+    table, first = table.contiguous(), first.contiguous()
+    squeeze = x.dim() == 1
+    x = x.detach()
+    if squeeze:
+        x = x.unsqueeze(0)
+    if x.dtype != torch.float32 or x.stride(1) != 1:
+        x = x.float().contiguous()
+    B, T = x.shape
+    T_out = (N * T + O - 1) // O
+    y = torch.empty((B, T_out), device=x.device, dtype=torch.float32)
+    lens_host = lens_dev = None
+    if lens is not None:
+        lens_host = (C.c_int * B)(*lens)
+        lens_dev = torch.tensor(lens, dtype=torch.int32).to(x.device)
+    L.check(L.load().cmwg_resample(x.data_ptr(), x.stride(0) if B > 1 else T, B, T, lens_host, L.ptr(lens_dev),
+                                   table.data_ptr(), first.data_ptr(), O, N, table.shape[0], w, y.data_ptr(),
+                                   T_out, T_out, L.stream_ptr(x.device)), "resample")
+    return y[0] if squeeze else y
+
+
 def selftest_tc_gemm(a: torch.Tensor, b: torch.Tensor, M: int, N: int, K: int, variant: int) -> torch.Tensor:
     """16-bit operands through the tcgen05 engine; see cmwg_selftest_tc_gemm."""
     is_fp16 = int(a.dtype == torch.float16)

@@ -321,6 +321,24 @@ int cmwg_denoise(const float* x, long long x_bstride, int B, int T, const int* l
                  void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Band-limited resampling: torchaudio.functional.resample(x, orig, new, lowpass_filter_width, rolloff, resampling_method,
+ * beta) per item, with the kernel of torchaudio/functional/functional.py `_get_sinc_resample_kernel` (windowed sinc at
+ * t = ((i - w) / O - j / N) * base, clamped to [-lpw, lpw]) applied as `_apply_sinc_resample_kernel` does (zero padding by
+ * w on the left, conv1d with stride O, output cut to ceil(N * len / O) samples), O = orig / gcd, N = new / gcd.
+ * Only the taps inside the window's support (|t| < lpw) are evaluated: table (L, N) fp32 holds, in row m and column j, tap
+ * first[j] + m of torchaudio's phase j (0 past the phase's span), first (N ints) the index of its first kept tap; w is
+ * torchaudio's `width`.  The host builds both (resample.py `resample_table`).
+ *   y (B, T_out), T_out = ceil(N * T / O) (64-bit arithmetic), at batch stride y_bstride <- per item b, over its first
+ *   len_b samples (len_b = lengths[b], or T when both length pointers are NULL; 1 <= len_b <= T):
+ *   y[b, kN + j] = sum_m table[m][j] * x[b, kO + first[j] + m - w] for kN + j < ceil(N len_b / O), x read as 0 outside
+ *   [0, len_b); y[b, n] = 0 after that.  Summed in ascending m with fmaf, without atomics: deterministic, and each item is
+ *   bit-identical to a call on that item alone.  x: (B, T) at batch stride x_bstride.  lengths_host (host) and lengths_dev
+ *   (device) hold the same B ints, or are both NULL.  Nothing is allocated.  Bad sizes or lengths: CMWG_ERR_ARG. */
+int cmwg_resample(const float* x, long long x_bstride, int B, int T, const int* lengths_host, const int* lengths_dev,
+                  const float* table, const int* first, int O, int N, int L, int w, float* y, long long y_bstride, int T_out,
+                  void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * WSRGlow conditioning front end (model/wsrglow.py:37-50, `_get_cond`), one kernel:
  *   c (B, Tc) fp32 low-rate signal, CLIPPED TO [-1, 1] IN PLACE like the reference's c.clip_(-1, 1) (:38);
  *   out (B, 8E + 9 + 9P, Tc/8) fp32 NCL = cat(mu-law code embedding rows (emb: n_codes x E, :39), the 9 magnitudes of
