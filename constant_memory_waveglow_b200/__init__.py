@@ -18,6 +18,7 @@ from .melglow import MelGlow, WN_LVC
 from .denoiser import Denoiser
 from .resample import Resample
 from .condition import MelSpec, TacotronSTFT
+from .distance import SpectralDistance
 from .nvidia import NvidiaWaveGlow, load_nvidia_waveglow
 
 __all__ = ["FlowBase", "Reversible", "AffineCouplingBlock", "InvertibleConv1x1", "AffineCouplingFunc",
@@ -25,4 +26,4 @@ __all__ = ["FlowBase", "Reversible", "AffineCouplingBlock", "InvertibleConv1x1",
            "WaveGlow", "WSRGlow", "MRWaveGlow", "MelGlow", "WN_LVC", "WaveFlow", "WN2D", "NonCausalLayer2D", "fused_gate", "add_weight_norms", "remove_weight_norms", "get_instance", "set_precision",
            "get_precision", "invalidate_packs", "pad_batch", "Denoiser",
            "NvidiaWaveGlow", "load_nvidia_waveglow", "MelSpec", "TacotronSTFT",
-           "Resample"]
+           "Resample", "SpectralDistance"]

@@ -98,6 +98,9 @@ SIGNATURES = {
     "cmwg_stft_frame_magnitude": (_I, [_VP, _I, _VP, _I, _I, _I, _VP, _VP]),
     "cmwg_denoise": (_I, [_VP, _LL, _I, _I, C.POINTER(C.c_int), _VP, _VP, _VP, C.c_float, _I, _I, _VP, _VP, _VP]),
     "cmwg_resample": (_I, [_VP, _LL, _I, _I, C.POINTER(C.c_int), _VP, _VP, _VP, _I, _I, _I, _I, _VP, _LL, _I, _VP]),
+    "cmwg_spectral_distance_workspace_bytes": (_SZ, [_I, _I, _I, _I]),
+    "cmwg_spectral_distance": (_I, [_VP, _VP, _LL, _I, _I, C.POINTER(C.c_int), _VP, _VP, _VP, _VP, _VP, _VP, _I, _I, _I, _I,
+                                    _VP, _VP, _VP]),
     "cmwg_wsrglow_cond": (_I, [_VP, _I, _I, _VP, _I, _I, _VP, _I, _I, _VP, _VP, _VP, _VP, _VP]),
     "cmwg_lvc_gate_forward": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _I, _I, _VP, _VP]),
     "cmwg_lvc_gate_backward": (_I, [_VP, _VP, _VP, _I, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP]),

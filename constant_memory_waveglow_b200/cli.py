@@ -1,4 +1,4 @@
-"""Command line of the harness: ``python -m constant_memory_waveglow_b200.cli {train,synth,synth-batch,vocode,score} ...``.
+"""Command line of the harness: ``python -m constant_memory_waveglow_b200.cli {train,synth,synth-batch,vocode,score,compare} ...``.
 
 The reference's own ``train.py`` runs unchanged on the ``pytorch_lightning`` / ``model`` / ``datasets`` shims at the
 repository root; its ``inference.py`` cannot in this image (``torchaudio.load`` / ``save`` need the absent TorchCodec),
@@ -12,7 +12,9 @@ given ``.wav`` files it computes their mels first (Tacotron2's ``TacotronSTFT`` 
 conditioner otherwise): copy synthesis.  ``score`` prints the per-file negative log-likelihood of WAV files under a
 checkpoint, in the convention of the training loss (``WaveGlowLoss``).  WAV inputs must be at the front end's rate unless
 ``--resample`` is given (``vocode``, ``score``): files at other rates are then resampled on the GPU (``Resample``, in
-length-sorted batches per source rate).  ``vocode --output-rate HZ`` resamples the synthesised audio to HZ.
+length-sorted batches per source rate).  ``vocode --output-rate HZ`` resamples the synthesised audio to HZ.  ``compare
+SYNTH_DIR REF.wav...`` prints the spectral distances (``SpectralDistance``: LSD, log-mel L1, MCD) between each reference and
+``SYNTH_DIR/<name>.wav``, the file ``vocode`` writes for it, in length-sorted batches with per-item lengths.
 """
 from __future__ import annotations
 
@@ -442,12 +444,79 @@ def score_files(ckpt: str, paths, sigma: float, max_batch: int, p: argparse.Argu
     return [(f, signals[i].numel(), nll[i]) for i, f in enumerate(paths)]
 
 
+def compare(argv) -> None:
+    p = argparse.ArgumentParser(prog="cli compare", description="spectral distances (SpectralDistance: LSD, log-mel L1, "
+                                "MCD) between reference WAV files and the files of the same names in SYNTH_DIR, as `cli "
+                                "vocode` writes them; prints name, samples, lsd, mel_l1 and mcd per pair, then their means")
+    p.add_argument("synth_dir", type=str)
+    p.add_argument("refs", type=str, nargs="+", help="reference .wav files; REF.wav is compared with SYNTH_DIR/REF.wav")
+    p.add_argument("--max-batch", type=int, default=16, help="pairs per distance call")
+    p.add_argument("--sampling-rate", type=int, default=22050,
+                   help="the rate both files of every pair must have (the rate of the STFT and mel)")
+    p.add_argument("--resample", action="store_true",
+                   help="accept files at any rate: they are resampled on the GPU to --sampling-rate first")
+    args = p.parse_args(argv)
+    if args.max_batch < 1:
+        p.error("--max-batch must be >= 1")
+    if args.sampling_rate < 1:
+        p.error("--sampling-rate must be >= 1")
+    for name, n, lsd, mel_l1, mcd in compare_files(args.synth_dir, args.refs, args.sampling_rate, args.max_batch, p,
+                                                   args.resample):
+        print(f"{name}\t{n}\t{lsd:.6f}\t{mel_l1:.6f}\t{mcd:.6f}")
+
+
+def compare_files(synth_dir: str, refs, rate: int, max_batch: int, p: argparse.ArgumentParser, resample: bool = False):
+    """[(name, samples, lsd, mel_l1, mcd)] for each reference in input order, then ("mean", total samples, the three means
+    over the pairs).  Each pair is compared over the shorter of its two sample counts (at `rate`, after resampling when
+    `resample`); counts that differ by more than a hop mean a wrong pairing and are refused.  Pairs run in length-sorted
+    batches of `max_batch`, one SpectralDistance call with the per-item lengths each."""
+    from .base import pad_batch
+    from .datasets import wav_info
+    from .distance import SpectralDistance
+    synths = [os.path.join(synth_dir, os.path.splitext(os.path.basename(f))[0] + ".wav") for f in refs]
+    for ref, syn in zip(refs, synths):
+        if not os.path.isfile(syn):
+            p.error(f"{syn}: no such file to compare with {ref}")
+    paths = list(refs) + synths
+    rates = [wav_info(f).sample_rate for f in paths]
+    for f, sr in zip(paths, rates):
+        if sr != rate and not resample:
+            p.error(f"{f}: sampled at {sr} Hz, not at --sampling-rate {rate} Hz (resample it first, or pass --resample)")
+    dist = SpectralDistance(sampling_rate=rate)
+    hop, half = dist.hop_length, dist.filter_length // 2
+    dev = torch.device("cuda")
+    signals = _resample_batches([wav_read(f).mean(0) for f in paths], rates, rate, max_batch, dev)
+    ref_sig, syn_sig = signals[:len(refs)], signals[len(refs):]
+    counts = []
+    for ref, syn, x, y in zip(refs, synths, ref_sig, syn_sig):
+        if abs(x.numel() - y.numel()) > hop:
+            p.error(f"{ref} has {x.numel()} samples and {syn} {y.numel()}: they differ by more than a hop ({hop}), so "
+                    "they are not a synthesis and its source")
+        n = min(x.numel(), y.numel())
+        if n <= half:
+            p.error(f"{ref}, {syn}: {n} samples are too few to compare (more than filter_length/2 = {half} needed)")
+        counts.append(n)
+    dist = dist.to(dev)
+    rows = [None] * len(refs)
+    order = sorted(range(len(refs)), key=lambda i: counts[i])
+    for s0 in range(0, len(order), max_batch):
+        idx = order[s0:s0 + max_batch]
+        x, lens = pad_batch([ref_sig[i][:counts[i]] for i in idx])
+        y, _ = pad_batch([syn_sig[i][:counts[i]] for i in idx])
+        d = torch.stack(dist(x.to(dev), y.to(dev), lengths=lens), 1).cpu()
+        for j, i in enumerate(idx):
+            rows[i] = (refs[i], counts[i], *(float(v) for v in d[j]))
+    means = [sum(r[k] for r in rows) / len(rows) for k in (2, 3, 4)]
+    return rows + [("mean", sum(counts), *means)]
+
+
 def main(argv=None) -> None:
     argv = list(sys.argv[1:] if argv is None else argv)
-    verbs = {"train": train, "synth": synth, "synth-batch": synth_batch, "vocode": vocode, "score": score}
+    verbs = {"train": train, "synth": synth, "synth-batch": synth_batch, "vocode": vocode, "score": score,
+             "compare": compare}
     if not argv or argv[0] not in verbs:
-        raise SystemExit("usage: python -m constant_memory_waveglow_b200.cli {train,synth,synth-batch,vocode,score} [flags]  "
-                         "(-h after the verb)")
+        raise SystemExit("usage: python -m constant_memory_waveglow_b200.cli {train,synth,synth-batch,vocode,score,compare} "
+                         "[flags]  (-h after the verb)")
     verbs[argv[0]](argv[1:])
 
 

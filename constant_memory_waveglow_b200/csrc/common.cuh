@@ -127,6 +127,19 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
+// sum of v over the CTA (blockDim.x <= 1024) in a fixed order; red holds 32 floats of shared memory
+__device__ __forceinline__ float block_sum_1024(float v, float* red) {
+  v = warp_sum(v);
+  int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  if (lane == 0) red[wid] = v;
+  __syncthreads();
+  int nw = (blockDim.x + 31) >> 5;
+  float r = (threadIdx.x < nw) ? red[threadIdx.x] : 0.f;
+  if (wid == 0) r = warp_sum(r);
+  __syncthreads();
+  return r;  // valid in warp 0
+}
+
 // accurate (fp32 mode) and fast (tensor-core modes) gate non-linearities
 template <bool FAST> __device__ __forceinline__ float tanh_f(float x) {
   if (FAST) {

@@ -590,18 +590,6 @@ __global__ void __launch_bounds__(256) squeeze_kernel(const float* __restrict__ 
 // ------------------------------------------------------------------------------------------------
 // reductions: per-batch sum, NLL loss
 // ------------------------------------------------------------------------------------------------
-__device__ float block_sum_1024(float v, float* red) {
-  v = warp_sum(v);
-  int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  if (lane == 0) red[wid] = v;
-  __syncthreads();
-  int nw = (blockDim.x + 31) >> 5;
-  float r = (threadIdx.x < nw) ? red[threadIdx.x] : 0.f;
-  if (wid == 0) r = warp_sum(r);
-  __syncthreads();
-  return r;  // valid in warp 0
-}
-
 __global__ void __launch_bounds__(1024) sum_per_batch_kernel(const float* __restrict__ a, long long a_bs, int N,
                                                              float* __restrict__ out, int accumulate,
                                                              float scale) {

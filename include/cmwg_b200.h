@@ -339,6 +339,26 @@ int cmwg_resample(const float* x, long long x_bstride, int B, int T, const int* 
                   void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Spectral distances between (reference, estimate) pairs: log-spectral distance, log-mel L1 and mel-cepstral distortion on
+ * Tacotron2's STFT and mel (the framing of cmwg_melspec_fwd_varlen with pad_left = n_fft/2 and power_is_one = 1).  Per item
+ * b, over the first len_b samples of both signals (len_b = lengths[b], or T when both length pointers are NULL;
+ * n_fft/2 < len_b <= T), with S, S^ the STFTs (reflect padding at len_b, len_b / hop + 1 frames, n_fft/2 + 1 bins) and per
+ * frame P = |S|^2, m = ln max(mel @ |S|, 1e-5), c = D m:
+ *   out[b][0] = mean_f sqrt(mean_k (log10 max(P, 1e-10) - log10 max(P^, 1e-10))^2)          (LSD)
+ *   out[b][1] = mean_f mean_j |m_j - m^_j|                                                  (log-mel L1)
+ *   out[b][2] = mean_f (10 / ln 10) sqrt(2 sum_{d=1}^{n_cep-1} (c_d - c^_d)^2)                (MCD, c0 excluded)
+ * window (n_fft), fbt / fb_lo / fb_hi as for cmwg_melspec_fwd; dct (n_cep, n_mels) row major, the orthonormal DCT-II;
+ * 2 <= n_cep <= n_mels.  ref, est: (B, T) at batch stride bstride; out (B, 3) contiguous.  workspace:
+ * cmwg_spectral_distance_workspace_bytes(B, T, n_fft, hop) bytes (the per-frame terms).  Summed in a fixed order without
+ * atomics: deterministic, and each item equals a call on that item alone bit for bit.  Nothing is allocated.
+ * n_fft other than a power of two in [128, 4096]: CMWG_ERR_UNSUPPORTED; bad sizes or lengths: CMWG_ERR_ARG. */
+size_t cmwg_spectral_distance_workspace_bytes(int B, int T, int n_fft, int hop);
+int cmwg_spectral_distance(const float* ref, const float* est, long long bstride, int B, int T, const int* lengths_host,
+                           const int* lengths_dev, const float* window, const float* fbt, const int* fb_lo,
+                           const int* fb_hi, const float* dct, int n_fft, int hop, int n_mels, int n_cep, void* workspace,
+                           float* out, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * WSRGlow conditioning front end (model/wsrglow.py:37-50, `_get_cond`), one kernel:
  *   c (B, Tc) fp32 low-rate signal, CLIPPED TO [-1, 1] IN PLACE like the reference's c.clip_(-1, 1) (:38);
  *   out (B, 8E + 9 + 9P, Tc/8) fp32 NCL = cat(mu-law code embedding rows (emb: n_codes x E, :39), the 9 magnitudes of
