@@ -133,3 +133,20 @@ def lengths_list(lengths: Lengths, batch: int, what: str, unit: str) -> List[int
     if len(out) != batch:
         raise ValueError(f"{what}: {len(out)} lengths for a batch of {batch}")
     return out
+
+
+def audio_lengths(x: Tensor, lengths: Optional[Lengths], pad: int, what: str,
+                  check_full: bool = True) -> Optional[List[int]]:
+    """The argument checks of an audio op with per-item lengths (no device needed): x (T,) or (B, T), and each length in
+    (pad, T], `pad` being the op's reflect padding (0 for none).  When `lengths` is None, T itself is checked unless
+    `check_full` is False.  Returns the lengths as a list of ints, or None."""
+    if x.dim() not in (1, 2):
+        raise ValueError(f"{what}: expected audio (T,) or (B, T), got {tuple(x.shape)}")
+    B = 1 if x.dim() == 1 else x.shape[0]
+    T = x.shape[-1]
+    lens = None if lengths is None else lengths_list(lengths, B, what, "samples")
+    for n in (lens if lens is not None else ([T] if B and check_full else [])):
+        if not pad < n <= T:
+            reason = f": reflect padding by {pad} samples needs more samples than the pad" if pad else ""
+            raise ValueError(f"{what}: length {n} outside ({pad}, {T}]{reason} (lengths are in samples)")
+    return lens

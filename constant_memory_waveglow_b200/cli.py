@@ -148,6 +148,20 @@ def item_noise(seed: int, index: int, n: int, sigma: float) -> torch.Tensor:
     return torch.randn(n, generator=g) * sigma
 
 
+def _group_noise(seed: int, idx, samples, sigma: float) -> torch.Tensor:
+    """The noise of one synthesis call over files `idx`: item_noise of file idx[j] with samples[j] samples, zero-padded to
+    the longest."""
+    from .base import pad_batch
+    return pad_batch([item_noise(seed, i, n, sigma) for i, n in zip(idx, samples)])[0]
+
+
+def _length_groups(items, length, max_batch: int) -> list:
+    """`items` sorted by `length(item)` (ties keep their order) and cut into consecutive groups of at most `max_batch`: the
+    batches of the batched verbs, which write each item of a group back to its own place in input order."""
+    order = sorted(items, key=length)
+    return [order[s0:s0 + max_batch] for s0 in range(0, len(order), max_batch)]
+
+
 def synth_batch(argv) -> None:
     p = argparse.ArgumentParser(prog="cli synth-batch",
                                 description="analysis + synthesis of many files, batched by length (one output per input)")
@@ -175,18 +189,14 @@ def synth_batch(argv) -> None:
         for f in args.infiles:
             rates.append(wav_info(f).sample_rate)
             conds.append(conditioner(wav_read(f).mean(0, keepdim=True).to(dev))[0])
-        order = sorted(range(len(conds)), key=lambda i: conds[i].shape[-1])
+        groups = _length_groups(range(len(conds)), lambda i: conds[i].shape[-1], args.max_batch)
         denoiser = None
         if args.denoiser_strength > 0:
-            denoiser = _denoiser(model, conds[order[0]].shape[-1] * hop, p)
+            denoiser = _denoiser(model, conds[groups[0][0]].shape[-1] * hop, p)
         total, cost = 0, 0.0
-        for s0 in range(0, len(order), args.max_batch):
-            idx = order[s0:s0 + args.max_batch]
+        for idx in groups:
             h, frames = pad_batch([conds[i] for i in idx])
-            z = torch.zeros((len(idx), h.shape[-1] * hop))
-            for j, i in enumerate(idx):
-                z[j, :frames[j] * hop] = item_noise(args.seed, i, frames[j] * hop, args.sigma)
-            z = z.to(dev)
+            z = _group_noise(args.seed, idx, [f * hop for f in frames], args.sigma).to(dev)
             x, dt = _timed(lambda: model.infer(h, args.sigma, z=z, lengths=frames))
             cost += dt
             if denoiser is not None:
@@ -267,9 +277,7 @@ def _resample_batches(signals, rates, rate: int, max_batch: int, dev) -> list:
     out = list(signals)
     for sr in sorted(set(rates) - {rate}):
         rs = Resample(sr, rate).to(dev)
-        order = sorted((i for i, r in enumerate(rates) if r == sr), key=lambda i: signals[i].numel())
-        for s0 in range(0, len(order), max_batch):
-            idx = order[s0:s0 + max_batch]
+        for idx in _length_groups([i for i, r in enumerate(rates) if r == sr], lambda i: signals[i].numel(), max_batch):
             x, lens = pad_batch([signals[i] for i in idx])
             with torch.no_grad():
                 y = rs(x.to(dev), lengths=lens)
@@ -284,12 +292,9 @@ def _frontend_mels(frontend, signals, names, max_batch: int, dev, p: argparse.Ar
     from .base import pad_batch
     from .condition import MelSpec, TacotronSTFT
     batched = isinstance(frontend, (MelSpec, TacotronSTFT))
-    step = max_batch if batched else 1
-    order = sorted(range(len(signals)), key=lambda i: signals[i].numel())
     hop = frontend.hop_length
     out = [None] * len(signals)
-    for s0 in range(0, len(order), step):
-        idx = order[s0:s0 + step]
+    for idx in _length_groups(range(len(signals)), lambda i: signals[i].numel(), max_batch if batched else 1):
         x, lens = pad_batch([signals[i] for i in idx])
         try:
             m = frontend(x.to(dev), lengths=lens) if batched else frontend(x.to(dev))
@@ -354,18 +359,15 @@ def vocode(argv) -> None:
         for i, m, x in zip(wav_idx, wav_mels, signals):
             mels[i], n_out[i] = m, x.numel()
     os.makedirs(args.outdir, exist_ok=True)
-    order = sorted(range(len(mels)), key=lambda i: mels[i].shape[-1])
     # families without per-item lengths (WaveFlow, WSRGlow, ...) synthesise one utterance per call
-    max_batch = args.max_batch if model._supports_lengths else 1
+    groups = _length_groups(range(len(mels)), lambda i: mels[i].shape[-1],
+                            args.max_batch if model._supports_lengths else 1)
     with torch.no_grad():
-        denoiser = _denoiser(model, mels[order[0]].shape[-1] * hop, p) if args.denoiser_strength > 0 else None
+        denoiser = _denoiser(model, mels[groups[0][0]].shape[-1] * hop, p) if args.denoiser_strength > 0 else None
         total, cost = 0, 0.0
-        for s0 in range(0, len(order), max_batch):
-            idx = order[s0:s0 + max_batch]
+        for idx in groups:
             h, frames = pad_batch([mels[i] for i in idx])
-            z = torch.zeros((len(idx), h.shape[-1] * hop))
-            for j, i in enumerate(idx):
-                z[j, :frames[j] * hop] = item_noise(args.seed, i, frames[j] * hop, args.sigma)
+            z = _group_noise(args.seed, idx, [f * hop for f in frames], args.sigma)
             h, z = h.to(dev), z.to(dev)
             lengths = frames if model._supports_lengths else None
             x, dt = _timed(lambda: model.infer(h, args.sigma, z=z, lengths=lengths).reshape(len(idx), -1))
@@ -424,8 +426,8 @@ def score_files(ckpt: str, paths, sigma: float, max_batch: int, p: argparse.Argu
     # The front end gives n / hop + 1 frames, one more when hop divides n, and this package's upsampler reaches back from
     # that frame into the item's last samples; such files run alone.  NVIDIA's upsampler only reaches forward.
     alone = [not model._supports_lengths or (x.numel() % hop == 0 and not isinstance(model, NvidiaWaveGlow)) for x in signals]
-    order = sorted((i for i in range(len(paths)) if not alone[i]), key=lambda i: signals[i].numel())
-    groups = [order[s0:s0 + max_batch] for s0 in range(0, len(order), max_batch)] + [[i] for i in range(len(paths)) if alone[i]]
+    groups = _length_groups([i for i in range(len(paths)) if not alone[i]], lambda i: signals[i].numel(), max_batch) \
+        + [[i] for i in range(len(paths)) if alone[i]]
     loss = WaveGlowLoss(sigma)
     nll = [None] * len(paths)
     with torch.no_grad():
@@ -498,9 +500,7 @@ def compare_files(synth_dir: str, refs, rate: int, max_batch: int, p: argparse.A
         counts.append(n)
     dist = dist.to(dev)
     rows = [None] * len(refs)
-    order = sorted(range(len(refs)), key=lambda i: counts[i])
-    for s0 in range(0, len(order), max_batch):
-        idx = order[s0:s0 + max_batch]
+    for idx in _length_groups(range(len(refs)), counts.__getitem__, max_batch):
         x, lens = pad_batch([ref_sig[i][:counts[i]] for i in idx])
         y, _ = pad_batch([syn_sig[i][:counts[i]] for i in idx])
         d = torch.stack(dist(x.to(dev), y.to(dev), lengths=lens), 1).cpu()

@@ -16,7 +16,6 @@ filterbank (librosa's ``filters.mel``) and ``log(clamp(x, min=1e-5))``, through 
 """
 from __future__ import annotations
 
-import ctypes as C
 import math
 from typing import List, Optional
 
@@ -25,6 +24,8 @@ import torch
 from torch import Tensor, nn
 
 from . import _lib as L
+from . import ops
+from .base import audio_lengths
 
 __all__ = ["MelSpec", "TacotronSTFT", "mel_filterbank", "slaney_mel_basis"]
 
@@ -89,38 +90,19 @@ def _kernel_tables(window: Tensor, fb: Tensor, n_fft: int, device):
 
 
 def mel_lengths(x: Tensor, lengths, n_fft: int, pad_left: int, what: str) -> Optional[List[int]]:
-    """The argument checks of the per-item-lengths mel transform (no device needed): x (T,) or (B, T), each length (or T
-    when `lengths` is None) in (max(pad_left, n_fft - pad_left), T].  Returns the lengths as a list of ints, or None."""
-    from .base import lengths_list
-    if x.dim() not in (1, 2):
-        raise ValueError(f"{what} expects (B, T) or (T,), got {tuple(x.shape)}")
-    B = 1 if x.dim() == 1 else x.shape[0]
-    T = x.shape[-1]
-    lens = None if lengths is None else lengths_list(lengths, B, what, "samples")
-    pad = max(pad_left, n_fft - pad_left)
-    for n in (lens if lens is not None else ([T] if B else [])):
-        if not pad < n <= T:
-            raise ValueError(f"{what}: length {n} outside ({pad}, {T}]: reflect padding by {pad} samples needs more "
-                             "samples than the pad (lengths are in samples)")
-    return lens
+    """audio_lengths for a mel transform that reflect-pads by pad_left and n_fft - pad_left: each length (T when `lengths`
+    is None) must exceed the larger pad."""
+    return audio_lengths(x, lengths, max(pad_left, n_fft - pad_left), what)
 
 
 def _melspec_varlen(x: Tensor, lens: Optional[List[int]], tables, n_fft: int, hop: int, n_mels: int, pad_left: int,
                     power_is_one: int, log_mode: int, eps: float) -> Tensor:
     """cmwg_melspec_fwd_varlen of x (B, T) or (T,) on the GPU -> (B, n_mels, T // hop + 1) (or (n_mels, frames))."""
-    squeeze = x.dim() == 1
-    x = x.detach()
-    if squeeze:
-        x = x.unsqueeze(0)
-    if x.dtype != torch.float32 or x.stride(1) != 1:
-        x = x.float().contiguous()
+    x, squeeze = ops.audio_batch(x)
     B, T = x.shape
     window, fbt, lo, hi = tables
     out = torch.empty((B, n_mels, T // hop + 1), device=x.device, dtype=torch.float32)
-    lens_host = lens_dev = None
-    if lens is not None:
-        lens_host = (C.c_int * B)(*lens)
-        lens_dev = torch.tensor(lens, dtype=torch.int32).to(x.device)
+    lens_host, lens_dev = ops.lengths_arg(lens, x.device)
     L.check(L.load().cmwg_melspec_fwd_varlen(x.data_ptr(), x.stride(0) if B > 1 else T, B, T, lens_host, L.ptr(lens_dev),
                                              window.data_ptr(), fbt.data_ptr(), lo.data_ptr(), hi.data_ptr(), n_fft, hop,
                                              n_mels, pad_left, power_is_one, log_mode, eps, out.data_ptr(),
@@ -237,20 +219,16 @@ class MelSpec(nn.Module):
     def forward(self, x: Tensor, lengths=None) -> Tensor:
         """``lengths``: valid samples per item of a zero-padded batch x (B, T).  Item b then gets ``len_b // hop + 1`` frames
         equal, bit for bit, to ``self(x[b, :len_b])``, and zeros after them."""
+        pad_left = self.n_fft // 2 - self.hop_length // 2
         if lengths is not None:
-            lens = mel_lengths(x, lengths, self.n_fft, self.n_fft // 2 - self.hop_length // 2, "MelSpec")
+            lens = mel_lengths(x, lengths, self.n_fft, pad_left, "MelSpec")
             L.require_cuda(x, op="MelSpec")
             return _melspec_varlen(x, lens, self._device_tables(x.device), self.n_fft, self.hop_length, self.n_mels,
-                                   self.n_fft // 2 - self.hop_length // 2, int(self.power == 1.0), 1, 1e-7)
+                                   pad_left, int(self.power == 1.0), 1, 1e-7)
         L.require_cuda(x, op="MelSpec")
-        squeeze = x.dim() == 1
-        if squeeze:
-            x = x.unsqueeze(0)
-        if x.dim() != 2:
-            raise ValueError(f"MelSpec expects (B, T) or (T,), got {tuple(x.shape)}")
-        x = x.detach()
-        if x.dtype != torch.float32 or x.stride(1) != 1:
-            x = x.float().contiguous()
+        if x.dim() not in (1, 2):
+            raise ValueError(f"MelSpec: expected audio (T,) or (B, T), got {tuple(x.shape)}")
+        x, squeeze = ops.audio_batch(x)
         B, T = x.shape
         lib = L.load()
         frames = lib.cmwg_melspec_frames(T, self.n_fft, self.hop_length)

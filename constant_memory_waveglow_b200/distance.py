@@ -4,7 +4,6 @@ csrc/distance.cu).  ``oracle/distance_oracle.py`` restates the definitions in fl
 """
 from __future__ import annotations
 
-import ctypes as C
 import math
 from typing import NamedTuple
 
@@ -12,6 +11,7 @@ import torch
 from torch import Tensor
 
 from . import _lib as L
+from . import ops
 from .condition import TacotronSTFT, mel_lengths
 
 __all__ = ["SpectralDistance", "Distances", "dct_matrix"]
@@ -78,9 +78,8 @@ class SpectralDistance(TacotronSTFT):
         L.require_cuda(ref, est, op="SpectralDistance")
         if ref.device != est.device:
             raise ValueError(f"SpectralDistance: ref on {ref.device} and est on {est.device}")
-        squeeze = ref.dim() == 1
-        x, y = (t.detach().unsqueeze(0) if squeeze else t.detach() for t in (ref, est))
-        x, y = (t.float().contiguous() for t in (x, y))
+        (x, squeeze), (y, _) = ops.audio_batch(ref), ops.audio_batch(est)
+        x, y = x.contiguous(), y.contiguous()   # the kernel takes one batch stride, T, for both
         B, T = x.shape
         window, fbt, lo, hi = self._device_tables(x.device)
         dct = self.dct.to(x.device)
@@ -88,10 +87,7 @@ class SpectralDistance(TacotronSTFT):
         workspace = torch.empty((max(int(lib.cmwg_spectral_distance_workspace_bytes(B, T, n_fft, self.hop_length)), 4),),
                                 device=x.device, dtype=torch.uint8)
         out = torch.empty((B, 3), device=x.device, dtype=torch.float32)
-        lens_host = lens_dev = None
-        if lens is not None:
-            lens_host = (C.c_int * B)(*lens)
-            lens_dev = torch.tensor(lens, dtype=torch.int32).to(x.device)
+        lens_host, lens_dev = ops.lengths_arg(lens, x.device)
         L.check(lib.cmwg_spectral_distance(x.data_ptr(), y.data_ptr(), T, B, T, lens_host, L.ptr(lens_dev),
                                            window.data_ptr(), fbt.data_ptr(), lo.data_ptr(), hi.data_ptr(),
                                            dct.data_ptr(), n_fft, self.hop_length, self.n_mel_channels,

@@ -15,7 +15,6 @@ split and early outputs -- with three differences that this module absorbs:
 from __future__ import annotations
 
 import collections
-import ctypes as C
 import io
 import os
 import pickle
@@ -32,7 +31,7 @@ from . import _lib as L
 from . import ops, precision
 from .base import FlowBase
 from .efficient_modules import AffineCouplingBlock, InvertibleConv1x1
-from .waveglow import WN, CondSlab, WaveGlow, _LogdetAccumulate, pack_generation
+from .waveglow import WN, CondSlab, WaveGlow, pack_generation
 
 HOP = 256        # NVIDIA's upsampler: ConvTranspose1d(n_mel, n_mel, 1024, stride=256)
 UP_KERNEL = 1024
@@ -132,7 +131,8 @@ class NvidiaWaveGlow(WaveGlow):
         return CondSlab(slab, (B, width, Tq), prec)
 
     def _prepare(self, x: Tensor, h: Tensor, lens: Optional[List[int]]):
-        """Squeezed input, conditioning, WN precision and (host, device) squeezed lengths or None."""
+        """The arguments of the direct loop: squeezed input, conditioning, the squeezed lengths (host, device) or (None,
+        None), and the WN precision, resolved once because the conditioning is built in it."""
         L.require_cuda(x, h, op="NvidiaWaveGlow")
         if h.shape[1] != self.n_mels:
             raise ValueError(f"NvidiaWaveGlow: expected {self.n_mels} mel channels, got {h.shape[1]}")
@@ -145,29 +145,12 @@ class NvidiaWaveGlow(WaveGlow):
             h = torch.where(torch.arange(h.shape[2], device=h.device)[None, None, :] < frames[:, None, None], h, 0.)
             x = torch.where(torch.arange(x.shape[1], device=x.device)[None, :] <
                             torch.tensor(lens, device=x.device)[:, None], x, 0.)
-            c = [n // self.n_group for n in lens]
-            cols = ((C.c_int * len(c))(*c), torch.tensor(c, dtype=torch.int32).to(x.device))
+            cols = [n // self.n_group for n in lens]
+        cols_host, cols_dev = ops.lengths_arg(cols, x.device)
         h = h.contiguous()
         xs = ops.squeeze(x.contiguous(), self.n_group, False)
         prec = precision.resolve(self.WNs[0].F._tc_supported(), training=False)
-        return xs, self._conditioning(h, xs.shape[2], prec), prec, cols
-
-    def _coupling(self, k: int, x: Tensor, y, prec: str, cols, inverse: bool) -> Tuple[Tensor, Tensor]:
-        F = self.WNs[k].F
-        if cols is None:
-            lst, _ = F._cmwg_forward(x, y, save=False, prec=prec)
-            z, neg = ops.coupling_apply(x, lst, inverse)
-        else:
-            lst = F._cmwg_forward_varlen(x, y, cols[0], cols[1], prec)
-            z, neg = ops.coupling_apply_varlen(x, lst, cols[1], inverse=inverse)
-        return z, (neg if inverse else lst[:, :F.in_chs])
-
-    def _conv_step(self, k: int, x: Tensor, inverse: bool, cols) -> Tuple[Tensor, Tensor]:
-        """The 1x1 conv of flow k and its log-det: of the whole call, or of one column when per-item lengths are given."""
-        if cols is None:
-            conv = self.invconv1x1[k]
-            return conv.reverse(x) if inverse else conv(x)
-        return self._varlen_conv(k, x, inverse)
+        return xs, self._conditioning(h, xs.shape[2], prec), cols_host, cols_dev, prec
 
     def _lens(self, x: Tensor, h: Tensor, lengths, what: str) -> Optional[List[int]]:
         self._require_no_grad(x, h, what)
@@ -180,43 +163,9 @@ class NvidiaWaveGlow(WaveGlow):
         lens = self._check_lengths(x, h, lengths, what)
         return lens if any(n != x.shape[1] for n in lens) else None   # all full: the ordinary call, same bits
 
-    def _accumulate(self, log_s: Tensor, cols, logdet, ldw):
-        if cols is None:
-            return _LogdetAccumulate.apply(logdet, ldw, log_s)
-        return ops.logdet_accumulate_varlen(log_s, cols[1], logdet, ldw)
-
-    def forward_computation(self, x: Tensor, h: Tensor, lengths=None) -> Tuple[Tensor, Tensor]:
-        lens = self._lens(x, h, lengths, "NvidiaWaveGlow.forward")
-        batch = x.shape[0]
-        x, y, prec, cols = self._prepare(x, h, lens)
-        early: List[Tensor] = []
-        logdet = None
-        for k in range(len(self.WNs)):
-            if k % self.n_early_every == 0 and k:
-                e, x = x.split([self.n_early_size, x.size(1) - self.n_early_size], 1)
-                early.append(e)
-            x, ldw = self._conv_step(k, x, False, cols)
-            x, log_s = self._coupling(k, x, y, prec, cols, False)
-            logdet = self._accumulate(log_s, cols, logdet, ldw)
-        early.append(x)
-        z = ops.squeeze(torch.cat(early, 1), self.n_group, True)
-        return z.view(batch, -1), logdet
-
-    def reverse_computation(self, z: Tensor, h: Tensor, lengths=None) -> Tuple[Tensor, Tensor]:
-        lens = self._lens(z, h, lengths, "NvidiaWaveGlow.reverse")
-        batch = z.shape[0]
-        z, y, prec, cols = self._prepare(z, h, lens)
-        parts = list(z.split(self.z_split_sizes, 1))
-        z = parts.pop()
-        logdet = None
-        for k in range(len(self.WNs) - 1, -1, -1):
-            z, log_s = self._coupling(k, z, y, prec, cols, True)
-            z, ldw = self._conv_step(k, z, True, cols)
-            logdet = self._accumulate(log_s, cols, logdet, ldw)
-            if k % self.n_early_every == 0 and k:
-                z = torch.cat((parts.pop(), z), 1)
-        x = ops.squeeze(z, self.n_group, True)
-        return x.view(batch, -1), logdet
+    def _direct_inputs(self, x: Tensor, h: Tensor, lengths, what: str):
+        """Every call takes the direct loop, with per-item lengths or without."""
+        return self._prepare(x, h, self._lens(x, h, lengths, what))
 
 
 # ---------------------------------------------------------------------------------------------------------------------

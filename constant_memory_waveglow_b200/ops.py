@@ -14,6 +14,7 @@ from typing import List, Optional, Tuple
 import torch
 
 from . import _lib as L
+from .base import audio_lengths
 
 
 def _ncl(t: torch.Tensor) -> torch.Tensor:
@@ -288,38 +289,38 @@ def stft_frame_magnitude(x: torch.Tensor, window: torch.Tensor, hop: int, frame:
     return mag
 
 
-def denoise_lengths(audio: torch.Tensor, n_fft: int, strength: float, lengths) -> Optional[List[int]]:
-    """The argument checks of denoise() (no device needed): audio (T,) or (B, T), strength >= 0, each length in
-    (n_fft // 2, T].  Returns the lengths as a list of ints, or None."""
-    from .base import lengths_list
-    if audio.dim() not in (1, 2):
-        raise ValueError(f"denoise: expected audio (T,) or (B, T), got {tuple(audio.shape)}")
-    if isinstance(strength, bool) or not isinstance(strength, numbers.Real) or not 0 <= strength < math.inf:
-        raise ValueError(f"denoise: strength must be a finite number >= 0, got {strength!r}")
-    B = 1 if audio.dim() == 1 else audio.shape[0]
-    T = audio.shape[-1]
-    lens = None if lengths is None else lengths_list(lengths, B, "denoise", "samples")
-    for n in (lens if lens is not None else ([T] if B else [])):
-        if not n_fft // 2 < n <= T:
-            raise ValueError(f"denoise: length {n} outside ({n_fft // 2}, {T}]: reflect padding by n_fft/2 needs more "
-                             "samples than the pad (lengths are in samples)")
-    return lens
+def lengths_arg(lens: Optional[List[int]], device) -> Tuple[Optional[C.Array], Optional[torch.Tensor]]:
+    """Per-item lengths as the C ABI takes them: a ctypes int array on the host and the same values as an int32 tensor on
+    `device`, or (None, None).  The upload waits for the stream (a blocking copy from pageable memory), so callers make it
+    just before the launch: host work between the two would leave the GPU idle."""
+    if lens is None:
+        return None, None
+    return (C.c_int * len(lens))(*lens), torch.tensor(lens, dtype=torch.int32).to(device)
+
+
+def audio_batch(x: torch.Tensor) -> Tuple[torch.Tensor, bool]:
+    """x (T,) or (B, T) as a (B, T) float32 tensor with unit time stride (x itself when it is one), and whether to index the
+    result back to x's rank."""
+    squeeze = x.dim() == 1
+    x = x.detach()
+    if squeeze:
+        x = x.unsqueeze(0)
+    if x.dtype != torch.float32 or x.stride(1) != 1:
+        x = x.float().contiguous()
+    return x, squeeze
 
 
 def denoise(audio: torch.Tensor, window: torch.Tensor, bias_mag: torch.Tensor, strength: float, hop: int,
             lengths=None, workspace: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Bias-spectrum subtraction (cmwg_denoise) of audio (T,) or (B, T) with optional per-item `lengths` in samples; returns
     a tensor of audio's shape, 0 after each item's length.  `workspace`: uint8 tensor of at least
-    cmwg_denoise_workspace_bytes bytes (allocated here when None)."""
+    cmwg_denoise_workspace_bytes bytes (allocated here when None).  Each length must exceed n_fft / 2."""
     n_fft = window.numel()
-    lens = denoise_lengths(audio, n_fft, strength, lengths)
+    if isinstance(strength, bool) or not isinstance(strength, numbers.Real) or not 0 <= strength < math.inf:
+        raise ValueError(f"denoise: strength must be a finite number >= 0, got {strength!r}")
+    lens = audio_lengths(audio, lengths, n_fft // 2, "denoise")
     L.require_cuda(audio, window, bias_mag, op="denoise")
-    x = audio.detach()
-    squeeze = x.dim() == 1
-    if squeeze:
-        x = x.unsqueeze(0)
-    if x.dtype != torch.float32 or x.stride(1) != 1:
-        x = x.float().contiguous()
+    x, squeeze = audio_batch(audio)
     B, T = x.shape
     out = torch.empty((B, T), device=x.device, dtype=torch.float32)
     lib = L.load()
@@ -328,10 +329,7 @@ def denoise(audio: torch.Tensor, window: torch.Tensor, bias_mag: torch.Tensor, s
         workspace = torch.empty((max(need, 4),), device=x.device, dtype=torch.uint8)
     elif workspace.numel() * workspace.element_size() < need:
         raise ValueError(f"denoise: workspace of {workspace.numel() * workspace.element_size()} bytes, {need} needed")
-    lens_host = lens_dev = None
-    if lens is not None:
-        lens_host = (C.c_int * B)(*lens)
-        lens_dev = torch.tensor(lens, dtype=torch.int32).to(x.device)
+    lens_host, lens_dev = lengths_arg(lens, x.device)
     L.check(lib.cmwg_denoise(x.data_ptr(), x.stride(0) if B > 1 else T, B, T, lens_host, L.ptr(lens_dev),
                              window.data_ptr(), bias_mag.data_ptr(), float(strength), n_fft, int(hop),
                              workspace.data_ptr(), out.data_ptr(), L.stream_ptr(x.device)), "denoise")
@@ -342,20 +340,9 @@ def denoise(audio: torch.Tensor, window: torch.Tensor, bias_mag: torch.Tensor, s
 # band-limited resampling
 # ---------------------------------------------------------------------------------------------
 def resample_lengths(x: Tensor, lengths) -> Optional[List[int]]:
-    """The argument checks of resample (no device needed): x (T,) or (B, T), each length in [1, T].  Returns the lengths
-    as a list of ints, or None."""
-    from .base import lengths_list
-    if x.dim() not in (1, 2):
-        raise ValueError(f"Resample expects (B, T) or (T,), got {tuple(x.shape)}")
-    if lengths is None:
-        return None
-    B = 1 if x.dim() == 1 else x.shape[0]
-    T = x.shape[-1]
-    lens = lengths_list(lengths, B, "Resample", "samples")
-    for n in lens:
-        if not 1 <= n <= T:
-            raise ValueError(f"Resample: length {n} outside [1, {T}] (lengths are in samples)")
-    return lens
+    """audio_lengths for resample: each length in [1, T]; T itself is not bounded, so an empty signal resamples to an empty
+    one."""
+    return audio_lengths(x, lengths, 0, "Resample", check_full=False)
 
 
 def resample(x: Tensor, table: Tensor, first: Tensor, O: int, N: int, w: int, lengths=None) -> Tensor:
@@ -373,19 +360,11 @@ def resample(x: Tensor, table: Tensor, first: Tensor, O: int, N: int, w: int, le
         raise ValueError(f"resample: expected table (L, {N}) float32 and first ({N},) int32, got {tuple(table.shape)} "
                          f"{table.dtype} and {tuple(first.shape)} {first.dtype}")
     table, first = table.contiguous(), first.contiguous()
-    squeeze = x.dim() == 1
-    x = x.detach()
-    if squeeze:
-        x = x.unsqueeze(0)
-    if x.dtype != torch.float32 or x.stride(1) != 1:
-        x = x.float().contiguous()
+    x, squeeze = audio_batch(x)
     B, T = x.shape
     T_out = (N * T + O - 1) // O
     y = torch.empty((B, T_out), device=x.device, dtype=torch.float32)
-    lens_host = lens_dev = None
-    if lens is not None:
-        lens_host = (C.c_int * B)(*lens)
-        lens_dev = torch.tensor(lens, dtype=torch.int32).to(x.device)
+    lens_host, lens_dev = lengths_arg(lens, x.device)
     L.check(L.load().cmwg_resample(x.data_ptr(), x.stride(0) if B > 1 else T, B, T, lens_host, L.ptr(lens_dev),
                                    table.data_ptr(), first.data_ptr(), O, N, table.shape[0], w, y.data_ptr(),
                                    T_out, T_out, L.stream_ptr(x.device)), "resample")

@@ -514,8 +514,9 @@ class WaveGlow(FlowBase):
         return lens
 
     def _varlen_prepare(self, x: Tensor, h: Tensor, lens: List[int]):
-        """x and h with their padding zeroed -> the squeezed input, the upsampled conditioning and the per-item lengths in
-        squeezed columns (host ctypes array and device int32 tensor)."""
+        """x and h with their padding zeroed -> the arguments of the direct loop: the squeezed input, the upsampled
+        conditioning, the per-item lengths in squeezed columns (host ctypes array and device int32 tensor) and None for the
+        precision (resolved per flow)."""
         L.require_cuda(x, h, op="WaveGlow")
         B, T = x.shape
         hop = self._hop_length
@@ -532,65 +533,87 @@ class WaveGlow(FlowBase):
         xs = ops.squeeze(x, self.n_group, False)
         assert xs.size(2) <= y.size(2)
         y = y[..., :xs.size(2)]
-        cols = [n // self.n_group for n in lens]
-        cols_host = (C.c_int * B)(*cols)
-        cols_dev = torch.tensor(cols, dtype=torch.int32).to(x.device)
-        return xs, y, cols_host, cols_dev
+        return (xs, y) + ops.lengths_arg([n // self.n_group for n in lens], x.device) + (None,)
 
-    # One flow's two steps on a padded batch.  `inverse` is the direction the model asks for; a module built with
-    # reverse_mode=True swaps it (Reversible._direction), exactly as the ordinary path's module calls do.
-    def _varlen_conv(self, k: int, x: Tensor, inverse: bool) -> Tuple[Tensor, Tensor]:
+    def _direct_inputs(self, x: Tensor, h: Tensor, lengths: Optional[Lengths], what: str):
+        """The arguments of the direct loop (_direct_forward / _direct_reverse), or None for the module path.  WaveGlow
+        takes the direct loop for per-item lengths that are not all T; all lengths == T is the ordinary call, same bits."""
+        if lengths is None:
+            return None
+        lens = self._check_lengths(x, h, lengths, what)
+        if all(n == x.shape[1] for n in lens):
+            return None
+        return self._varlen_prepare(x, h, lens)
+
+    # ---- the direct loop: inference straight on the kernels, with or without per-item lengths ---------------------------
+    # x is the squeezed input, y the conditioning; lengths_host / lengths_dev the per-item lengths in squeezed columns or
+    # None; `prec` the WN precision of every flow, or None to resolve it per flow.  `inverse` is the direction the model asks
+    # for; a module built with reverse_mode=True swaps it (Reversible._direction), exactly as the module path's calls do.
+    def _direct_conv(self, k: int, x: Tensor, inverse: bool) -> Tuple[Tensor, Tensor]:
+        """The 1x1 conv of flow k and the log-det of one column."""
         conv = self.invconv1x1[k]
         inv = inverse != bool(conv._reverse_mode)
         w2 = conv.weight.detach().reshape(conv.weight.shape[0], -1).float().contiguous()
         winv, ld = ops.small_inverse_logdet(w2)
         return ops.conv1x1_apply(winv if inv else w2, x), (-ld if inv else ld)
 
-    def _varlen_coupling(self, k: int, x: Tensor, y: Tensor, cols_host, cols_dev: Tensor,
+    def _direct_coupling(self, k: int, x: Tensor, y, lengths_host, lengths_dev: Optional[Tensor], prec: Optional[str],
                          inverse: bool) -> Tuple[Tensor, Tensor]:
         coup = self.WNs[k]
         inv = inverse != bool(coup._reverse_mode)
         F = coup.F
-        lst = F._cmwg_forward_varlen(x, y, cols_host, cols_dev, precision.resolve(F._tc_supported(), training=False))
-        z, neg_log_s = ops.coupling_apply_varlen(x, lst, cols_dev, inverse=inv)
+        if prec is None:
+            prec = precision.resolve(F._tc_supported(), training=False)
+        if lengths_dev is None:
+            lst, _ = F._cmwg_forward(x, y, save=False, prec=prec)
+            z, neg_log_s = ops.coupling_apply(x, lst, inv)
+        else:
+            lst = F._cmwg_forward_varlen(x, y, lengths_host, lengths_dev, prec)
+            z, neg_log_s = ops.coupling_apply_varlen(x, lst, lengths_dev, inverse=inv)
         return z, (neg_log_s if inv else lst[:, :F.in_chs])
 
-    def _forward_varlen(self, x: Tensor, h: Tensor, lens: List[int]) -> Tuple[Tensor, Tensor]:
+    @staticmethod
+    def _direct_logdet(log_s: Tensor, lengths_dev: Optional[Tensor], prev, ldw_col: Tensor) -> Tensor:
+        """prev + the conv's log-det over each item's columns + the sum of log_s over them."""
+        if lengths_dev is None:
+            return ops.logdet_accumulate(log_s, prev, ldw_col * log_s.shape[2])
+        return ops.logdet_accumulate_varlen(log_s, lengths_dev, prev, ldw_col)
+
+    def _direct_forward(self, x: Tensor, y, lengths_host, lengths_dev: Optional[Tensor],
+                        prec: Optional[str]) -> Tuple[Tensor, Tensor]:
         batch = x.size(0)
-        x, y, cols_host, cols_dev = self._varlen_prepare(x, h, lens)
         early: List[Tensor] = []
         logdet = None
         for k in range(len(self.WNs)):
             if k % self.n_early_every == 0 and k:
                 e, x = x.split([self.n_early_size, x.size(1) - self.n_early_size], 1)
                 early.append(e)
-            x, ldw = self._varlen_conv(k, x, False)
-            x, log_s = self._varlen_coupling(k, x, y, cols_host, cols_dev, False)
-            logdet = ops.logdet_accumulate_varlen(log_s, cols_dev, logdet, ldw)
+            x, ldw = self._direct_conv(k, x, False)
+            x, log_s = self._direct_coupling(k, x, y, lengths_host, lengths_dev, prec, False)
+            logdet = self._direct_logdet(log_s, lengths_dev, logdet, ldw)
         early.append(x)
         z = ops.squeeze(torch.cat(early, 1), self.n_group, True)
         return z.view(batch, -1), logdet
 
-    def _reverse_varlen(self, z: Tensor, h: Tensor, lens: List[int]) -> Tuple[Tensor, Tensor]:
+    def _direct_reverse(self, z: Tensor, y, lengths_host, lengths_dev: Optional[Tensor],
+                        prec: Optional[str]) -> Tuple[Tensor, Tensor]:
         batch = z.size(0)
-        z, y, cols_host, cols_dev = self._varlen_prepare(z, h, lens)
         parts = list(z.split(self.z_split_sizes, 1))
         z = parts.pop()
         logdet = None
         for k in range(len(self.WNs) - 1, -1, -1):
-            z, log_s = self._varlen_coupling(k, z, y, cols_host, cols_dev, True)
-            z, ldw = self._varlen_conv(k, z, True)
-            logdet = ops.logdet_accumulate_varlen(log_s, cols_dev, logdet, ldw)
+            z, log_s = self._direct_coupling(k, z, y, lengths_host, lengths_dev, prec, True)
+            z, ldw = self._direct_conv(k, z, True)
+            logdet = self._direct_logdet(log_s, lengths_dev, logdet, ldw)
             if k % self.n_early_every == 0 and k:
                 z = torch.cat((parts.pop(), z), 1)
         x = ops.squeeze(z, self.n_group, True)
         return x.view(batch, -1), logdet
 
     def forward_computation(self, x: Tensor, h: Tensor, lengths: Optional[Lengths] = None) -> Tuple[Tensor, Tensor]:
-        if lengths is not None:
-            lens = self._check_lengths(x, h, lengths, "WaveGlow.forward")
-            if any(n != x.shape[1] for n in lens):   # all lengths == T: the ordinary call, same bits
-                return self._forward_varlen(x, h, lens)
+        direct = self._direct_inputs(x, h, lengths, f"{type(self).__name__}.forward")
+        if direct is not None:
+            return self._direct_forward(*direct)
         L.require_cuda(x, h, op="WaveGlow.forward")
         y = self._upsample_h(h)
         batch = x.size(0)
@@ -614,10 +637,9 @@ class WaveGlow(FlowBase):
         return z.view(batch, -1), logdet
 
     def reverse_computation(self, z: Tensor, h: Tensor, lengths: Optional[Lengths] = None) -> Tuple[Tensor, Tensor]:
-        if lengths is not None:
-            lens = self._check_lengths(z, h, lengths, "WaveGlow.reverse")
-            if any(n != z.shape[1] for n in lens):
-                return self._reverse_varlen(z, h, lens)
+        direct = self._direct_inputs(z, h, lengths, f"{type(self).__name__}.reverse")
+        if direct is not None:
+            return self._direct_reverse(*direct)
         L.require_cuda(z, h, op="WaveGlow.reverse")
         y = self._upsample_h(h)
         batch = z.size(0)

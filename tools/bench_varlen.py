@@ -113,14 +113,15 @@ def main():
     z10 = torch.randn(4, f10 * HOP, generator=g).to(dev) * SIGMA
     lens10 = [f10 * HOP] * 4
     with torch.no_grad():
-        reg = {"ordinary": lambda: m.reverse(z10, h10), "varlen": lambda: m._reverse_varlen(z10, h10, lens10)}
+        reg = {"ordinary": lambda: m.reverse(z10, h10),
+               "varlen": lambda: m._direct_reverse(*m._varlen_prepare(z10, h10, lens10))}
         for fn in reg.values():
             fn()
         rt = {k: [] for k in reg}
         for _ in range(args.reps * 2):
             for k, fn in reg.items():
                 rt[k].append(timed(fn))
-        same = torch.equal(m.reverse(z10, h10)[0], m._reverse_varlen(z10, h10, lens10)[0])
+        same = torch.equal(m.reverse(z10, h10)[0], reg["varlen"]()[0])
     name, power = gpu_info()
     print(json.dumps({
         "gpu": name, "power_limit": power, "utterances": len(frames), "valid_samples": valid,
